@@ -15,6 +15,10 @@ uniform ACGT, '%' between records, '$' at the end; u64 SA/LCP as the config name
   configs      : the other BASELINE.json configs (1, 3, 4, 5 and the repetitive variant 2b) at their full sizes
                  on one GPU, each with its own value, job roofline and full verification (--no-configs to skip)
 
+`--dump-outputs DIR` writes what the last timed step returned (see write_outputs), so that two builds of the project
+can be compared output for output: the workload text is generated from a fixed seed, so equal arguments give equal
+inputs.
+
 `--impl reference` times the reference's CPU algorithm (oracle port; the Rust reference cannot be compiled
 in this image) with the flags the workload names (-n 16, u64 indices) on a bounded sample of the same
 workload; the sample size is part of `config` in BOTH arms (reference_arm_sample_bases).
@@ -152,6 +156,51 @@ def oracle_run(sample: bytes, threads: int, partitions: int, index_bits: int = 6
     return r, dt
 
 
+DUMP_SAMPLE = 1 << 20  # entries per dumped array: about 38 MB in all
+DUMP_SEED = 20261020
+
+
+def dump_sample(n: int, seed: int) -> np.ndarray:
+    """Sorted, seeded sample of range(n), a function of (n, seed) only; all of range(n) when n <= DUMP_SAMPLE."""
+    if n <= DUMP_SAMPLE:
+        return np.arange(n, dtype=np.int64)
+    return np.unique(np.random.default_rng(seed).integers(0, n, DUMP_SAMPLE, dtype=np.int64))
+
+
+def write_outputs(out_dir, total_suffixes, ranks, sa, lcp, text_len, positions, text):
+    """--dump-outputs: sizes.npy = [suffixes, text bytes]; sa.npy / lcp.npy = the suffix and LCP arrays at the sampled
+    ranks (ranks.npy); text.npy = the transformed text at the sampled positions (positions.npy).  Indices are float64
+    (exact below 2^53), text bytes float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("sizes", [total_suffixes, text_len]), ("ranks", ranks), ("sa", sa), ("lcp", lcp),
+                    ("positions", positions)):
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float64))
+    np.save(os.path.join(out_dir, "text.npy"), np.asarray(text, dtype=np.float32))
+
+
+def dump_device_result(out_dir, res, rank, world, dev):
+    """write_outputs for a device result; with N > 1 every rank reads the sampled ranks of its shard and rank 0
+    writes them."""
+    import torch
+    import torch.distributed as dist
+    ranks = dump_sample(res.total_suffixes, DUMP_SEED)
+    lo = res.shard_offset
+    idx = torch.from_numpy(ranks[(ranks >= lo) & (ranks < lo + res.num_suffixes)] - lo).to(dev)
+
+    def read(t):
+        t = t[idx].to(torch.int64)
+        return (t & 0xFFFFFFFF if res.index_bits == 32 else t).cpu().numpy()  # u32 read through an int32 view
+    parts = [(read(res.sa_tensor()), read(res.lcp_tensor()))]
+    if world > 1:
+        mine, parts = parts[0], [None] * world
+        dist.all_gather_object(parts, mine)
+    if rank == 0:
+        positions = dump_sample(res.text_len, DUMP_SEED + 1)
+        text = res.text_tensor()[torch.from_numpy(positions).to(dev)].cpu().numpy()
+        write_outputs(out_dir, res.total_suffixes, ranks, np.concatenate([p[0] for p in parts]),
+                      np.concatenate([p[1] for p in parts]), res.text_len, positions, text)
+
+
 def reference_sample_bases(args):
     """Bases per step of the reference arm: bounded so that (steps + warmup) builds end within a few minutes
     at the ~25 M suffixes/s the port reaches, at most 1 Gbp."""
@@ -183,6 +232,10 @@ def run_reference(args):
         t += dt
         nsuf += r.num_suffixes
     value = nsuf / t
+    if args.dump_outputs:
+        ranks, positions = dump_sample(r.num_suffixes, DUMP_SEED), dump_sample(len(r.text), DUMP_SEED + 1)
+        write_outputs(args.dump_outputs, r.num_suffixes, ranks, r.sa[ranks], r.lcp[ranks], len(r.text), positions,
+                      np.frombuffer(r.text, dtype=np.uint8)[positions])
     line = {
         "impl": "reference", "metric": "suffixes/sec (SA+LCP)", "value": value, "unit": "suffixes/s",
         "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * t / args.steps,
@@ -225,7 +278,11 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--verify", type=int, default=1, help="0 = skip the full on-device verification of the last result")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's suffix array, LCP array and text (seeded sample) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: W >= 3
     if args.impl == "reference":
@@ -296,6 +353,8 @@ def main():
 
     # ---------------- FULL verification of the last timed result on the device (outside the timed region)
     verify = verify_full(last, last_meta, rank, world, dev) if args.verify else None
+    if args.dump_outputs:
+        dump_device_result(args.dump_outputs, last, rank, world, dev)
     last.free()
 
     # ---------------- e2e: host text in, host SA/LCP out, copies inside the timed region

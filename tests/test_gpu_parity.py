@@ -367,6 +367,36 @@ def test_bench_workload_generator_matches_cpu_restatement(S):
 
 
 @pytest.mark.parametrize("bits", [32, 64])
+def test_bench_dump_outputs_match_oracle(tmp_path, bits):
+    """`bench.py --dump-outputs`: the sampled suffix array, LCP array and text of the last timed step are the oracle's
+    at the dumped ranks and positions, and --steps sets the number of timed steps."""
+    import json
+    import subprocess
+    import sys
+    import bench
+    from conftest import ROOT
+    bases = 2_000_000  # more suffixes than bench.DUMP_SAMPLE: the sampled path
+    p = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--bases", str(bases), "--index-bits", str(bits),
+                        "--steps", "2", "--warmup", "3", "--no-configs", "--no-e2e", "--no-cpu",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert p.returncode == 0, p.stderr[-3000:]
+    line = json.loads(p.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2 and line["verify"]["ok"]
+    text_len, starts = bench.record_layout(bases)
+    want = O.oracle_build(bench.synth_prefix_numpy(text_len, text_len, starts), is_dna=True, threads=8, index_bits=bits)
+    d = {f.stem: np.load(f) for f in tmp_path.glob("*.npy")}
+    assert d["sizes"].tolist() == [want.num_suffixes, text_len]
+    assert d["sa"].dtype == np.float64 and d["text"].dtype == np.float32
+    ranks, positions = d["ranks"].astype(np.int64), d["positions"].astype(np.int64)
+    assert bench.DUMP_SAMPLE // 2 < len(ranks) <= bench.DUMP_SAMPLE < want.num_suffixes
+    assert (np.diff(ranks) > 0).all() and ranks[0] >= 0 and ranks[-1] < want.num_suffixes
+    assert np.array_equal(d["sa"], want.sa[ranks].astype(np.float64))
+    assert np.array_equal(d["lcp"], want.lcp[ranks].astype(np.float64))
+    assert np.array_equal(d["text"], np.frombuffer(want.text, np.uint8)[positions].astype(np.float32))
+    assert sum(f.stat().st_size for f in tmp_path.iterdir()) <= 64 << 20
+
+
+@pytest.mark.parametrize("bits", [32, 64])
 def test_positions_above_2_31(S, bits):
     """2.3 Gbp: suffix positions that do not fit 31 bits, u32 and u64 results (what `sufr create` writes for a
     human genome is u32).  Checked with the size-independent sample check of the bench."""

@@ -1,6 +1,7 @@
 """The full on-device verifier (sufr_b200_verify): it accepts results that are bit-exact with the oracle, in every
 mode, and it catches corrupted suffix / LCP arrays.  Also the large oracle comparisons (>= 100 M suffixes)."""
 import random
+import zlib
 
 import numpy as np
 import pytest
@@ -24,6 +25,11 @@ def device_build(S, text, index_bits=32, **kw):
     r = S.build(args, index_bits=index_bits, result_memory=S.MEM_DEVICE, device_text=(t.data_ptr(), t.numel()))
     r._keep = t
     return r
+
+
+def seed_of(*parts) -> int:
+    """Deterministic seed (Python's hash() of str is randomised per process)."""
+    return zlib.crc32(repr(parts).encode()) & 0xFFFF
 
 
 def rand_dna(seed, n, repeat_p=0.0, max_rep=60, alphabet=b"ACGT"):
@@ -53,7 +59,7 @@ MODES = {
 def test_verifier_accepts_oracle_exact_results(S, mode, bits):
     kw = MODES[mode]
     alphabet = b"ACGTNacgtn%" if kw.get("is_dna") else b"ACDEFGHIKLMNPQRSTVWY%"
-    text = rand_dna(hash((mode, bits)) & 0xFFFF, 60_000, repeat_p=0.02, alphabet=alphabet)
+    text = rand_dna(seed_of(mode, bits), 60_000, repeat_p=0.02, alphabet=alphabet)
     want = O.oracle_build(text, num_partitions=8, threads=4, index_bits=bits, **kw)
     r = device_build(S, text, bits, **kw)
     try:
@@ -279,7 +285,7 @@ def test_64bit_positions_forced_on_short_texts(S, monkeypatch, case, world):
     from sufr_b200.distributed import previous_last_suffix, shard_layout
     monkeypatch.setenv("SUFR_B200_DEBUG_POS64", "1")
     kw, alphabet, bits = POS64_CASES[case]
-    text = rand_dna(hash(case) & 0xFFFF, 120_000, repeat_p=0.02, alphabet=alphabet)
+    text = rand_dna(seed_of(case), 120_000, repeat_p=0.02, alphabet=alphabet)
     want = O.oracle_build(text, num_partitions=8, threads=4, index_bits=bits, **kw)
     shards = [S.build(S.SufrBuilderArgs(text=text, **kw), index_bits=bits, rank=r, world_size=world) for r in range(world)]
     try:

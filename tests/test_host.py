@@ -328,6 +328,28 @@ def test_cli_flag_surface(S):
     assert r.returncode == 1 and r.stderr.startswith("Error: ")        # cli.rs:102-109 create_empty_dies
 
 
+def test_bench_reference_arm_dump_outputs(tmp_path):
+    """`bench.py --impl reference --dump-outputs` (CPU only): the last timed step's arrays, whole below
+    bench.DUMP_SAMPLE, and --steps sets the number of timed steps."""
+    import json
+    import bench
+    bases = 300_000
+    p = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--bases", str(bases),
+                        "--cpu-sample", str(bases), "--steps", "2", "--warmup", "0", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600)
+    assert p.returncode == 0, p.stderr[-3000:]
+    assert json.loads(p.stdout.strip().splitlines()[-1])["steps"] == 2
+    text_len, starts = bench.record_layout(bases)
+    text = bench.synth_prefix_numpy(bases, text_len, starts)[:-1] + b"$"  # the arm's prefix of the workload text
+    want = O.oracle_build(text, is_dna=True, index_bits=64)
+    d = {f.stem: np.load(f) for f in tmp_path.glob("*.npy")}
+    assert d["sizes"].tolist() == [want.num_suffixes, len(text)]
+    assert d["ranks"].tolist() == list(range(want.num_suffixes))
+    assert np.array_equal(d["sa"], want.sa.astype(np.float64))
+    assert np.array_equal(d["lcp"], want.lcp.astype(np.float64))
+    assert np.array_equal(d["text"], np.frombuffer(text, np.uint8).astype(np.float32))
+
+
 def test_distributed_meta_logic():
     from sufr_b200.distributed import previous_last_suffix, shard_layout
     meta = [(0, 0, 0), (5, 10, 11), (0, 0, 0), (7, 3, 4), (2, 8, 9)]
@@ -372,9 +394,13 @@ print("ok", rank)
 
 def test_distributed_gloo_world2(tmp_path):
     """N>1 host logic under torch.distributed (gloo, 2 processes, CPU)."""
+    import socket
     script = tmp_path / "w.py"
     script.write_text(GLOO_WORKER)
-    env = dict(os.environ, MASTER_ADDR="127.0.0.1", MASTER_PORT="29613", WORLD_SIZE="2")
+    with socket.socket() as s:  # a free port: a fixed one collides with another run on the same host
+        s.bind(("127.0.0.1", 0))
+        port = s.getsockname()[1]
+    env = dict(os.environ, MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), WORLD_SIZE="2")
     procs = [subprocess.Popen([sys.executable, str(script), str(ROOT)], env=dict(env, RANK=str(r)),
                               stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True) for r in range(2)]
     outs = [p.communicate(timeout=180)[0] for p in procs]
