@@ -162,7 +162,8 @@ int sufr_b200_verify(SufrB200Ctx* ctx, const SufrB200Args* args, const SufrB200R
                      uint64_t prev_last_suffix, SufrB200VerifyReport* out);
 
 /* -- the consumer of the LCP array (SURVEY 8(f) rank 4): LCP-subsampled suffix array + batched search over a
- *    device-resident index.  An index borrows text / SA / LCP of a DEVICE result, which must outlive it.
+ *    device-resident index.  An index made by index_create borrows text / SA / LCP of a DEVICE result, which must
+ *    outlive it; one made by index_open (below) owns copies read from a `.sufr` file.
  *      subsample  SufrFile::subsample_suffix_array (sufr_file.rs:429-456): the entries with lcp < max_query_len and
  *                 their ranks ("compressed" in-memory suffix array)
  *      search     SufrSearch::search (sufr_search.rs:104-350) for a batch of queries, one GPU thread per query:
@@ -180,6 +181,52 @@ int sufr_b200_index_search(SufrB200Index* index, const uint8_t* queries, const u
                            uint64_t* rank_end);
 int sufr_b200_index_suffixes(SufrB200Index* index, uint64_t rank_begin, uint64_t count, uint64_t* out);
 void sufr_b200_index_free(SufrB200Index* index);
+
+/* -- the read side of a `.sufr` file (SufrFile::read, sufr_file.rs:145-275), version 6 only.
+ *    file_info  header, sequence starts, seed mask and names, validated (host only, no device needed): the sections
+ *               must follow each other without gaps up to exactly the end of the file, element width 4 or 8
+ *               ((lcp_pos - sa_pos) / num_suffixes), num_suffixes <= text_len, sequence starts strictly increasing
+ *               and below text_len, mask bytes 0 / 1 forming a valid mask.  A file that fails a check gives
+ *               SUFR_B200_ERR_IO ("{path}: invalid .sufr file: ..."); a version other than 6 SUFR_B200_ERR_UNSUPPORTED.
+ *    index_open an index that OWNS device copies of text, suffix array, LCP array and sequence starts (host threads
+ *               pread the file into pinned buffers that are copied to the device as they fill).  Every suffix array
+ *               entry is checked to be below text_len on the device before the index is returned.
+ *    index_locate  index_search + per-query hit offsets: hit_offsets[num_queries + 1] (exclusive scan of the counts).
+ *               low_memory == 0 searches the LCP-subsampled array when the effective max_query_len is shorter than
+ *               the build's (sufr_file.rs:514-560; the subsample is made and kept as needed, replacing one of
+ *               another max_query_len that index_subsample made), low_memory != 0 the full array.  Ranges and offsets stay on the device for index_hits.
+ *    index_hits hits [first_hit, first_hit + count) of the last index_locate, in query order and rank order within a
+ *               query: suffix = SA[rank], sequence = index of the record holding it, sequence_pos = suffix - its
+ *               start.  An index without sequence starts gives sequence = UINT64_MAX and sequence_pos = suffix.
+ *               Any of the three outputs may be NULL.  A window beyond the total is SUFR_B200_ERR_ARGUMENT.
+ *    An index made by index_create takes its sequence starts from args (none when args->num_sequences == 0). */
+typedef struct SufrB200FileInfo {
+    uint32_t version;
+    uint32_t index_bits;          /* 32 or 64: width of SA / LCP entries and sequence starts in the file */
+    uint8_t is_dna;
+    uint8_t allow_ambiguity;
+    uint8_t ignore_softmask;
+    uint8_t reserved[5];
+    uint64_t text_len;
+    uint64_t num_suffixes;
+    uint64_t max_query_len;       /* of the build; 0 = none (always 0 with a seed mask) */
+    uint64_t num_sequences;
+    uint64_t text_pos;
+    uint64_t sa_pos;
+    uint64_t lcp_pos;
+    uint64_t file_bytes;
+    char* seed_mask;              /* NULL = none, else "1101..." */
+    uint64_t* sequence_starts;    /* num_sequences entries */
+    char** sequence_names;        /* num_sequences NUL-terminated strings */
+} SufrB200FileInfo;
+int sufr_b200_file_info(const char* path, SufrB200FileInfo* out);
+void sufr_b200_file_info_free(SufrB200FileInfo* info);
+int sufr_b200_index_open(SufrB200Ctx* ctx, const char* path, SufrB200Index** out);
+int sufr_b200_index_locate(SufrB200Index* index, const uint8_t* queries, const uint64_t* offsets, uint64_t num_queries,
+                           int has_max_query_len, uint64_t max_query_len, int low_memory, uint64_t* rank_begin,
+                           uint64_t* rank_end, uint64_t* hit_offsets);
+int sufr_b200_index_hits(SufrB200Index* index, uint64_t first_hit, uint64_t count, uint64_t* suffix, uint64_t* sequence,
+                         uint64_t* sequence_pos);
 
 /* -- write: replaces SufrBuilder::write (sufr_builder.rs:817-918), version-6 `.sufr` layout.
  *    Single shard: writes the whole file.  Sharded: every rank calls it with the same path; rank 0

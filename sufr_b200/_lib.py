@@ -111,13 +111,37 @@ class Sequences(C.Structure):
     ]
 
 
+class FileInfo(C.Structure):
+    """struct SufrB200FileInfo"""
+    _fields_ = [
+        ("version", C.c_uint32),
+        ("index_bits", C.c_uint32),
+        ("is_dna", C.c_uint8),
+        ("allow_ambiguity", C.c_uint8),
+        ("ignore_softmask", C.c_uint8),
+        ("reserved", C.c_uint8 * 5),
+        ("text_len", C.c_uint64),
+        ("num_suffixes", C.c_uint64),
+        ("max_query_len", C.c_uint64),
+        ("num_sequences", C.c_uint64),
+        ("text_pos", C.c_uint64),
+        ("sa_pos", C.c_uint64),
+        ("lcp_pos", C.c_uint64),
+        ("file_bytes", C.c_uint64),
+        ("seed_mask", C.c_char_p),
+        ("sequence_starts", C.POINTER(C.c_uint64)),
+        ("sequence_names", C.POINTER(C.c_char_p)),
+    ]
+
+
 # every symbol include/sufr_b200.h declares (tests check that the library exports all of them)
 ABI_SYMBOLS = [
     "sufr_b200_ctx_create", "sufr_b200_ctx_destroy", "sufr_b200_ctx_reserve", "sufr_b200_ctx_trim",
     "sufr_b200_build", "sufr_b200_result_free", "sufr_b200_patch_seam", "sufr_b200_verify", "sufr_b200_write",
     "sufr_b200_create", "sufr_b200_create_multi",
     "sufr_b200_index_create", "sufr_b200_index_subsample", "sufr_b200_index_search", "sufr_b200_index_suffixes",
-    "sufr_b200_index_free",
+    "sufr_b200_index_free", "sufr_b200_file_info", "sufr_b200_file_info_free", "sufr_b200_index_open",
+    "sufr_b200_index_locate", "sufr_b200_index_hits",
     "sufr_b200_seed_mask", "sufr_b200_find_lcp_full_offset", "sufr_b200_read_sequence_file",
     "sufr_b200_sequences_free", "sufr_b200_synth_dna", "sufr_b200_last_error", "sufr_b200_abi_version",
     "sufr_b200_device_count",
@@ -176,6 +200,17 @@ def lib():
     L.sufr_b200_index_suffixes.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p]
     L.sufr_b200_index_free.restype = None
     L.sufr_b200_index_free.argtypes = [C.c_void_p]
+    L.sufr_b200_file_info.restype = C.c_int
+    L.sufr_b200_file_info.argtypes = [C.c_char_p, C.POINTER(FileInfo)]
+    L.sufr_b200_file_info_free.restype = None
+    L.sufr_b200_file_info_free.argtypes = [C.POINTER(FileInfo)]
+    L.sufr_b200_index_open.restype = C.c_int
+    L.sufr_b200_index_open.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(C.c_void_p)]
+    L.sufr_b200_index_locate.restype = C.c_int
+    L.sufr_b200_index_locate.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_uint64, C.c_int,
+                                         C.c_void_p, C.c_void_p, C.c_void_p]
+    L.sufr_b200_index_hits.restype = C.c_int
+    L.sufr_b200_index_hits.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]
     L.sufr_b200_seed_mask.restype = C.c_int64
     L.sufr_b200_seed_mask.argtypes = [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.sufr_b200_find_lcp_full_offset.restype = C.c_uint64

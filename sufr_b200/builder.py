@@ -332,21 +332,64 @@ def build(args: SufrBuilderArgs, *, index_bits: int = 0, ctx: Optional[Context] 
     return BuildResult(ctx, cargs, res)
 
 
+def file_info(path) -> dict:
+    """Header, sequence starts / names and seed mask of a version-6 `.sufr` file, validated (sufr_b200_file_info;
+    host only).  Raises SufrError (ERR_IO for a malformed file, ERR_UNSUPPORTED for another version)."""
+    fi = _lib.FileInfo()
+    _check(_lib.lib().sufr_b200_file_info(str(path).encode(), C.byref(fi)))
+    try:
+        n = int(fi.num_sequences)
+        return {"version": int(fi.version), "index_bits": int(fi.index_bits), "is_dna": bool(fi.is_dna),
+                "allow_ambiguity": bool(fi.allow_ambiguity), "ignore_softmask": bool(fi.ignore_softmask),
+                "text_len": int(fi.text_len), "num_suffixes": int(fi.num_suffixes),
+                "max_query_len": int(fi.max_query_len), "num_sequences": n, "text_pos": int(fi.text_pos),
+                "sa_pos": int(fi.sa_pos), "lcp_pos": int(fi.lcp_pos), "file_bytes": int(fi.file_bytes),
+                "seed_mask": fi.seed_mask.decode() if fi.seed_mask else None,
+                "sequence_starts": [int(fi.sequence_starts[i]) for i in range(n)],
+                "sequence_names": [fi.sequence_names[i].decode(errors="replace") for i in range(n)]}
+    finally:
+        _lib.lib().sufr_b200_file_info_free(C.byref(fi))
+
+
 class SufrIndex:
-    """Device-resident index over a DEVICE build result: the read side that consumes the LCP array
-    (``SufrFile::subsample_suffix_array`` sufr_file.rs:429-456, ``suffix_search`` :777-836, ``locate`` :1132-1169,
-    ``SufrSearch`` sufr_search.rs:104-350).  ``count`` / ``locate`` take a batch of queries; one GPU thread each."""
+    """Device-resident index: the read side that consumes the LCP array (``SufrFile::subsample_suffix_array``
+    sufr_file.rs:429-456, ``suffix_search`` :777-836, ``locate`` :1132-1169, ``SufrSearch`` sufr_search.rs:104-350).
+    ``count`` / ``locate`` take a batch of queries; one GPU thread each.
+
+    ``SufrIndex(result, args)`` borrows the arrays of a DEVICE build result; ``SufrIndex.open(path)`` reads a `.sufr`
+    file into device memory the index owns (``.info`` holds its header, names, starts and mask)."""
+
+    HITS_WINDOW = 1 << 24  # hits fetched per sufr_b200_index_hits call: bounds device memory for very frequent queries
 
     def __init__(self, result: "BuildResult", args: SufrBuilderArgs):
-        self._res, self._args = result, args
+        self._res, self._args, self._ctx = result, args, result._ctx
+        self.info = None
         self._h = C.c_void_p()
         _check(_lib.lib().sufr_b200_index_create(result._ctx.handle, C.byref(result._cargs.c), C.byref(result.c),
                                                  C.byref(self._h)))
         self._sub_mql = None
+        self._names = list(args.sequence_names)
         if args.seed_mask is not None:
             self._built = SeedMask.new(args.seed_mask).weight        # sufr_file.rs:528
         else:
             self._built = args.max_query_len or result.text_len       # sufr_file.rs:521-527
+
+    @classmethod
+    def open(cls, path, ctx: Optional[Context] = None, device: int = 0) -> "SufrIndex":
+        """SufrFile::read + the in-memory arrays (sufr_file.rs:145-275) on the GPU: sufr_b200_index_open."""
+        self = cls.__new__(cls)
+        self._h = C.c_void_p()
+        self._res, self._args = None, None
+        self._ctx = ctx or default_context(device)
+        self.info = file_info(path)
+        _check(_lib.lib().sufr_b200_index_open(self._ctx.handle, str(path).encode(), C.byref(self._h)))
+        self._sub_mql = None
+        self._names = self.info["sequence_names"]
+        if self.info["seed_mask"] is not None:
+            self._built = SeedMask.new(self.info["seed_mask"]).weight
+        else:
+            self._built = self.info["max_query_len"] or self.info["text_len"]
+        return self
 
     def close(self):
         if self._h:
@@ -365,6 +408,14 @@ class SufrIndex:
         self._sub_mql = max_query_len
         return int(kept.value)
 
+    def _subsample_mql(self, max_query_len, low_memory):
+        """set_suffix_array_mem (sufr_file.rs:514-560): the max_query_len of the LCP-subsampled array a search in this
+        mode uses, or None when it searches the full array.  sufr_b200_index_locate makes the same choice."""
+        if low_memory:
+            return None
+        eff = min(max_query_len, self._built) if max_query_len else self._built
+        return eff if eff != self._built else None
+
     def search(self, queries: Sequence[str], max_query_len: Optional[int] = None, low_memory: bool = False):
         """SufrFile::suffix_search: per query the half-open rank range in the full suffix array, or None.
         low_memory=False mirrors set_suffix_array_mem (sufr_file.rs:514-560): when the effective max_query_len is
@@ -373,13 +424,10 @@ class SufrIndex:
         offs = np.zeros(len(qs) + 1, dtype=np.uint64)
         offs[1:] = np.cumsum([len(q) for q in qs])
         blob = np.frombuffer(b"".join(qs) or b"\0", dtype=np.uint8)
-        use_sub = 0
-        if not low_memory:
-            eff = min(max_query_len, self._built) if max_query_len else self._built
-            if eff != self._built:
-                if self._sub_mql != eff:
-                    self.subsample(eff)
-                use_sub = 1
+        eff = self._subsample_mql(max_query_len, low_memory)
+        if eff is not None and self._sub_mql != eff:
+            self.subsample(eff)
+        use_sub = int(eff is not None)
         b = np.zeros(max(1, len(qs)), dtype=np.uint64)
         e = np.zeros(max(1, len(qs)), dtype=np.uint64)
         _check(_lib.lib().sufr_b200_index_search(self._h, blob.ctypes.data, offs.ctypes.data, len(qs),
@@ -396,18 +444,52 @@ class SufrIndex:
         _check(_lib.lib().sufr_b200_index_suffixes(self._h, rank_begin, count, out.ctypes.data))
         return out[:count]
 
+    def locate_ranges(self, queries, max_query_len=None, low_memory=False):
+        """sufr_b200_index_locate: (rank_begin, rank_end, hit_offsets) as numpy arrays; hits of query i are
+        hit_offsets[i] .. hit_offsets[i + 1] in :meth:`hits`.  Absent queries have rank_begin == rank_end == 2**64-1.
+        low_memory=False searches the LCP-subsampled array when the effective max_query_len is shorter than the
+        build's (sufr_file.rs:514-560), as :meth:`search` does."""
+        qs = [q.encode() if isinstance(q, str) else bytes(q) for q in queries]
+        offs = np.zeros(len(qs) + 1, dtype=np.uint64)
+        offs[1:] = np.cumsum([len(q) for q in qs])
+        blob = np.frombuffer(b"".join(qs) or b"\0", dtype=np.uint8)
+        b = np.zeros(max(1, len(qs)), dtype=np.uint64)
+        e = np.zeros(max(1, len(qs)), dtype=np.uint64)
+        ho = np.zeros(len(qs) + 1, dtype=np.uint64)
+        # the library replaces the index's subsample when this mode needs another one: keep the cache of search() true
+        eff = self._subsample_mql(max_query_len, low_memory)
+        if eff is not None:
+            self._sub_mql = None
+        _check(_lib.lib().sufr_b200_index_locate(self._h, blob.ctypes.data, offs.ctypes.data, len(qs),
+                                                 int(max_query_len is not None), int(max_query_len or 0),
+                                                 int(low_memory), b.ctypes.data, e.ctypes.data, ho.ctypes.data))
+        if eff is not None:
+            self._sub_mql = eff
+        return b[:len(qs)], e[:len(qs)], ho
+
+    def hits(self, first: int, count: int):
+        """sufr_b200_index_hits: (suffix, sequence, sequence_pos) of hits [first, first + count) of the last locate."""
+        suf = np.zeros(max(1, count), dtype=np.uint64)
+        seq = np.zeros(max(1, count), dtype=np.uint64)
+        pos = np.zeros(max(1, count), dtype=np.uint64)
+        _check(_lib.lib().sufr_b200_index_hits(self._h, first, count, suf.ctypes.data, seq.ctypes.data,
+                                               pos.ctypes.data))
+        return suf[:count], seq[:count], pos[:count]
+
     def locate(self, queries, max_query_len=None, low_memory=False):
-        """SufrFile::locate: per query a list of (rank, suffix, sequence_name, sequence_position) in rank order."""
-        import bisect
-        starts, names = list(self._args.sequence_starts), list(self._args.sequence_names)
+        """SufrFile::locate: per query a list of (rank, suffix, sequence_name, sequence_position) in rank order
+        (name None and position = suffix for an index without sequence starts)."""
+        b, _, ho = self.locate_ranges(queries, max_query_len, low_memory)
+        total = int(ho[-1])
+        parts = [self.hits(f, min(self.HITS_WINDOW, total - f)) for f in range(0, total, self.HITS_WINDOW)]
+        suf = np.concatenate([p[0] for p in parts]).tolist() if parts else []
+        seq = np.concatenate([p[1] for p in parts]).tolist() if parts else []
+        pos = np.concatenate([p[2] for p in parts]).tolist() if parts else []
+        names, none = self._names, 0xFFFFFFFFFFFFFFFF
         out = []
-        for r in self.search(queries, max_query_len, low_memory):
-            hits = []
-            if r is not None:
-                for k, suf in enumerate(self.suffixes(r[0], r[1] - r[0]).tolist()):
-                    i = bisect.bisect_right(starts, suf) - 1
-                    hits.append((r[0] + k, suf, names[i], suf - starts[i]))
-            out.append(hits)
+        for i in range(len(b)):
+            lo, hi, r0 = int(ho[i]), int(ho[i + 1]), int(b[i])
+            out.append([(r0 + k - lo, suf[k], None if seq[k] == none else names[seq[k]], pos[k]) for k in range(lo, hi)])
         return out
 
 

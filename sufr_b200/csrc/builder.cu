@@ -277,6 +277,70 @@ static int guarded(F&& f) {
     }
 }
 
+// A ring of pinned host buffers, each with an event that marks the end of the last copy that used it.  Shared by the
+// two directions of the file path: StreamWriter (device -> slot -> file) and upload_file_sections (file -> slot ->
+// device).  acquire() blocks until a slot is free and returns -1 once abort() has been called.
+class PinnedSlots {
+   public:
+    PinnedSlots(size_t slot_bytes, int nslots) : slot_bytes_(slot_bytes) {
+        try {
+            for (int i = 0; i < nslots; i++) {
+                slots_.push_back(Slot{nullptr, nullptr});
+                SUFR_CUDA_CHECK(cudaMallocHost(&slots_.back().buf, slot_bytes_));
+                SUFR_CUDA_CHECK(cudaEventCreateWithFlags(&slots_.back().ev, cudaEventDisableTiming));
+                free_.push_back(i);
+            }
+        } catch (...) {  // a constructor that throws runs no destructor: release what was allocated
+            release();
+            throw;
+        }
+    }
+    ~PinnedSlots() { release(); }
+    PinnedSlots(const PinnedSlots&) = delete;
+    PinnedSlots& operator=(const PinnedSlots&) = delete;
+    size_t slot_bytes() const { return slot_bytes_; }
+    void* buf(int i) const { return slots_[i].buf; }
+    cudaEvent_t event(int i) const { return slots_[i].ev; }
+    int acquire() {
+        std::unique_lock<std::mutex> lock(mu_);
+        cv_.wait(lock, [&] { return !free_.empty() || aborted_; });
+        if (aborted_) return -1;
+        const int i = free_.front();
+        free_.pop_front();
+        return i;
+    }
+    void put(int i) {
+        {
+            std::lock_guard<std::mutex> lock(mu_);
+            free_.push_back(i);
+        }
+        cv_.notify_one();
+    }
+    void abort() {
+        {
+            std::lock_guard<std::mutex> lock(mu_);
+            aborted_ = true;
+        }
+        cv_.notify_all();
+    }
+
+   private:
+    struct Slot { void* buf; cudaEvent_t ev; };
+    void release() {
+        for (auto& sl : slots_) {
+            if (sl.buf) cudaFreeHost(sl.buf);
+            if (sl.ev) cudaEventDestroy(sl.ev);
+        }
+        slots_.clear();
+    }
+    size_t slot_bytes_;
+    std::vector<Slot> slots_;
+    std::deque<int> free_;
+    std::mutex mu_;
+    std::condition_variable cv_;
+    bool aborted_ = false;
+};
+
 // sufr_b200_create: the sections of the file go from device memory to the file through a small ring of pinned
 // buffers -- the device->host copy of one chunk overlaps the pwrite of the previous ones, and no host copy of the
 // suffix / LCP arrays is ever allocated (page-locking 2 * s * sizeof(T) bytes costs seconds by itself).
@@ -284,40 +348,24 @@ class StreamWriter {
    public:
     StreamWriter(OutputFile& file, int device, cudaStream_t stream, size_t slot_bytes = 64u << 20, int nslots = 6,
                  int nworkers = 4)
-        : file_(file), device_(device), stream_(stream), slot_bytes_(slot_bytes) {
-        try {
-            for (int i = 0; i < nslots; i++) {
-                Slot sl{nullptr, nullptr};
-                SUFR_CUDA_CHECK(cudaMallocHost(&sl.buf, slot_bytes_));
-                slots_.push_back(sl);
-                SUFR_CUDA_CHECK(cudaEventCreateWithFlags(&slots_.back().ev, cudaEventDisableTiming));
-                free_.push_back(i);
-            }
-        } catch (...) {  // a constructor that throws runs no destructor: release what was allocated
-            release_slots();
-            throw;
-        }
+        : file_(file), device_(device), stream_(stream), slots_(slot_bytes, nslots) {
         for (int i = 0; i < nworkers; i++) workers_.emplace_back([this] { work(); });
     }
     ~StreamWriter() {
         try { finish(); } catch (...) {}
-        release_slots();
     }
     // Queue `len` bytes of device memory for file offset `off`; `host_copy` (optional) also receives them.
     void submit(const void* dev, size_t len, uint64_t off, uint8_t* host_copy = nullptr) {
         const char* p = (const char*)dev;
         while (len) {
-            const size_t chunk = std::min(len, slot_bytes_);
-            int slot;
-            {
-                std::unique_lock<std::mutex> lock(mu_);
-                cv_free_.wait(lock, [&] { return !free_.empty() || err_; });
-                if (err_) std::rethrow_exception(err_);
-                slot = free_.front();
-                free_.pop_front();
+            const size_t chunk = std::min(len, slots_.slot_bytes());
+            const int slot = slots_.acquire();
+            if (slot < 0) {
+                std::lock_guard<std::mutex> lock(mu_);
+                std::rethrow_exception(err_);
             }
-            SUFR_CUDA_CHECK(cudaMemcpyAsync(slots_[slot].buf, p, chunk, cudaMemcpyDeviceToHost, stream_));
-            SUFR_CUDA_CHECK(cudaEventRecord(slots_[slot].ev, stream_));
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(slots_.buf(slot), p, chunk, cudaMemcpyDeviceToHost, stream_));
+            SUFR_CUDA_CHECK(cudaEventRecord(slots_.event(slot), stream_));
             {
                 std::lock_guard<std::mutex> lock(mu_);
                 jobs_.push_back({slot, chunk, off, host_copy});
@@ -344,15 +392,7 @@ class StreamWriter {
     uint64_t bytes() const { return bytes_; }
 
    private:
-    struct Slot { void* buf; cudaEvent_t ev; };
     struct Job { int slot; size_t len; uint64_t off; uint8_t* host_copy; };
-    void release_slots() {
-        for (auto& sl : slots_) {
-            if (sl.buf) cudaFreeHost(sl.buf);
-            if (sl.ev) cudaEventDestroy(sl.ev);
-        }
-        slots_.clear();
-    }
     void work() {
         cudaSetDevice(device_);
         for (;;) {
@@ -365,35 +405,91 @@ class StreamWriter {
                 jobs_.pop_front();
             }
             try {
-                cudaError_t e = cudaEventSynchronize(slots_[j.slot].ev);
+                cudaError_t e = cudaEventSynchronize(slots_.event(j.slot));
                 if (e != cudaSuccess) throw Error(100 + (int)e, std::string("CUDA error in the file writer: ") + cudaGetErrorString(e));
-                if (j.host_copy) memcpy(j.host_copy, slots_[j.slot].buf, j.len);
-                file_.write(j.off, slots_[j.slot].buf, j.len);
+                if (j.host_copy) memcpy(j.host_copy, slots_.buf(j.slot), j.len);
+                file_.write(j.off, slots_.buf(j.slot), j.len);
             } catch (...) {
-                std::lock_guard<std::mutex> lock(mu_);
-                if (!err_) err_ = std::current_exception();
+                {
+                    std::lock_guard<std::mutex> lock(mu_);
+                    if (!err_) err_ = std::current_exception();
+                }
+                slots_.abort();
             }
-            {
-                std::lock_guard<std::mutex> lock(mu_);
-                free_.push_back(j.slot);
-            }
-            cv_free_.notify_one();
+            slots_.put(j.slot);
         }
     }
     OutputFile& file_;
     int device_;
     cudaStream_t stream_;
-    size_t slot_bytes_;
-    std::vector<Slot> slots_;
-    std::deque<int> free_;
+    PinnedSlots slots_;
     std::deque<Job> jobs_;
     std::vector<std::thread> workers_;
     std::mutex mu_;
-    std::condition_variable cv_free_, cv_work_;
+    std::condition_variable cv_work_;
     bool done_ = false;
     std::exception_ptr err_;
     uint64_t bytes_ = 0;
 };
+
+// sufr_b200_index_open, the mirror of StreamWriter: host threads pread chunks of the file into the pinned slots and
+// queue each slot's host->device copy on the context's stream.  A slot is refilled once the event recorded behind its
+// last copy has completed, so reads, copies and the other threads' reads overlap.  Returns after a synchronise.
+struct FileSection {
+    uint64_t file_off;
+    uint64_t len;
+    void* dev;
+};
+static void upload_file_sections(int fd, const std::string& path, int device, cudaStream_t stream,
+                                 const std::vector<FileSection>& sections) {
+    const size_t slot_bytes = 32u << 20;
+    struct Chunk { uint64_t file_off; size_t len; char* dev; };
+    std::vector<Chunk> chunks;
+    for (const auto& s : sections)
+        for (uint64_t o = 0; o < s.len; o += slot_bytes)
+            chunks.push_back({s.file_off + o, (size_t)std::min<uint64_t>(slot_bytes, s.len - o), (char*)s.dev + o});
+    if (chunks.empty()) return;
+    const int hw = std::max(2, (int)std::thread::hardware_concurrency());
+    const int readers = std::min<int>(std::min(16, hw), (int)chunks.size());
+    PinnedSlots slots(slot_bytes, readers + 4);
+    std::atomic<size_t> next{0};
+    std::mutex err_mu;
+    std::exception_ptr err;
+    auto work = [&]() {
+        try {
+            SUFR_CUDA_CHECK(cudaSetDevice(device));
+            for (;;) {
+                const size_t c = next.fetch_add(1);
+                if (c >= chunks.size()) return;
+                const int slot = slots.acquire();
+                if (slot < 0) return;
+                try {
+                    SUFR_CUDA_CHECK(cudaEventSynchronize(slots.event(slot)));  // the slot's previous copy is done
+                    pread_all(fd, slots.buf(slot), chunks[c].len, chunks[c].file_off, path);
+                    SUFR_CUDA_CHECK(cudaMemcpyAsync(chunks[c].dev, slots.buf(slot), chunks[c].len, cudaMemcpyHostToDevice, stream));
+                    SUFR_CUDA_CHECK(cudaEventRecord(slots.event(slot), stream));
+                } catch (...) {
+                    slots.put(slot);
+                    throw;
+                }
+                slots.put(slot);
+            }
+        } catch (...) {
+            {
+                std::lock_guard<std::mutex> lock(err_mu);
+                if (!err) err = std::current_exception();
+            }
+            slots.abort();
+        }
+    };
+    std::vector<std::thread> pool;
+    for (int t = 1; t < readers; t++) pool.emplace_back(work);
+    work();
+    for (auto& th : pool) th.join();
+    const cudaError_t e = cudaStreamSynchronize(stream);  // before the slots are released
+    if (err) std::rethrow_exception(err);
+    SUFR_CUDA_CHECK(e);
+}
 
 // Writes the file of a DEVICE result (sufr_builder.rs:817-918) and returns the transformed text in `host_text`
 // (malloc; what SufrBuilder.text holds after `new`).
@@ -763,9 +859,44 @@ struct SufrB200Index {
     uint32_t weight = 0, mask_len = 0;
     DevBuf<uint32_t> maskpos;
     DevBuf<unsigned char> sub_sa, sub_rank;
-    uint64_t sub_len = 0;
+    uint64_t sub_len = 0, sub_mql = 0;
     bool has_sub = false;
+    // an index opened from a file owns its arrays (text / sa / lcp above point into these)
+    DevBuf<unsigned char> own_text, own_sa, own_lcp;
+    // sequence starts (u64) for locate; num_starts == 0: none
+    DevBuf<unsigned long long> starts;
+    uint64_t num_starts = 0;
+    // the last sufr_b200_index_locate: rank ranges and hit offsets of its queries, for sufr_b200_index_hits
+    DevBuf<unsigned long long> loc_begin, loc_end, loc_offsets;
+    uint64_t loc_queries = 0, loc_hits = 0;
+    bool has_loc = false;
+    // max_query_len the index was built with, as sufr_file.rs:521-528 defines it: the mask weight, else the build's
+    // max_query_len, else the text length
+    uint64_t built_mql() const { return is_mask ? weight : (build_mql ? build_mql : n); }
 };
+
+static void index_set_mask(SufrB200Index& idx, Ctx& ctx, const char* seed_mask, bool has_mql, uint64_t mql) {
+    SeedMaskInfo mask;
+    if (seed_mask && parse_seed_mask(seed_mask, mask)) {
+        idx.is_mask = true;
+        idx.weight = (uint32_t)mask.weight;
+        idx.mask_len = (uint32_t)mask.bytes.size();
+        std::vector<uint32_t> mp(mask.positions.begin(), mask.positions.end());
+        idx.maskpos = DevBuf<uint32_t>(ctx.pool, mp.size());
+        SUFR_CUDA_CHECK(cudaMemcpyAsync(idx.maskpos.get(), mp.data(), mp.size() * 4, cudaMemcpyHostToDevice, ctx.stream));
+        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+    } else {
+        idx.build_mql = has_mql ? mql : 0;
+    }
+}
+
+static void index_set_starts(SufrB200Index& idx, Ctx& ctx, const uint64_t* starts, uint64_t count) {
+    idx.num_starts = count;
+    if (!count) return;
+    idx.starts = DevBuf<unsigned long long>(ctx.pool, count);
+    SUFR_CUDA_CHECK(cudaMemcpyAsync(idx.starts.get(), starts, count * 8, cudaMemcpyHostToDevice, ctx.stream));
+    SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+}
 
 int sufr_b200_index_create(SufrB200Ctx* c, const SufrB200Args* args, const SufrB200Result* r, SufrB200Index** out) {
     return guarded([&] {
@@ -782,41 +913,39 @@ int sufr_b200_index_create(SufrB200Ctx* c, const SufrB200Args* args, const SufrB
         idx->n = r->text_len;
         idx->s = r->num_suffixes;
         idx->wide = r->index_bits == 64;
-        SeedMaskInfo mask;
-        if (args->seed_mask && parse_seed_mask(args->seed_mask, mask)) {
-            std::lock_guard<std::mutex> lock(ctx->mu);
-            SUFR_CUDA_CHECK(cudaSetDevice(ctx->device));
-            idx->is_mask = true;
-            idx->weight = (uint32_t)mask.weight;
-            idx->mask_len = (uint32_t)mask.bytes.size();
-            std::vector<uint32_t> mp(mask.positions.begin(), mask.positions.end());
-            idx->maskpos = DevBuf<uint32_t>(ctx->pool, mp.size());
-            SUFR_CUDA_CHECK(cudaMemcpyAsync(idx->maskpos.get(), mp.data(), mp.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-            SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
-        } else {
-            idx->build_mql = args->has_max_query_len ? args->max_query_len : 0;
-        }
+        if (args->num_sequences && !args->sequence_starts) throw Error(SUFR_B200_ERR_ARGUMENT, "sequence_starts is NULL");
+        std::lock_guard<std::mutex> lock(ctx->mu);
+        SUFR_CUDA_CHECK(cudaSetDevice(ctx->device));
+        index_set_mask(*idx, *ctx, args->seed_mask, args->has_max_query_len, args->max_query_len);
+        index_set_starts(*idx, *ctx, args->sequence_starts, args->num_sequences);
         *out = idx.release();
     });
 }
 
 void sufr_b200_index_free(SufrB200Index* idx) {
     if (!idx) return;
+    DeviceRestore restore;
     {
         std::lock_guard<std::mutex> lock(idx->ctx->mu);
+        cudaSetDevice(idx->ctx->device);
+        cudaStreamSynchronize(idx->ctx->stream);
         idx->maskpos.reset();
         idx->sub_sa.reset();
         idx->sub_rank.reset();
+        idx->own_text.reset();
+        idx->own_sa.reset();
+        idx->own_lcp.reset();
+        idx->starts.reset();
+        idx->loc_begin.reset();
+        idx->loc_end.reset();
+        idx->loc_offsets.reset();
     }
     delete idx;
 }
 
-int sufr_b200_index_subsample(SufrB200Index* idx, uint64_t max_query_len, uint64_t* kept) {
-    return guarded([&] {
-        if (!idx) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+// with the context's lock held
+static uint64_t index_subsample_locked(SufrB200Index* idx, uint64_t max_query_len) {
         Ctx& ctx = *idx->ctx;
-        std::lock_guard<std::mutex> lock(ctx.mu);
-        SUFR_CUDA_CHECK(cudaSetDevice(ctx.device));
         idx->sub_sa.reset();
         idx->sub_rank.reset();
         idx->has_sub = false;
@@ -838,9 +967,39 @@ int sufr_b200_index_subsample(SufrB200Index* idx, uint64_t max_query_len, uint64
             SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
         }
         idx->sub_len = total;
+        idx->sub_mql = max_query_len;
         idx->has_sub = true;
+        return total;
+}
+
+int sufr_b200_index_subsample(SufrB200Index* idx, uint64_t max_query_len, uint64_t* kept) {
+    return guarded([&] {
+        if (!idx) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        std::lock_guard<std::mutex> lock(idx->ctx->mu);
+        SUFR_CUDA_CHECK(cudaSetDevice(idx->ctx->device));
+        const uint64_t total = index_subsample_locked(idx, max_query_len);
         if (kept) *kept = total;
     });
+}
+
+static void launch_search(SufrB200Index* idx, const uint8_t* d_q, const uint64_t* d_off, uint64_t nq, int has_mql,
+                          uint64_t mql, int use_subsample, unsigned long long* d_b, unsigned long long* d_e) {
+    search::Params P{};
+    P.text = idx->text;
+    P.n = idx->n;
+    P.sa = use_subsample ? (const void*)idx->sub_sa.get() : idx->sa;
+    P.rank = use_subsample ? (const void*)idx->sub_rank.get() : nullptr;
+    P.len = use_subsample ? idx->sub_len : idx->s;
+    P.wide = idx->wide;
+    P.is_mask = idx->is_mask;
+    P.build_mql = idx->build_mql;
+    P.has_run_mql = has_mql ? 1 : 0;
+    P.run_mql = mql;
+    P.mask_pos = idx->maskpos.get();
+    P.weight = idx->weight;
+    P.mask_len = idx->mask_len;
+    search::search_kernel<<<(unsigned)div_up(nq, 128), 128, 0, idx->ctx->stream>>>(P, d_q, d_off, nq, d_b, d_e);
+    SUFR_KERNEL_CHECK();
 }
 
 int sufr_b200_index_search(SufrB200Index* idx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq, int has_mql,
@@ -858,22 +1017,7 @@ int sufr_b200_index_search(SufrB200Index* idx, const uint8_t* queries, const uin
         DevBuf<unsigned long long> d_b(ctx.pool, nq), d_e(ctx.pool, nq);
         if (bytes) SUFR_CUDA_CHECK(cudaMemcpyAsync(d_q.get(), queries, bytes, cudaMemcpyHostToDevice, ctx.stream));
         SUFR_CUDA_CHECK(cudaMemcpyAsync(d_off.get(), offsets, (nq + 1) * 8, cudaMemcpyHostToDevice, ctx.stream));
-        search::Params P{};
-        P.text = idx->text;
-        P.n = idx->n;
-        P.sa = use_subsample ? (const void*)idx->sub_sa.get() : idx->sa;
-        P.rank = use_subsample ? (const void*)idx->sub_rank.get() : nullptr;
-        P.len = use_subsample ? idx->sub_len : idx->s;
-        P.wide = idx->wide;
-        P.is_mask = idx->is_mask;
-        P.build_mql = idx->build_mql;
-        P.has_run_mql = has_mql ? 1 : 0;
-        P.run_mql = mql;
-        P.mask_pos = idx->maskpos.get();
-        P.weight = idx->weight;
-        P.mask_len = idx->mask_len;
-        search::search_kernel<<<(unsigned)div_up(nq, 128), 128, 0, ctx.stream>>>(P, d_q.get(), d_off.get(), nq, d_b.get(), d_e.get());
-        SUFR_KERNEL_CHECK();
+        launch_search(idx, d_q.get(), d_off.get(), nq, has_mql, mql, use_subsample, d_b.get(), d_e.get());
         SUFR_CUDA_CHECK(cudaMemcpyAsync(rank_begin, d_b.get(), nq * 8, cudaMemcpyDeviceToHost, ctx.stream));
         SUFR_CUDA_CHECK(cudaMemcpyAsync(rank_end, d_e.get(), nq * 8, cudaMemcpyDeviceToHost, ctx.stream));
         SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
@@ -897,6 +1041,186 @@ int sufr_b200_index_suffixes(SufrB200Index* idx, uint64_t rank_begin, uint64_t c
             SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
             for (uint64_t i = 0; i < count; i++) out[i] = tmp[i];
         }
+    });
+}
+
+static char* dup_cstr(const std::string& s) {
+    char* p = (char*)malloc(s.size() + 1);
+    if (!p) throw std::bad_alloc();
+    memcpy(p, s.data(), s.size());
+    p[s.size()] = 0;
+    return p;
+}
+
+int sufr_b200_file_info(const char* path, SufrB200FileInfo* out) {
+    return guarded([&] {
+        if (!path || !out) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        memset(out, 0, sizeof(*out));
+        SufrFileInfo fi;
+        read_sufr_info(path, fi);
+        SufrB200FileInfo r;
+        memset(&r, 0, sizeof(r));
+        r.version = fi.version;
+        r.index_bits = fi.index_bits;
+        r.is_dna = fi.is_dna;
+        r.allow_ambiguity = fi.allow_ambiguity;
+        r.ignore_softmask = fi.ignore_softmask;
+        r.text_len = fi.text_len;
+        r.num_suffixes = fi.num_suffixes;
+        r.max_query_len = fi.max_query_len;
+        r.num_sequences = fi.sequence_starts.size();
+        r.text_pos = fi.text_pos;
+        r.sa_pos = fi.sa_pos;
+        r.lcp_pos = fi.lcp_pos;
+        r.file_bytes = fi.file_bytes;
+        try {
+            if (!fi.seed_mask.empty()) r.seed_mask = dup_cstr(fi.seed_mask);
+            r.sequence_starts = (uint64_t*)calloc(std::max<size_t>(1, fi.sequence_starts.size()), 8);
+            r.sequence_names = (char**)calloc(std::max<size_t>(1, fi.sequence_names.size()), sizeof(char*));
+            if (!r.sequence_starts || !r.sequence_names) throw std::bad_alloc();
+            for (size_t i = 0; i < fi.sequence_starts.size(); i++) {
+                r.sequence_starts[i] = fi.sequence_starts[i];
+                r.sequence_names[i] = dup_cstr(fi.sequence_names[i]);
+            }
+        } catch (...) {
+            sufr_b200_file_info_free(&r);
+            throw;
+        }
+        *out = r;
+    });
+}
+
+void sufr_b200_file_info_free(SufrB200FileInfo* info) {
+    if (!info) return;
+    free(info->seed_mask);
+    if (info->sequence_names)
+        for (uint64_t i = 0; i < info->num_sequences; i++) free(info->sequence_names[i]);
+    free(info->sequence_names);
+    free(info->sequence_starts);
+    memset(info, 0, sizeof(*info));
+}
+
+int sufr_b200_index_open(SufrB200Ctx* c, const char* path, SufrB200Index** out) {
+    return guarded([&] {
+        Ctx* ctx = reinterpret_cast<Ctx*>(c);
+        if (!ctx || !path || !out) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        SufrFileInfo fi;
+        read_sufr_info(path, fi);
+        const int fd = open(path, O_RDONLY);
+        if (fd < 0) throw Error(SUFR_B200_ERR_IO, std::string(path) + ": " + strerror(errno));
+        struct FdCloser { int fd; ~FdCloser() { close(fd); } } closer{fd};
+        std::lock_guard<std::mutex> lock(ctx->mu);
+        SUFR_CUDA_CHECK(cudaSetDevice(ctx->device));
+        auto idx = std::make_unique<SufrB200Index>();  // (on failure freed before the lock is released)
+        idx->ctx = ctx;
+        idx->n = fi.text_len;
+        idx->s = fi.num_suffixes;
+        idx->wide = fi.index_bits == 64;
+        const size_t w = fi.index_bits / 8;
+        idx->own_text = DevBuf<unsigned char>(ctx->pool, fi.text_len + 16);
+        idx->own_sa = DevBuf<unsigned char>(ctx->pool, fi.num_suffixes * w + 16);
+        idx->own_lcp = DevBuf<unsigned char>(ctx->pool, fi.num_suffixes * w + 16);
+        idx->text = idx->own_text.get();
+        idx->sa = idx->own_sa.get();
+        idx->lcp = idx->own_lcp.get();
+        upload_file_sections(fd, path, ctx->device, ctx->stream,
+                             {{fi.text_pos, fi.text_len, idx->own_text.get()},
+                              {fi.sa_pos, fi.num_suffixes * w, idx->own_sa.get()},
+                              {fi.lcp_pos, fi.num_suffixes * w, idx->own_lcp.get()}});
+        // a corrupt suffix array would send the searches outside the text: refused here, before any search runs
+        if (fi.num_suffixes) {
+            DevBuf<unsigned long long> d_max(ctx->pool, 1);
+            SUFR_CUDA_CHECK(cudaMemsetAsync(d_max.get(), 0, 8, ctx->stream));
+            const uint32_t grid = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(1, div_up(fi.num_suffixes, 256 * 8)),
+                                                               (uint64_t)num_sms() * 8);
+            search::max_entry_kernel<<<grid, 256, 0, ctx->stream>>>(idx->sa, fi.num_suffixes, idx->wide, d_max.get());
+            SUFR_KERNEL_CHECK();
+            unsigned long long mx = 0;
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(&mx, d_max.get(), 8, cudaMemcpyDeviceToHost, ctx->stream));
+            SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
+            if (mx >= fi.text_len)
+                throw Error(SUFR_B200_ERR_IO, std::string(path) + ": invalid .sufr file: suffix array entry " + std::to_string(mx) +
+                                                  " is not below the text length " + std::to_string(fi.text_len));
+        }
+        index_set_mask(*idx, *ctx, fi.seed_mask.empty() ? nullptr : fi.seed_mask.c_str(), fi.max_query_len > 0,
+                       fi.max_query_len);
+        index_set_starts(*idx, *ctx, fi.sequence_starts.data(), fi.sequence_starts.size());
+        *out = idx.release();
+    });
+}
+
+int sufr_b200_index_locate(SufrB200Index* idx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq, int has_mql,
+                           uint64_t mql, int low_memory, uint64_t* rank_begin, uint64_t* rank_end, uint64_t* hit_offsets) {
+    return guarded([&] {
+        if (!idx || !offsets || (nq && (!rank_begin || !rank_end)) || !hit_offsets || (nq && !queries && offsets[nq]))
+            throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        for (uint64_t i = 0; i < nq; i++)
+            if (offsets[i + 1] < offsets[i]) throw Error(SUFR_B200_ERR_ARGUMENT, "query offsets are not ascending");
+        Ctx& ctx = *idx->ctx;
+        std::lock_guard<std::mutex> lock(ctx.mu);
+        SUFR_CUDA_CHECK(cudaSetDevice(ctx.device));
+        idx->has_loc = false;
+        idx->loc_begin.reset();
+        idx->loc_end.reset();
+        idx->loc_offsets.reset();
+        // sufr_file.rs:514-560: the in-memory mode searches the LCP-subsampled array when the effective max_query_len
+        // is shorter than the build's
+        int use_sub = 0;
+        if (!low_memory) {
+            const uint64_t built = idx->built_mql();
+            const uint64_t eff = (has_mql && mql > 0) ? std::min(mql, built) : built;
+            if (eff != built) {
+                if (!idx->has_sub || idx->sub_mql != eff) index_subsample_locked(idx, eff);
+                use_sub = 1;
+            }
+        }
+        idx->loc_begin = DevBuf<unsigned long long>(ctx.pool, nq + 1);
+        idx->loc_end = DevBuf<unsigned long long>(ctx.pool, nq + 1);
+        idx->loc_offsets = DevBuf<unsigned long long>(ctx.pool, nq + 1);
+        SUFR_CUDA_CHECK(cudaMemsetAsync(idx->loc_offsets.get(), 0, 8, ctx.stream));
+        if (nq) {
+            const uint64_t bytes = offsets[nq];
+            DevBuf<uint8_t> d_q(ctx.pool, bytes + 8);
+            DevBuf<uint64_t> d_off(ctx.pool, nq + 1);
+            if (bytes) SUFR_CUDA_CHECK(cudaMemcpyAsync(d_q.get(), queries, bytes, cudaMemcpyHostToDevice, ctx.stream));
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(d_off.get(), offsets, (nq + 1) * 8, cudaMemcpyHostToDevice, ctx.stream));
+            launch_search(idx, d_q.get(), d_off.get(), nq, has_mql, mql, use_sub, idx->loc_begin.get(), idx->loc_end.get());
+            DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(nq));
+            scan::inclusive_scan(nq, search::HitCountIn{idx->loc_begin.get(), idx->loc_end.get()}, scan::SumU64{},
+                                 search::HitOffsetOut{idx->loc_offsets.get()}, partials.get(), ctx.stream);
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(rank_begin, idx->loc_begin.get(), nq * 8, cudaMemcpyDeviceToHost, ctx.stream));
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(rank_end, idx->loc_end.get(), nq * 8, cudaMemcpyDeviceToHost, ctx.stream));
+        }
+        SUFR_CUDA_CHECK(cudaMemcpyAsync(hit_offsets, idx->loc_offsets.get(), (nq + 1) * 8, cudaMemcpyDeviceToHost, ctx.stream));
+        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+        idx->loc_queries = nq;
+        idx->loc_hits = hit_offsets[nq];
+        idx->has_loc = true;
+    });
+}
+
+int sufr_b200_index_hits(SufrB200Index* idx, uint64_t first, uint64_t count, uint64_t* suffix, uint64_t* sequence,
+                         uint64_t* sequence_pos) {
+    return guarded([&] {
+        if (!idx) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        Ctx& ctx = *idx->ctx;
+        std::lock_guard<std::mutex> lock(ctx.mu);  // (the state of the last locate is read under the lock it is written under)
+        if (!idx->has_loc) throw Error(SUFR_B200_ERR_ARGUMENT, "sufr_b200_index_locate has not been called");
+        if (first > idx->loc_hits || count > idx->loc_hits - first)
+            throw Error(SUFR_B200_ERR_ARGUMENT, "hit window [" + std::to_string(first) + ", +" + std::to_string(count) +
+                                                    ") is beyond the " + std::to_string(idx->loc_hits) + " hits of the last locate");
+        if (count == 0) return;
+        SUFR_CUDA_CHECK(cudaSetDevice(ctx.device));
+        DevBuf<unsigned long long> d_out(ctx.pool, 3 * count);
+        unsigned long long* d_suf = d_out.get();
+        search::hits_kernel<<<(unsigned)div_up(count, 256), 256, 0, ctx.stream>>>(
+            idx->sa, idx->wide, idx->loc_begin.get(), idx->loc_offsets.get(), idx->loc_queries, idx->starts.get(),
+            idx->num_starts, first, count, d_suf, d_suf + count, d_suf + 2 * count);
+        SUFR_KERNEL_CHECK();
+        uint64_t* outs[3] = {suffix, sequence, sequence_pos};
+        for (int k = 0; k < 3; k++)
+            if (outs[k]) SUFR_CUDA_CHECK(cudaMemcpyAsync(outs[k], d_suf + k * count, count * 8, cudaMemcpyDeviceToHost, ctx.stream));
+        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
     });
 }
 

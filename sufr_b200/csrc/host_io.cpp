@@ -205,6 +205,156 @@ void write_sufr_file(const SufrB200Args& args, const SufrB200Result& r) {
     out.close();
 }
 
+// ------------------------------------------------------------------ `.sufr` reader (header, starts, mask, names)
+void pread_all(int fd, void* buf, size_t len, uint64_t off, const std::string& path) {
+    char* p = (char*)buf;
+    while (len) {
+        const ssize_t got = pread(fd, p, std::min<size_t>(len, 1u << 30), (off_t)off);
+        if (got < 0 && errno == EINTR) continue;
+        if (got < 0) throw Error(SUFR_B200_ERR_IO, path + ": " + strerror(errno));
+        if (got == 0) throw Error(SUFR_B200_ERR_IO, path + ": invalid .sufr file: unexpected end of file");
+        p += got;
+        off += (uint64_t)got;
+        len -= (size_t)got;
+    }
+}
+
+static uint64_t get_u64(const uint8_t* p) {
+    uint64_t v = 0;
+    for (int i = 7; i >= 0; i--) v = (v << 8) | p[i];
+    return v;
+}
+
+void read_sufr_info(const std::string& path, SufrFileInfo& info) {
+    info = SufrFileInfo();
+    const int fd = open(path.c_str(), O_RDONLY);
+    if (fd < 0) throw Error(SUFR_B200_ERR_IO, path + ": " + strerror(errno));
+    struct FdCloser { int fd; ~FdCloser() { close(fd); } } closer{fd};
+    auto bad = [&](const std::string& what) { return Error(SUFR_B200_ERR_IO, path + ": invalid .sufr file: " + what); };
+    struct stat st;
+    if (fstat(fd, &st) != 0) throw Error(SUFR_B200_ERR_IO, path + ": " + strerror(errno));
+    if (!S_ISREG(st.st_mode)) throw bad("not a regular file");
+    const uint64_t size = (uint64_t)st.st_size;
+    info.file_bytes = size;
+    if (size == 0) throw bad("empty file");
+    uint8_t head[60];
+    pread_all(fd, head, 1, 0, path);
+    info.version = head[0];
+    if (info.version != 6)
+        throw Error(SUFR_B200_ERR_UNSUPPORTED,
+                    path + ": unsupported .sufr version " + std::to_string(info.version) + " (only version 6 is read)");
+    if (size < 60 + 8) throw bad("truncated header (" + std::to_string(size) + " bytes)");
+    pread_all(fd, head, 60, 0, path);
+    // sufr_builder.rs:826-867
+    info.is_dna = head[1] != 0;
+    info.allow_ambiguity = head[2] != 0;
+    info.ignore_softmask = head[3] != 0;
+    info.text_len = get_u64(head + 4);
+    info.text_pos = get_u64(head + 12);
+    info.sa_pos = get_u64(head + 20);
+    info.lcp_pos = get_u64(head + 28);
+    info.num_suffixes = get_u64(head + 36);
+    info.max_query_len = get_u64(head + 44);
+    const uint64_t nseq = get_u64(head + 52);
+    const uint64_t n = info.text_len, s = info.num_suffixes;
+    if (n > size || s > size) throw bad("text length / suffix count larger than the file");
+    if (s > n) throw bad("num_suffixes " + std::to_string(s) + " exceeds the text length " + std::to_string(n));
+
+    // element width: from the section sizes (--index-bits 64 writes u64 files of short texts); with no suffixes the
+    // reference's rule (u32 iff text_len < u32::MAX, suffix_array.rs:460-470)
+    uint64_t w;
+    if (s > 0) {
+        if (info.lcp_pos < info.sa_pos || (info.lcp_pos - info.sa_pos) % s != 0) throw bad("suffix array section size");
+        w = (info.lcp_pos - info.sa_pos) / s;
+        if (w != 4 && w != 8) throw bad("element width " + std::to_string(w) + " (must be 4 or 8 bytes)");
+    } else {
+        w = n < 0xFFFFFFFFull ? 4 : 8;
+    }
+    info.index_bits = (uint32_t)(w * 8);
+    if (nseq > (size - 68) / w) throw bad("num_sequences " + std::to_string(nseq) + " does not fit the file");
+
+    // sequence starts, then the seed mask (u64 length + one byte per position)
+    std::vector<uint8_t> buf(nseq * w + 8);
+    pread_all(fd, buf.data(), buf.size(), 60, path);
+    info.sequence_starts.resize(nseq);
+    for (uint64_t i = 0; i < nseq; i++) {
+        uint64_t v = 0;
+        for (int k = (int)w - 1; k >= 0; k--) v = (v << 8) | buf[i * w + k];
+        info.sequence_starts[i] = v;
+        if (v >= n) throw bad("sequence start " + std::to_string(v) + " is not below the text length");
+        if (i > 0 && v <= info.sequence_starts[i - 1]) throw bad("sequence starts are not strictly increasing");
+    }
+    const uint64_t mask_off = 60 + nseq * w;
+    const uint64_t mask_len = get_u64(buf.data() + nseq * w);
+    if (mask_len > size - mask_off - 8) throw bad("seed mask length " + std::to_string(mask_len) + " does not fit the file");
+    if (mask_len) {
+        std::vector<uint8_t> mb(mask_len);
+        pread_all(fd, mb.data(), mask_len, mask_off + 8, path);
+        std::string mask(mask_len, '0');
+        for (uint64_t i = 0; i < mask_len; i++) {
+            if (mb[i] > 1) throw bad("seed mask byte " + std::to_string(mb[i]) + " (must be 0 or 1)");
+            mask[i] = mb[i] ? '1' : '0';
+        }
+        SeedMaskInfo m;
+        if (!parse_seed_mask(mask.c_str(), m)) throw bad("invalid seed mask '" + mask + "'");
+        info.seed_mask = mask;
+    }
+
+    // the sections follow each other without gaps (sufr_builder.rs:841-867)
+    if (info.text_pos != mask_off + 8 + mask_len)
+        throw bad("text_pos " + std::to_string(info.text_pos) + " (expected " + std::to_string(mask_off + 8 + mask_len) + ")");
+    if (info.sa_pos != info.text_pos + n)
+        throw bad("sa_pos " + std::to_string(info.sa_pos) + " (expected " + std::to_string(info.text_pos + n) + ")");
+    if (info.lcp_pos != info.sa_pos + s * w)
+        throw bad("lcp_pos " + std::to_string(info.lcp_pos) + " (expected " + std::to_string(info.sa_pos + s * w) + ")");
+    const uint64_t names_pos = info.lcp_pos + s * w;
+    if (names_pos > size) throw bad("truncated (no sequence names after the LCP array)");
+
+    // names: bincode Vec<String> up to exactly the end of the file (sufr_builder.rs:909), read through a small buffer
+    // as they are parsed, so that a file with junk behind its names is refused without reading the junk
+    struct TailReader {
+        int fd;
+        const std::string& path;
+        uint64_t pos, end;
+        std::vector<uint8_t> buf;
+        size_t at = 0;
+        bool take(void* dst, uint64_t len) {  // false: the file ends first
+            if (len > end - pos + (buf.size() - at)) return false;
+            uint8_t* d = (uint8_t*)dst;
+            while (len) {
+                if (at == buf.size()) {
+                    buf.resize((size_t)std::min<uint64_t>(1u << 20, end - pos));
+                    pread_all(fd, buf.data(), buf.size(), pos, path);
+                    pos += buf.size();
+                    at = 0;
+                }
+                const size_t k = (size_t)std::min<uint64_t>(len, buf.size() - at);
+                memcpy(d, buf.data() + at, k);
+                d += k;
+                at += k;
+                len -= k;
+            }
+            return true;
+        }
+        uint64_t left() const { return end - pos + (buf.size() - at); }
+    } tail{fd, path, names_pos, size, {}};
+    uint8_t word[8];
+    if (!tail.take(word, 8)) throw bad("truncated (no sequence names after the LCP array)");
+    const uint64_t count = get_u64(word);
+    if (count != nseq)
+        throw bad("the names tail holds " + std::to_string(count) + " names for " + std::to_string(nseq) + " sequences");
+    info.sequence_names.reserve(nseq);
+    for (uint64_t i = 0; i < nseq; i++) {
+        if (!tail.take(word, 8)) throw bad("truncated sequence names");
+        const uint64_t len = get_u64(word);
+        if (len > tail.left()) throw bad("truncated sequence names");
+        std::string name((size_t)len, '\0');
+        tail.take(&name[0], len);
+        info.sequence_names.push_back(std::move(name));
+    }
+    if (tail.left()) throw bad(std::to_string(tail.left()) + " unexpected bytes after the sequence names");
+}
+
 // ------------------------------------------------------------------ FASTA / FASTQ ingest (util.rs:51-89)
 // The reference delegates parsing to needletail 0.6 (not vendored).  This follows its documented
 // behaviour for plain-text input: FASTA records may span lines, FASTQ records are 4 lines, '\r' is

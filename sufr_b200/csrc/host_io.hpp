@@ -30,6 +30,22 @@ struct SufrFrame {
 SufrFrame make_sufr_frame(const SufrB200Args& args, uint32_t index_bits, uint64_t text_len, uint64_t total_suffixes);
 void pwrite_all(int fd, const void* buf, size_t len, uint64_t off, const std::string& path);
 
+// The header, sequence starts, seed mask and names tail of a version-6 `.sufr` file (read side of the layout above,
+// sufr_file.rs:145-275), validated so that every section offset and every sequence start can be trusted: a file that
+// fails a check is refused with SUFR_B200_ERR_IO ("{path}: invalid .sufr file: ..."), a version other than 6 with
+// SUFR_B200_ERR_UNSUPPORTED.  The three big sections are not read.
+struct SufrFileInfo {
+    uint32_t version = 0, index_bits = 0;
+    bool is_dna = false, allow_ambiguity = false, ignore_softmask = false;
+    uint64_t text_len = 0, num_suffixes = 0, max_query_len = 0;
+    uint64_t text_pos = 0, sa_pos = 0, lcp_pos = 0, file_bytes = 0;
+    std::string seed_mask;  // "" = none
+    std::vector<uint64_t> sequence_starts;
+    std::vector<std::string> sequence_names;
+};
+void read_sufr_info(const std::string& path, SufrFileInfo& out);
+void pread_all(int fd, void* buf, size_t len, uint64_t off, const std::string& path);
+
 // The output file of a build, written by many threads (and, sharded, by several ranks) at known offsets.  Concurrent
 // pwrite()s to ONE file serialise on the inode lock (3.5 GB/s on a RAM disk, whatever the thread count), so the file is
 // sized up front and mapped: the writers copy into the mapping and fault its pages in parallel.  Falls back to pwrite

@@ -181,5 +181,73 @@ struct SubsampleOut {
     }
 };
 
+// ---- locate (SufrFile::locate, sufr_file.rs:1132-1169) on the device: the search above, an exclusive scan of the
+// per-query hit counts (hit_offsets[num_queries + 1]), then one thread per hit of a window of the total.
+struct HitCountIn {
+    const unsigned long long* begin;
+    const unsigned long long* end;
+    __device__ unsigned long long operator()(uint64_t i) const {
+        return begin[i] == ~0ull || end[i] <= begin[i] ? 0ull : end[i] - begin[i];  // (ranks stay below num_suffixes)
+    }
+};
+struct HitOffsetOut {  // offsets[0] = 0 is set by the caller
+    unsigned long long* offsets;
+    __device__ void operator()(uint64_t i, unsigned long long, unsigned long long incl) const { offsets[i + 1] = incl; }
+};
+
+// last index i in [0, n) with a[i] <= v, or -1 (upper_bound - 1)
+__device__ __forceinline__ long long last_at_or_below(const unsigned long long* a, uint64_t n, uint64_t v) {
+    uint64_t lo = 0, hi = n;
+    while (lo < hi) {
+        const uint64_t mid = lo + (hi - lo) / 2;
+        if (a[mid] <= v) lo = mid + 1; else hi = mid;
+    }
+    return (long long)lo - 1;
+}
+
+// Hit h of [first, first + count): its query q (hit_offsets[q] <= h < hit_offsets[q + 1]), its rank in the full suffix
+// array, the suffix, and the record holding it (sequence starts ascend; none = UINT64_MAX and the suffix itself).
+// Consecutive hits of a query read consecutive suffix array entries.
+__global__ void __launch_bounds__(256) hits_kernel(const void* sa, int wide, const unsigned long long* __restrict__ rank_begin,
+                                                   const unsigned long long* __restrict__ hit_offsets, uint64_t num_queries,
+                                                   const unsigned long long* __restrict__ starts, uint64_t num_starts,
+                                                   uint64_t first, uint64_t count, unsigned long long* __restrict__ suffix,
+                                                   unsigned long long* __restrict__ sequence,
+                                                   unsigned long long* __restrict__ sequence_pos) {
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= count) return;
+    const uint64_t h = first + t;
+    const long long q = last_at_or_below(hit_offsets, num_queries + 1, h);
+    const uint64_t rank = rank_begin[q] + (h - hit_offsets[q]);
+    const uint64_t suf = entry(sa, rank, wide);
+    const long long seq = num_starts ? last_at_or_below(starts, num_starts, suf) : -1;
+    suffix[t] = suf;
+    sequence[t] = seq < 0 ? ~0ull : (unsigned long long)seq;
+    sequence_pos[t] = seq < 0 ? suf : suf - starts[seq];
+}
+
+// max over the entries of a suffix array read from a file (checked against the text length before any search):
+// 16-byte loads (`a` is 16-byte aligned), the last few entries one by one
+__global__ void __launch_bounds__(256) max_entry_kernel(const void* a, uint64_t len, int wide, unsigned long long* out) {
+    unsigned long long m = 0;
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const uint64_t per = wide ? 2 : 4;  // entries per 16 bytes
+    const uint4* v = reinterpret_cast<const uint4*>(a);
+    for (uint64_t i = t; i < len / per; i += stride) {
+        const uint4 x = v[i];
+        if (wide) {
+            m = max(m, ((unsigned long long)x.y << 32) | x.x);
+            m = max(m, ((unsigned long long)x.w << 32) | x.z);
+        } else {
+            m = max(m, (unsigned long long)max(max(x.x, x.y), max(x.z, x.w)));
+        }
+    }
+    for (uint64_t i = len / per * per + t; i < len; i += stride) m = max(m, (unsigned long long)entry(a, i, wide));
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) m = max(m, __shfl_down_sync(0xffffffffu, m, off));
+    if ((threadIdx.x & 31) == 0) atomicMax(out, m);
+}
+
 }  // namespace search
 }  // namespace sufr

@@ -1,9 +1,12 @@
 // `sufr-b200 create`: command-line mirror of `sufr create` (reference: sufr/src/lib.rs:83-125 flag
 // definitions, :321-371 create(), sufr/src/main.rs:8-41 global flags and error exit).
-// Only the `create` subcommand (alias `cr`) exists here; the query commands stay with the reference.
+// `sufr-b200 count` / `sufr-b200 locate`: the reference's query commands (sufr/src/lib.rs:467-530) over a `.sufr` file
+// opened into GPU memory (sufr_b200_index_open / _locate / _hits).  extract, list and summarize stay with the reference.
+#include <algorithm>
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
+#include <cerrno>
 #include <cstring>
 #include <string>
 #include <sys/stat.h>
@@ -33,13 +36,21 @@ struct CreateArgs {  // sufr/src/lib.rs:85-125
     uint32_t index_bits = 0;  // 0 = the reference's dispatch (u32 below u32::MAX bytes, suffix_array.rs:460-470)
 };
 
+const char* g_usage = "sufr-b200 create [OPTIONS] <INPUT>";
+
 [[noreturn]] void usage_error(const std::string& msg) {
-    fprintf(stderr, "error: %s\n\nUsage: sufr-b200 create [OPTIONS] <INPUT>\n\nFor more information, try '--help'.\n",
-            msg.c_str());
+    fprintf(stderr, "error: %s\n\nUsage: %s\n\nFor more information, try '--help'.\n", msg.c_str(), g_usage);
     exit(2);  // clap's usage-error exit code
 }
 
-void print_help() {
+// top_level: `sufr-b200` alone or `sufr-b200 --help`: the subcommands first, then the help of `create`
+void print_help(bool top_level) {
+    if (top_level)
+        puts("Usage: sufr-b200 [-t THREADS] [-l LOG] [--log-file FILE] <COMMAND> ...\n\n"
+             "Commands:\n"
+             "  create  Create sufr file (alias: cr)\n"
+             "  count   Count occurrences of sequences in a sufr file (see `sufr-b200 count --help`)\n"
+             "  locate  Locate sequences in a sufr file (see `sufr-b200 locate --help`)\n");
     puts("Create sufr file\n\n"
          "Usage: sufr-b200 [-t THREADS] [-l LOG] [--log-file FILE] create [OPTIONS] <INPUT>\n\n"
          "Arguments:\n  <INPUT>  Input file\n\nOptions:\n"
@@ -103,7 +114,219 @@ double now_s() {
 
 }  // namespace
 
+// ------------------------------------------------------------------ count / locate
+void print_query_help(bool locate) {
+    if (locate)
+        puts("Locate sequences\n\n"
+             "Usage: sufr-b200 locate [OPTIONS] <SUFR> [QUERY]...\n\n"
+             "Arguments:\n  <SUFR>      Sufr file\n  [QUERY]...  Query strings\n\nOptions:\n"
+             "  -f, --query-file <FILE>       Read queries from a file, one per line (empty lines are skipped)\n"
+             "  -m, --max-query-len <LEN>     Maximum query length: only the first LEN symbols (seed-mask positions) must match\n"
+             "  -a, --abs                     Show absolute position in the text: one line `QUERY POS POS ...`, in suffix order\n"
+             "      --low-memory              Search the full suffix array (default: the LCP-subsampled array when\n"
+             "                                --max-query-len is shorter than the one the file was built with)\n"
+             "      --device <ORDINAL>        CUDA device [default: 0]\n"
+             "  -h, --help                    Print help\n\n"
+             "Output: per query the query line, then one line `NAME POS,POS,...` per sequence that holds a match (names in\n"
+             "byte order, positions ascending), then `//`.  A query without a match prints its line and `//` only\n"
+             "(with --abs: the query alone on its line).");
+    else
+        puts("Count occurrences of sequences\n\n"
+             "Usage: sufr-b200 count [OPTIONS] <SUFR> [QUERY]...\n\n"
+             "Arguments:\n  <SUFR>      Sufr file\n  [QUERY]...  Query strings\n\nOptions:\n"
+             "  -f, --query-file <FILE>       Read queries from a file, one per line (empty lines are skipped)\n"
+             "  -m, --max-query-len <LEN>     Maximum query length: only the first LEN symbols (seed-mask positions) must match\n"
+             "      --low-memory              Search the full suffix array (default: the LCP-subsampled array when\n"
+             "                                --max-query-len is shorter than the one the file was built with)\n"
+             "      --device <ORDINAL>        CUDA device [default: 0]\n"
+             "  -h, --help                    Print help\n\n"
+             "Output: one line `QUERY COUNT` per query, in the order given (COUNT is 0 for a query without a match).");
+}
+
+struct Out {  // buffered stdout: a locate of frequent queries prints millions of positions
+    std::string buf;
+    void put(const std::string& s) { buf += s; flush_if(); }
+    void put(const char* p, size_t n) { buf.append(p, n); flush_if(); }
+    void num(uint64_t v) {
+        char t[24];
+        int k = snprintf(t, sizeof(t), "%llu", (unsigned long long)v);
+        buf.append(t, (size_t)k);
+    }
+    void flush_if() { if (buf.size() > (1u << 20)) flush(); }
+    void flush() { fwrite(buf.data(), 1, buf.size(), stdout); buf.clear(); }
+};
+
+int run_query(int argc, char** argv, bool locate) {
+    g_usage = locate ? "sufr-b200 locate [OPTIONS] <SUFR> [QUERY]..." : "sufr-b200 count [OPTIONS] <SUFR> [QUERY]...";
+    bool has_mql = false, low_memory = false, abs = false;
+    uint64_t mql = 0;
+    int device = 0;
+    std::vector<std::string> pos, files;
+    bool saw_cmd = false;
+    for (int i = 1; i < argc; i++) {
+        std::string s = argv[i];
+        auto value = [&](const std::string& flag) -> const char* {
+            size_t eq = s.find('=');
+            if (s.rfind("--", 0) == 0 && eq != std::string::npos) return argv[i] + eq + 1;
+            if (i + 1 >= argc) usage_error("a value is required for '" + flag + "' but none was supplied");
+            return argv[++i];
+        };
+        std::string key = s.rfind("--", 0) == 0 ? s.substr(0, s.find('=')) : s;
+        if (key == "-h" || key == "--help") { print_query_help(locate); return 0; }
+        else if (key == "-t" || key == "--threads") parse_u64(key, value(key));  // global flags: accepted, unused
+        else if (key == "-l" || key == "--log" || key == "--log-file") value(key);
+        else if (key == "-m" || key == "--max-query-len") { mql = parse_u64(key, value(key)); has_mql = true; }
+        else if (key == "--low-memory") low_memory = true;
+        else if (key == "--device") device = (int)parse_u64(key, value(key));
+        else if (key == "-f" || key == "--query-file") files.push_back(value(key));
+        else if (locate && (key == "-a" || key == "--abs")) abs = true;
+        else if (!s.empty() && s[0] == '-' && s.size() > 1) usage_error("unexpected argument '" + s + "' found");
+        else if (!saw_cmd && s == (locate ? "locate" : "count")) saw_cmd = true;
+        else pos.push_back(s);
+    }
+    if (pos.empty()) usage_error("the following required arguments were not provided:\n  <SUFR>");
+    const std::string path = pos[0];
+    std::vector<std::string> queries(pos.begin() + 1, pos.end());
+    for (const auto& f : files) {
+        FILE* fp = fopen(f.c_str(), "rb");
+        if (!fp) { fprintf(stderr, "Error: %s: %s\n", f.c_str(), strerror(errno)); return 1; }
+        std::string line;
+        int c;
+        auto push = [&] {
+            if (!line.empty() && line.back() == '\r') line.pop_back();
+            if (!line.empty()) queries.push_back(line);
+            line.clear();
+        };
+        while ((c = fgetc(fp)) != EOF) {
+            if (c == '\n') push(); else line.push_back((char)c);
+        }
+        push();
+        fclose(fp);
+    }
+    if (queries.empty()) usage_error("the following required arguments were not provided:\n  <QUERY>...");
+
+    SufrB200FileInfo info;
+    if (sufr_b200_file_info(path.c_str(), &info) != SUFR_B200_OK) {
+        fprintf(stderr, "Error: %s\n", sufr_b200_last_error());
+        return 1;
+    }
+    SufrB200Ctx* ctx = nullptr;
+    SufrB200Index* idx = nullptr;
+    auto fail = [&]() {
+        fprintf(stderr, "Error: %s\n", sufr_b200_last_error());
+        if (idx) sufr_b200_index_free(idx);
+        if (ctx) sufr_b200_ctx_destroy(ctx);
+        sufr_b200_file_info_free(&info);
+        return 1;
+    };
+    if (sufr_b200_ctx_create(device, &ctx) != SUFR_B200_OK) return fail();
+    if (sufr_b200_index_open(ctx, path.c_str(), &idx) != SUFR_B200_OK) return fail();
+
+    const uint64_t nq = queries.size();
+    std::string blob;
+    std::vector<uint64_t> offsets(nq + 1, 0);
+    for (uint64_t i = 0; i < nq; i++) {
+        blob += queries[i];
+        offsets[i + 1] = blob.size();
+    }
+    std::vector<uint64_t> rb(nq), re(nq), ho(nq + 1);
+    if (sufr_b200_index_locate(idx, (const uint8_t*)blob.data(), offsets.data(), nq, has_mql, mql, low_memory, rb.data(),
+                               re.data(), ho.data()) != SUFR_B200_OK)
+        return fail();
+
+    Out out;
+    if (!locate) {
+        for (uint64_t i = 0; i < nq; i++) {
+            out.put(queries[i]);
+            out.put(" ", 1);
+            out.num(ho[i + 1] - ho[i]);
+            out.put("\n", 1);
+        }
+    } else {
+        // names in byte order: rank of every record's name (equal names share a rank and a line)
+        const uint64_t ns = info.num_sequences;
+        std::vector<uint64_t> order(ns), name_rank(ns + 1);
+        for (uint64_t i = 0; i < ns; i++) order[i] = i;
+        std::sort(order.begin(), order.end(),
+                  [&](uint64_t x, uint64_t y) { return strcmp(info.sequence_names[x], info.sequence_names[y]) < 0; });
+        std::vector<const char*> rank_name;
+        for (uint64_t k = 0; k < ns; k++) {
+            if (k == 0 || strcmp(info.sequence_names[order[k]], info.sequence_names[order[k - 1]]) != 0)
+                rank_name.push_back(info.sequence_names[order[k]]);
+            name_rank[order[k]] = rank_name.size() - 1;
+        }
+        name_rank[ns] = rank_name.size();
+        rank_name.push_back("");  // hits outside every record (an index without sequence starts)
+
+        const uint64_t total = ho[nq], window = 1ull << 24;
+        std::vector<uint64_t> suf, seq, spos;
+        std::vector<std::pair<uint64_t, uint64_t>> cur;  // (name rank, position) of the current query
+        uint64_t q = 0;
+        auto begin_query = [&](uint64_t i) {
+            out.put(queries[i]);
+            if (!abs) out.put("\n", 1);
+        };
+        auto end_query = [&]() {
+            if (abs) { out.put("\n", 1); return; }
+            std::sort(cur.begin(), cur.end());
+            for (size_t k = 0; k < cur.size();) {
+                out.put(rank_name[cur[k].first]);
+                out.put(" ", 1);
+                size_t j = k;
+                for (; j < cur.size() && cur[j].first == cur[k].first; j++) {
+                    if (j > k) out.put(",", 1);
+                    out.num(cur[j].second);
+                }
+                out.put("\n", 1);
+                k = j;
+            }
+            out.put("//\n", 3);
+            cur.clear();
+        };
+        while (q < nq && ho[q + 1] == 0) { begin_query(q); end_query(); q++; }
+        if (q < nq) begin_query(q);
+        for (uint64_t first = 0; first < total; first += window) {
+            const uint64_t count = std::min(window, total - first);
+            suf.resize(count);
+            seq.resize(count);
+            spos.resize(count);
+            if (sufr_b200_index_hits(idx, first, count, suf.data(), abs ? nullptr : seq.data(), abs ? nullptr : spos.data()) !=
+                SUFR_B200_OK)
+                return fail();
+            for (uint64_t k = 0; k < count; k++) {
+                const uint64_t h = first + k;
+                while (h >= ho[q + 1]) {  // the hits of query q are done: close it and every empty query behind it
+                    end_query();
+                    q++;
+                    begin_query(q);
+                }
+                if (abs) {
+                    out.put(" ", 1);
+                    out.num(suf[k]);
+                } else {
+                    cur.push_back({seq[k] == UINT64_MAX ? ns : name_rank[seq[k]], spos[k]});
+                }
+            }
+        }
+        if (q < nq) {
+            end_query();
+            for (q++; q < nq; q++) { begin_query(q); end_query(); }
+        }
+    }
+    out.flush();
+    sufr_b200_index_free(idx);
+    sufr_b200_ctx_destroy(ctx);
+    sufr_b200_file_info_free(&info);
+    return 0;
+}
+
 int main(int argc, char** argv) {
+    // the subcommand is the first of the known names on the command line
+    for (int i = 1; i < argc; i++) {
+        const std::string s = argv[i];
+        if (s == "create" || s == "cr") break;
+        if (s == "count" || s == "locate") return run_query(argc, argv, s == "locate");
+    }
     CreateArgs a;
     std::vector<std::string> pos;
     bool saw_create = false;
@@ -116,7 +339,7 @@ int main(int argc, char** argv) {
             return argv[++i];
         };
         std::string key = s.rfind("--", 0) == 0 ? s.substr(0, s.find('=')) : s;
-        if (key == "-h" || key == "--help") { print_help(); return 0; }
+        if (key == "-h" || key == "--help") { print_help(!saw_create); return 0; }
         else if (key == "-t" || key == "--threads") a.threads = (int)parse_u64(key, value(key));
         else if (key == "-l" || key == "--log") a.log_level = value(key);
         else if (key == "--log-file") a.log_file = value(key);
@@ -144,8 +367,8 @@ int main(int argc, char** argv) {
         else pos.push_back(s);
     }
     if (!saw_create) {
-        if (argc <= 1) { print_help(); return 2; }
-        usage_error("unrecognized subcommand (only 'create' is provided by sufr-b200)");
+        if (argc <= 1) { print_help(true); return 2; }
+        usage_error("unrecognized subcommand (sufr-b200 provides 'create', 'count' and 'locate')");
     }
     if (pos.size() != 1) usage_error(pos.empty() ? "the following required arguments were not provided:\n  <INPUT>"
                                                  : "unexpected argument '" + pos[1] + "' found");
