@@ -199,7 +199,32 @@ void sufr_b200_index_free(SufrB200Index* index);
  *               query: suffix = SA[rank], sequence = index of the record holding it, sequence_pos = suffix - its
  *               start.  An index without sequence starts gives sequence = UINT64_MAX and sequence_pos = suffix.
  *               Any of the three outputs may be NULL.  A window beyond the total is SUFR_B200_ERR_ARGUMENT.
- *    An index made by index_create takes its sequence starts from args (none when args->num_sequences == 0). */
+ *    An index made by index_create takes its sequence starts from args (none when args->num_sequences == 0).
+ *
+ * -- extract, list, string_at (SufrFile::extract, SufrFile::list, SuffixArray::string_at) on the device, on an index
+ *    from index_open or index_create.  t = the text, n = its length, SA / LCP = the full arrays (s entries), sequence
+ *    starts s_0 < ... < s_{k-1} (k may be 0).
+ *      records    record i owns [s_i, e_i) with e_i = s_{i+1}, e_{k-1} = n (the rule of index_hits: a record's region
+ *                 can include its delimiter or the final '$').  A position outside every record (k = 0 or p < s_0)
+ *                 belongs to [0, s_0), or to [0, n) when k = 0; its sequence is UINT64_MAX.
+ *    index_extract  hits [first_hit, first_hit + max_hits) of the last index_locate, in its order (query order, then
+ *               rank order).  For a hit at suffix p in record [a, e): rel = p - a, start = rel - min(rel, prefix_len),
+ *               end = min(rel + suffix_len, e - a) (suffix_len UINT64_MAX = to the end of the record);
+ *               region_start / region_end = start / end, relative to the record start, and the bytes are
+ *               t[a + start, a + end).  The offset of the suffix in its region is rel - start = p - a - start.
+ *    index_list rows [first_rank, first_rank + max_rows): suffix = SA[r], lcp = LCP[r] as stored, bytes =
+ *               t[SA[r], min(SA[r] + len, n)) (len UINT64_MAX = the whole suffix).
+ *    byte budget  both calls take the longest leading run of their window whose bytes fit in max_bytes: its length
+ *               goes to *num_hits / *num_rows, its bytes to bytes[0 .. byte_offsets[num]), and byte_offsets[0 .. num]
+ *               are the entries' exclusive offsets into `bytes`.  byte_offsets needs max_hits / max_rows + 1 entries
+ *               and receives the offsets of the WHOLE window, so byte_offsets[i + 1] - byte_offsets[i] is the size of
+ *               entry i also where it did not fit.  When the first entry alone does not fit, the call returns OK with
+ *               num = 0 and byte_offsets[1] = that entry's size: retry with a buffer of at least that many bytes.
+ *               suffix, sequence, region_start, region_end and lcp may be NULL (their first num entries are written);
+ *               byte_offsets and bytes may not.
+ *    index_string_at  t[pos, min(pos + len, n)) to out, its length to *out_len (pos = n: empty).
+ *    SUFR_B200_ERR_ARGUMENT, before any device work: extract without a prior index_locate, a hit window beyond the
+ *    last locate's hits, a rank window beyond s, pos > n, NULL required pointers. */
 typedef struct SufrB200FileInfo {
     uint32_t version;
     uint32_t index_bits;          /* 32 or 64: width of SA / LCP entries and sequence starts in the file */
@@ -227,6 +252,14 @@ int sufr_b200_index_locate(SufrB200Index* index, const uint8_t* queries, const u
                            uint64_t* rank_end, uint64_t* hit_offsets);
 int sufr_b200_index_hits(SufrB200Index* index, uint64_t first_hit, uint64_t count, uint64_t* suffix, uint64_t* sequence,
                          uint64_t* sequence_pos);
+int sufr_b200_index_extract(SufrB200Index* index, uint64_t first_hit, uint64_t max_hits, uint64_t prefix_len,
+                            uint64_t suffix_len /* UINT64_MAX = to the end of the record */, uint64_t max_bytes,
+                            uint64_t* num_hits, uint64_t* suffix, uint64_t* sequence, uint64_t* region_start,
+                            uint64_t* region_end, uint64_t* byte_offsets /* max_hits + 1 */, uint8_t* bytes);
+int sufr_b200_index_list(SufrB200Index* index, uint64_t first_rank, uint64_t max_rows,
+                         uint64_t len /* UINT64_MAX = whole suffix */, uint64_t max_bytes, uint64_t* num_rows,
+                         uint64_t* suffix, uint64_t* lcp, uint64_t* byte_offsets /* max_rows + 1 */, uint8_t* bytes);
+int sufr_b200_index_string_at(SufrB200Index* index, uint64_t pos, uint64_t len, uint8_t* out, uint64_t* out_len);
 
 /* -- write: replaces SufrBuilder::write (sufr_builder.rs:817-918), version-6 `.sufr` layout.
  *    Single shard: writes the whole file.  Sharded: every rank calls it with the same path; rank 0

@@ -351,6 +351,29 @@ def file_info(path) -> dict:
         _lib.lib().sufr_b200_file_info_free(C.byref(fi))
 
 
+@dataclass
+class ExtractSequence:
+    """One hit of :meth:`SufrIndex.extract` (SufrFile::extract): the region around suffix ``suffix`` (rank ``rank``)
+    in the record named ``sequence_name`` that starts at text position ``sequence_start`` (None and 0 outside every
+    record).  ``sequence_range`` = (start, end) relative to the record start, ``suffix_offset`` = where the suffix
+    starts in ``sequence``, the region's bytes."""
+    rank: int
+    suffix: int
+    sequence_name: Optional[str]
+    sequence_start: int
+    sequence_range: Tuple[int, int]
+    suffix_offset: int
+    sequence: bytes
+
+
+@dataclass
+class ExtractResult:
+    """The hits of one query of :meth:`SufrIndex.extract`, in rank order (empty when it does not occur)."""
+    query_num: int
+    query: str
+    sequences: List[ExtractSequence]
+
+
 class SufrIndex:
     """Device-resident index: the read side that consumes the LCP array (``SufrFile::subsample_suffix_array``
     sufr_file.rs:429-456, ``suffix_search`` :777-836, ``locate`` :1132-1169, ``SufrSearch`` sufr_search.rs:104-350).
@@ -360,6 +383,7 @@ class SufrIndex:
     file into device memory the index owns (``.info`` holds its header, names, starts and mask)."""
 
     HITS_WINDOW = 1 << 24  # hits fetched per sufr_b200_index_hits call: bounds device memory for very frequent queries
+    EXTRACT_BYTES = 1 << 28  # default byte budget of one extract / list window (host buffer of that size)
 
     def __init__(self, result: "BuildResult", args: SufrBuilderArgs):
         self._res, self._args, self._ctx = result, args, result._ctx
@@ -369,6 +393,8 @@ class SufrIndex:
                                                  C.byref(self._h)))
         self._sub_mql = None
         self._names = list(args.sequence_names)
+        self._starts = [int(x) for x in args.sequence_starts]
+        self._n, self._s = result.text_len, result.num_suffixes
         if args.seed_mask is not None:
             self._built = SeedMask.new(args.seed_mask).weight        # sufr_file.rs:528
         else:
@@ -385,6 +411,8 @@ class SufrIndex:
         _check(_lib.lib().sufr_b200_index_open(self._ctx.handle, str(path).encode(), C.byref(self._h)))
         self._sub_mql = None
         self._names = self.info["sequence_names"]
+        self._starts = self.info["sequence_starts"]
+        self._n, self._s = self.info["text_len"], self.info["num_suffixes"]
         if self.info["seed_mask"] is not None:
             self._built = SeedMask.new(self.info["seed_mask"]).weight
         else:
@@ -491,6 +519,116 @@ class SufrIndex:
             lo, hi, r0 = int(ho[i]), int(ho[i + 1]), int(b[i])
             out.append([(r0 + k - lo, suf[k], None if seq[k] == none else names[seq[k]], pos[k]) for k in range(lo, hi)])
         return out
+
+    def extract_window(self, first: int, max_hits: int, prefix_len: Optional[int] = None,
+                       suffix_len: Optional[int] = None, max_bytes: Optional[int] = None):
+        """sufr_b200_index_extract: the regions of the longest leading run of hits [first, first + max_hits) of the
+        last locate whose bytes fit in ``max_bytes``.  Returns ((suffix, sequence, region_start, region_end,
+        byte_offsets), bytes) with numpy arrays of the run's length (byte_offsets one longer; sequence 2**64-1 outside
+        every record).  A first region larger than the budget gets one retry with a buffer of its size."""
+        max_bytes = self.EXTRACT_BYTES if max_bytes is None else max_bytes
+        _non_negative(first=first, max_hits=max_hits, prefix_len=prefix_len, suffix_len=suffix_len, max_bytes=max_bytes)
+        outs = [np.zeros(max(1, max_hits), dtype=np.uint64) for _ in range(4)]
+        offs = np.zeros(max_hits + 1, dtype=np.uint64)
+        num = C.c_uint64()
+        P = 0 if prefix_len is None else prefix_len
+        S = _U64_MAX if suffix_len is None else suffix_len
+        while True:
+            buf = np.empty(max(1, max_bytes), dtype=np.uint8)
+            _check(_lib.lib().sufr_b200_index_extract(self._h, first, max_hits, P, S, max_bytes, C.byref(num),
+                                                      *[o.ctypes.data for o in outs], offs.ctypes.data, buf.ctypes.data))
+            k = int(num.value)
+            if k or max_hits == 0 or int(offs[1]) <= max_bytes:
+                break
+            max_bytes = int(offs[1])  # the first region alone: retry with a buffer that holds it
+        return tuple(o[:k] for o in outs) + (offs[:k + 1],), buf[:int(offs[k])].tobytes()
+
+    def extract(self, queries, prefix_len: Optional[int] = None, suffix_len: Optional[int] = None,
+                max_query_len: Optional[int] = None, low_memory: bool = False) -> List[ExtractResult]:
+        """SufrFile::extract: per query the text around each hit, in rank order.  ``prefix_len`` bytes before the
+        suffix (default 0) and ``suffix_len`` from it (default: to the end of its record), clipped to the record;
+        see include/sufr_b200.h for the rule."""
+        b, _, ho = self.locate_ranges(queries, max_query_len, low_memory)
+        total = int(ho[-1])
+        parts, first = [], 0
+        while first < total:
+            arrs, data = self.extract_window(first, min(self.HITS_WINDOW, total - first), prefix_len, suffix_len)
+            parts.append((arrs, data))
+            first += len(arrs[0])
+        names, starts, none = self._names, self._starts, 0xFFFFFFFFFFFFFFFF
+        flat = []
+        for (suf, seq, rs, re_, offs), data in parts:
+            suf, seq, rs, re_, offs = suf.tolist(), seq.tolist(), rs.tolist(), re_.tolist(), offs.tolist()
+            for k in range(len(suf)):
+                a = 0 if seq[k] == none else starts[seq[k]]
+                flat.append(ExtractSequence(0, suf[k], None if seq[k] == none else names[seq[k]], a, (rs[k], re_[k]),
+                                            suf[k] - a - rs[k], data[offs[k]:offs[k + 1]]))
+        out = []
+        for i, q in enumerate(queries):
+            lo, hi, r0 = int(ho[i]), int(ho[i + 1]), int(b[i])
+            seqs = flat[lo:hi]
+            for k, e in enumerate(seqs):
+                e.rank = r0 + k
+            out.append(ExtractResult(i, q if isinstance(q, str) else bytes(q).decode("latin-1"), seqs))
+        return out
+
+    def list(self, first_rank: int = 0, count: Optional[int] = None, len: Optional[int] = None,
+             rows_window: int = 1 << 24, max_bytes: Optional[int] = None):
+        """SufrFile::list over ranks [first_rank, first_rank + count) (default: to the last rank): (suffix, lcp,
+        byte_offsets, bytes) with bytes[byte_offsets[i]:byte_offsets[i + 1]] = the first ``len`` bytes of suffix i
+        (default: the whole suffix).  Fetched in windows of ``rows_window`` rows and ``max_bytes`` bytes."""
+        _non_negative(first_rank=first_rank, count=count, len=len, max_bytes=max_bytes)
+        if count is None:
+            count = max(0, self._s - first_rank)
+        max_bytes = self.EXTRACT_BYTES if max_bytes is None else max_bytes
+        L = _U64_MAX if len is None else len
+        sufs, lcps, offs, datas = [], [], [np.zeros(1, np.uint64)], []
+        num, base, r, end = C.c_uint64(), 0, first_rank, first_rank + count
+        while True:
+            m = min(rows_window, end - r)
+            suf, lcp = np.zeros(max(1, m), np.uint64), np.zeros(max(1, m), np.uint64)
+            o = np.zeros(m + 1, np.uint64)
+            budget = max_bytes
+            while True:
+                buf = np.empty(max(1, budget), np.uint8)
+                _check(_lib.lib().sufr_b200_index_list(self._h, r, m, L, budget, C.byref(num), suf.ctypes.data,
+                                                       lcp.ctypes.data, o.ctypes.data, buf.ctypes.data))
+                k = int(num.value)
+                if k or m == 0 or int(o[1]) <= budget:
+                    break
+                budget = int(o[1])
+            if m == 0:
+                break
+            sufs.append(suf[:k])
+            lcps.append(lcp[:k])
+            offs.append(o[1:k + 1] + np.uint64(base))
+            datas.append(buf[:int(o[k])].tobytes())
+            base += int(o[k])
+            r += k
+            if r >= end:
+                break
+        cat = (lambda xs: np.concatenate(xs) if xs else np.zeros(0, np.uint64))
+        return cat(sufs), cat(lcps), np.concatenate(offs), b"".join(datas)
+
+    def string_at(self, pos: int, len: Optional[int] = None) -> bytes:
+        """SuffixArray::string_at: text[pos : pos + len] (default: to the end of the text); pos > text length raises."""
+        _non_negative(pos=pos, len=len)
+        want = max(0, self._n - pos) if len is None else min(len, max(0, self._n - pos))
+        out = np.empty(max(1, want), np.uint8)
+        got = C.c_uint64()
+        _check(_lib.lib().sufr_b200_index_string_at(self._h, pos, _U64_MAX if len is None else len, out.ctypes.data,
+                                                    C.byref(got)))
+        return out[:int(got.value)].tobytes()
+
+
+_U64_MAX = 0xFFFFFFFFFFFFFFFF
+
+
+def _non_negative(**values):
+    """Positions, counts and lengths travel as u64: a negative one would wrap to a huge value instead of failing."""
+    for name, v in values.items():
+        if v is not None and v < 0:
+            raise SufrError(_lib.ERR_ARGUMENT, f"{name} must not be negative (got {v})")
 
 
 def create_multi(args: SufrBuilderArgs, devices: Sequence[int], index_bits: int = 0) -> dict:

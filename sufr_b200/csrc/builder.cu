@@ -853,6 +853,9 @@ struct SufrB200Index {
     const void* sa = nullptr;
     const void* lcp = nullptr;
     uint64_t n = 0, s = 0;
+    // bytes from `text` on that may be read with 16-byte loads: n + 16 for an index that owns its (padded) text, n for
+    // one that borrows a build result's (gather_regions_kernel reads the last chunk byte by byte then)
+    uint64_t text_readable = 0;
     int wide = 0;
     bool is_mask = false;
     uint64_t build_mql = 0;
@@ -911,6 +914,7 @@ int sufr_b200_index_create(SufrB200Ctx* c, const SufrB200Args* args, const SufrB
         idx->sa = r->sa;
         idx->lcp = r->lcp;
         idx->n = r->text_len;
+        idx->text_readable = r->text_len;
         idx->s = r->num_suffixes;
         idx->wide = r->index_bits == 64;
         if (args->num_sequences && !args->sequence_starts) throw Error(SUFR_B200_ERR_ARGUMENT, "sequence_starts is NULL");
@@ -1118,6 +1122,7 @@ int sufr_b200_index_open(SufrB200Ctx* c, const char* path, SufrB200Index** out) 
         idx->wide = fi.index_bits == 64;
         const size_t w = fi.index_bits / 8;
         idx->own_text = DevBuf<unsigned char>(ctx->pool, fi.text_len + 16);
+        idx->text_readable = fi.text_len + 16;
         idx->own_sa = DevBuf<unsigned char>(ctx->pool, fi.num_suffixes * w + 16);
         idx->own_lcp = DevBuf<unsigned char>(ctx->pool, fi.num_suffixes * w + 16);
         idx->text = idx->own_text.get();
@@ -1221,6 +1226,114 @@ int sufr_b200_index_hits(SufrB200Index* idx, uint64_t first, uint64_t count, uin
         for (int k = 0; k < 3; k++)
             if (outs[k]) SUFR_CUDA_CHECK(cudaMemcpyAsync(outs[k], d_suf + k * count, count * 8, cudaMemcpyDeviceToHost, ctx.stream));
         SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+    });
+}
+
+// extract / list, with the context's lock held, after the window's kernel left the regions of its m entries in
+// d_src / d_len: scans the lengths into byte offsets (copied to byte_offsets[0..m]), takes the longest leading run of
+// entries whose bytes fit in max_bytes, gathers that run's bytes into `bytes` and returns its length.  The copies to
+// the caller's other outputs are queued by the caller, which then synchronises.
+static uint64_t index_gather(SufrB200Index* idx, uint64_t m, const unsigned long long* d_src, const unsigned long long* d_len,
+                             uint64_t max_bytes, uint64_t* byte_offsets, uint8_t* bytes, DevBuf<uint8_t>& d_bytes) {
+    Ctx& ctx = *idx->ctx;
+    DevBuf<unsigned long long> d_off(ctx.pool, m + 1);
+    DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(m));
+    SUFR_CUDA_CHECK(cudaMemsetAsync(d_off.get(), 0, 8, ctx.stream));
+    scan::inclusive_scan(m, search::ArrayIn{d_len}, scan::SumU64{}, search::HitOffsetOut{d_off.get()}, partials.get(),
+                         ctx.stream);
+    SUFR_CUDA_CHECK(cudaMemcpyAsync(byte_offsets, d_off.get(), (m + 1) * 8, cudaMemcpyDeviceToHost, ctx.stream));
+    SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+    const uint64_t k = (uint64_t)(std::upper_bound(byte_offsets, byte_offsets + m + 1, max_bytes) - byte_offsets) - 1;
+    const uint64_t total = byte_offsets[k];
+    if (total) {
+        d_bytes = DevBuf<uint8_t>(ctx.pool, div_up(total, 16) * 16);
+        const uint64_t chunks = div_up(total, 16);
+        search::gather_regions_kernel<<<(unsigned)div_up(chunks, 256), 256, 0, ctx.stream>>>(
+            idx->text, idx->n, idx->text_readable, d_src, d_off.get(), k, total, d_bytes.get());
+        SUFR_KERNEL_CHECK();
+        SUFR_CUDA_CHECK(cudaMemcpyAsync(bytes, d_bytes.get(), total, cudaMemcpyDeviceToHost, ctx.stream));
+    }
+    return k;
+}
+
+int sufr_b200_index_extract(SufrB200Index* idx, uint64_t first, uint64_t max_hits, uint64_t prefix_len,
+                            uint64_t suffix_len, uint64_t max_bytes, uint64_t* num_hits, uint64_t* suffix,
+                            uint64_t* sequence, uint64_t* region_start, uint64_t* region_end, uint64_t* byte_offsets,
+                            uint8_t* bytes) {
+    return guarded([&] {
+        if (!idx || !num_hits || !byte_offsets || !bytes) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        Ctx& ctx = *idx->ctx;
+        std::lock_guard<std::mutex> lock(ctx.mu);  // (the state of the last locate is read under the lock it is written under)
+        if (!idx->has_loc) throw Error(SUFR_B200_ERR_ARGUMENT, "sufr_b200_index_locate has not been called");
+        if (first > idx->loc_hits || max_hits > idx->loc_hits - first)
+            throw Error(SUFR_B200_ERR_ARGUMENT, "hit window [" + std::to_string(first) + ", +" + std::to_string(max_hits) +
+                                                    ") is beyond the " + std::to_string(idx->loc_hits) + " hits of the last locate");
+        *num_hits = 0;
+        byte_offsets[0] = 0;
+        if (max_hits == 0) return;
+        SUFR_CUDA_CHECK(cudaSetDevice(ctx.device));
+        const uint64_t m = max_hits;
+        DevBuf<unsigned long long> d_out(ctx.pool, 6 * m);
+        unsigned long long* d = d_out.get();
+        search::extract_regions_kernel<<<(unsigned)div_up(m, 256), 256, 0, ctx.stream>>>(
+            idx->sa, idx->wide, idx->loc_begin.get(), idx->loc_offsets.get(), idx->loc_queries, idx->starts.get(),
+            idx->num_starts, idx->n, first, m, prefix_len, suffix_len, d, d + m, d + 2 * m, d + 3 * m, d + 4 * m, d + 5 * m);
+        SUFR_KERNEL_CHECK();
+        DevBuf<uint8_t> d_bytes;
+        const uint64_t k = index_gather(idx, m, d + 4 * m, d + 5 * m, max_bytes, byte_offsets, bytes, d_bytes);
+        uint64_t* outs[4] = {suffix, sequence, region_start, region_end};
+        for (int o = 0; o < 4; o++)
+            if (outs[o] && k) SUFR_CUDA_CHECK(cudaMemcpyAsync(outs[o], d + o * m, k * 8, cudaMemcpyDeviceToHost, ctx.stream));
+        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+        *num_hits = k;
+    });
+}
+
+int sufr_b200_index_list(SufrB200Index* idx, uint64_t first, uint64_t max_rows, uint64_t len, uint64_t max_bytes,
+                         uint64_t* num_rows, uint64_t* suffix, uint64_t* lcp, uint64_t* byte_offsets, uint8_t* bytes) {
+    return guarded([&] {
+        if (!idx || !num_rows || !byte_offsets || !bytes) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        if (first > idx->s || max_rows > idx->s - first)
+            throw Error(SUFR_B200_ERR_ARGUMENT, "rank window [" + std::to_string(first) + ", +" + std::to_string(max_rows) +
+                                                    ") is beyond the " + std::to_string(idx->s) + " suffixes");
+        *num_rows = 0;
+        byte_offsets[0] = 0;
+        if (max_rows == 0) return;
+        Ctx& ctx = *idx->ctx;
+        std::lock_guard<std::mutex> lock(ctx.mu);
+        SUFR_CUDA_CHECK(cudaSetDevice(ctx.device));
+        const uint64_t m = max_rows;
+        DevBuf<unsigned long long> d_out(ctx.pool, 4 * m);
+        unsigned long long* d = d_out.get();
+        search::list_rows_kernel<<<(unsigned)div_up(m, 256), 256, 0, ctx.stream>>>(idx->sa, idx->lcp, idx->wide, idx->n, first,
+                                                                                   m, len, d, d + m, d + 2 * m, d + 3 * m);
+        SUFR_KERNEL_CHECK();
+        DevBuf<uint8_t> d_bytes;
+        const uint64_t k = index_gather(idx, m, d + 2 * m, d + 3 * m, max_bytes, byte_offsets, bytes, d_bytes);
+        if (suffix && k) SUFR_CUDA_CHECK(cudaMemcpyAsync(suffix, d, k * 8, cudaMemcpyDeviceToHost, ctx.stream));
+        if (lcp && k) SUFR_CUDA_CHECK(cudaMemcpyAsync(lcp, d + m, k * 8, cudaMemcpyDeviceToHost, ctx.stream));
+        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+        *num_rows = k;
+    });
+}
+
+int sufr_b200_index_string_at(SufrB200Index* idx, uint64_t pos, uint64_t len, uint8_t* out, uint64_t* out_len) {
+    return guarded([&] {
+        if (!idx || !out_len) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        if (pos > idx->n)
+            throw Error(SUFR_B200_ERR_ARGUMENT, "position " + std::to_string(pos) + " is beyond the text length " +
+                                                    std::to_string(idx->n));
+        const uint64_t k = std::min(len, idx->n - pos);
+        if (k && !out) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        *out_len = 0;
+        if (k) {
+            Ctx& ctx = *idx->ctx;
+            std::lock_guard<std::mutex> lock(ctx.mu);
+            SUFR_CUDA_CHECK(cudaSetDevice(ctx.device));
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(out, idx->text + pos, k, cudaMemcpyDeviceToHost, ctx.stream));
+            SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+        }
+        *out_len = k;
     });
 }
 

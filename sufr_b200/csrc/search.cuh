@@ -205,9 +205,25 @@ __device__ __forceinline__ long long last_at_or_below(const unsigned long long* 
     return (long long)lo - 1;
 }
 
-// Hit h of [first, first + count): its query q (hit_offsets[q] <= h < hit_offsets[q + 1]), its rank in the full suffix
-// array, the suffix, and the record holding it (sequence starts ascend; none = UINT64_MAX and the suffix itself).
-// Consecutive hits of a query read consecutive suffix array entries.
+// Hit h of the last locate: its query q (hit_offsets[q] <= h < hit_offsets[q + 1]), its rank in the full suffix array,
+// the suffix, and the record holding it (sequence starts ascend; -1 = none).  Consecutive hits of a query read
+// consecutive suffix array entries.
+struct HitLocation {
+    uint64_t suffix;
+    long long sequence;
+};
+__device__ __forceinline__ HitLocation locate_hit(const void* sa, int wide, const unsigned long long* rank_begin,
+                                                  const unsigned long long* hit_offsets, uint64_t num_queries,
+                                                  const unsigned long long* starts, uint64_t num_starts, uint64_t h) {
+    const long long q = last_at_or_below(hit_offsets, num_queries + 1, h);
+    const uint64_t rank = rank_begin[q] + (h - hit_offsets[q]);
+    HitLocation r;
+    r.suffix = entry(sa, rank, wide);
+    r.sequence = num_starts ? last_at_or_below(starts, num_starts, r.suffix) : -1;
+    return r;
+}
+
+// Hit first + t for t < count: suffix, record (none = UINT64_MAX) and position in the record (none: the suffix itself).
 __global__ void __launch_bounds__(256) hits_kernel(const void* sa, int wide, const unsigned long long* __restrict__ rank_begin,
                                                    const unsigned long long* __restrict__ hit_offsets, uint64_t num_queries,
                                                    const unsigned long long* __restrict__ starts, uint64_t num_starts,
@@ -216,14 +232,126 @@ __global__ void __launch_bounds__(256) hits_kernel(const void* sa, int wide, con
                                                    unsigned long long* __restrict__ sequence_pos) {
     const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= count) return;
-    const uint64_t h = first + t;
-    const long long q = last_at_or_below(hit_offsets, num_queries + 1, h);
-    const uint64_t rank = rank_begin[q] + (h - hit_offsets[q]);
-    const uint64_t suf = entry(sa, rank, wide);
-    const long long seq = num_starts ? last_at_or_below(starts, num_starts, suf) : -1;
+    const HitLocation l = locate_hit(sa, wide, rank_begin, hit_offsets, num_queries, starts, num_starts, first + t);
+    suffix[t] = l.suffix;
+    sequence[t] = l.sequence < 0 ? ~0ull : (unsigned long long)l.sequence;
+    sequence_pos[t] = l.sequence < 0 ? l.suffix : l.suffix - starts[l.sequence];
+}
+
+// ---- extract / list (SufrFile::extract, SufrFile::list): one thread per hit or rank computes the text region
+// [src, src + len) of its entry; an inclusive scan of the lengths (ArrayIn + HitOffsetOut) gives the byte offsets of
+// the entries in the output, and gather_regions_kernel copies the regions there.
+
+// Hit first + t: the region around its suffix p in record [a, e) (include/sufr_b200.h): rel = p - a,
+// start = rel - min(rel, prefix_len), end = min(rel + suffix_len, e - a); src = a + start, len = end - start.
+// A suffix outside every record belongs to [0, s_0), or to [0, n) without sequence starts.
+__global__ void __launch_bounds__(256) extract_regions_kernel(
+    const void* sa, int wide, const unsigned long long* __restrict__ rank_begin,
+    const unsigned long long* __restrict__ hit_offsets, uint64_t num_queries, const unsigned long long* __restrict__ starts,
+    uint64_t num_starts, uint64_t n, uint64_t first, uint64_t count, uint64_t prefix_len, uint64_t suffix_len,
+    unsigned long long* __restrict__ suffix, unsigned long long* __restrict__ sequence,
+    unsigned long long* __restrict__ region_start, unsigned long long* __restrict__ region_end,
+    unsigned long long* __restrict__ src, unsigned long long* __restrict__ len) {
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= count) return;
+    const HitLocation l = locate_hit(sa, wide, rank_begin, hit_offsets, num_queries, starts, num_starts, first + t);
+    const uint64_t a = l.sequence < 0 ? 0 : starts[l.sequence];
+    const uint64_t e = l.sequence < 0 ? (num_starts ? starts[0] : n)
+                                      : ((uint64_t)l.sequence + 1 < num_starts ? starts[l.sequence + 1] : n);
+    const uint64_t rel = l.suffix - a, span = e - a;
+    const uint64_t start = rel - (prefix_len < rel ? prefix_len : rel);
+    const uint64_t end = suffix_len >= span - rel ? span : rel + suffix_len;  // (p < e: no overflow)
+    suffix[t] = l.suffix;
+    sequence[t] = l.sequence < 0 ? ~0ull : (unsigned long long)l.sequence;
+    region_start[t] = start;
+    region_end[t] = end;
+    src[t] = a + start;
+    len[t] = end - start;
+}
+
+// Rank first + t: SA[r], LCP[r] as stored, and the first min(max_len, n - SA[r]) bytes of the suffix.
+__global__ void __launch_bounds__(256) list_rows_kernel(const void* sa, const void* lcp, int wide, uint64_t n, uint64_t first,
+                                                        uint64_t count, uint64_t max_len,
+                                                        unsigned long long* __restrict__ suffix,
+                                                        unsigned long long* __restrict__ lcp_out,
+                                                        unsigned long long* __restrict__ src,
+                                                        unsigned long long* __restrict__ len) {
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= count) return;
+    const uint64_t suf = entry(sa, first + t, wide);
+    const uint64_t rest = n - suf;
     suffix[t] = suf;
-    sequence[t] = seq < 0 ? ~0ull : (unsigned long long)seq;
-    sequence_pos[t] = seq < 0 ? suf : suf - starts[seq];
+    lcp_out[t] = entry(lcp, first + t, wide);
+    src[t] = suf;
+    len[t] = max_len < rest ? max_len : rest;
+}
+
+struct ArrayIn {
+    const unsigned long long* a;
+    __device__ unsigned long long operator()(uint64_t i) const { return a[i]; }
+};
+
+// The 16 text bytes at the 16-byte aligned address `al`.  Vector load when the whole chunk lies in
+// [text, text + readable) (the text plus the padding its allocation is known to have), else byte by byte with the
+// bytes outside [text, text + n) read as 0: no load leaves the text allocation, whatever its padding and alignment.
+__device__ __forceinline__ unsigned __int128 load_chunk(const uint8_t* text, uint64_t n, uint64_t readable, uintptr_t al) {
+    const uintptr_t base = (uintptr_t)text;
+    if (al >= base && al + 16 <= base + readable) {
+        const uint4 v = __ldg(reinterpret_cast<const uint4*>(al));
+        return ((unsigned __int128)(((unsigned long long)v.w << 32) | v.z) << 64) | (((unsigned long long)v.y << 32) | v.x);
+    }
+    unsigned __int128 r = 0;
+    for (int k = 0; k < 16; k++)
+        if (al + k >= base && al + k < base + n) r |= (unsigned __int128)text[al + k - base] << (8 * k);
+    return r;
+}
+
+// Copies t[src_i, src_i + len_i) to out + off_i for the m entries (off[0] = 0, off[i + 1] = off[i] + len_i,
+// total = off[m]).  Parallel over OUTPUT bytes, so one region of tens of MB spreads over the whole GPU like millions
+// of short ones: thread c owns output bytes [16c, 16c + 16) and writes them with one 16-byte store (out is 16-byte
+// aligned and holds total rounded up to 16 bytes; the bytes past total are written as 0).  Its entries come from a
+// binary search over the offsets, narrowed to the warp's range by two searches per warp; each run of bytes from one
+// entry is two aligned 16-byte loads and a shift.
+__global__ void __launch_bounds__(256) gather_regions_kernel(const uint8_t* __restrict__ text, uint64_t n, uint64_t readable,
+                                                             const unsigned long long* __restrict__ src,
+                                                             const unsigned long long* __restrict__ off, uint64_t m,
+                                                             uint64_t total, uint8_t* __restrict__ out) {
+    const uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int lane = threadIdx.x & 31;
+    const uint64_t warp_first = (c - lane) * 16;
+    if (warp_first >= total) return;  // (warp-uniform)
+    const uint64_t warp_last = ((c - lane) + 32) * 16 < total ? ((c - lane) + 32) * 16 - 1 : total - 1;
+    long long lo = 0, hi = 0;
+    if (lane == 0) lo = last_at_or_below(off, m, warp_first);
+    if (lane == 31) hi = last_at_or_below(off, m, warp_last);
+    lo = __shfl_sync(0xffffffffu, lo, 0);
+    hi = __shfl_sync(0xffffffffu, hi, 31);
+    const uint64_t j0 = c * 16;
+    if (j0 >= total) return;
+    const uint64_t jend = j0 + 16 < total ? j0 + 16 : total;
+    uint64_t i = (uint64_t)lo + (uint64_t)last_at_or_below(off + lo, (uint64_t)(hi - lo) + 1, j0);
+    unsigned __int128 acc = 0;
+    for (uint64_t j = j0; j < jend; i++) {
+        const uint64_t o = off[i], seg_end = off[i + 1] < jend ? off[i + 1] : jend;
+        if (seg_end <= j) continue;  // an empty entry
+        const uint64_t s = src[i] + (j - o), seg = seg_end - j;
+        const uintptr_t addr = (uintptr_t)(text + s), al = addr & ~(uintptr_t)15;
+        const int sh = (int)(addr & 15);
+        unsigned __int128 v = load_chunk(text, n, readable, al);
+        if (sh) {
+            v >>= 8 * sh;
+            if (sh + seg > 16) v |= load_chunk(text, n, readable, al + 16) << (8 * (16 - sh));
+        }
+        if (seg < 16) v &= ((unsigned __int128)1 << (8 * seg)) - 1;
+        acc |= v << (8 * (j - j0));
+        j = seg_end;
+    }
+    uint4 w;
+    w.x = (uint32_t)acc;
+    w.y = (uint32_t)(acc >> 32);
+    w.z = (uint32_t)(acc >> 64);
+    w.w = (uint32_t)(acc >> 96);
+    reinterpret_cast<uint4*>(out)[c] = w;
 }
 
 // max over the entries of a suffix array read from a file (checked against the text length before any search):
