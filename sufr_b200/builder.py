@@ -391,14 +391,8 @@ class SufrIndex:
         self._h = C.c_void_p()
         _check(_lib.lib().sufr_b200_index_create(result._ctx.handle, C.byref(result._cargs.c), C.byref(result.c),
                                                  C.byref(self._h)))
-        self._sub_mql = None
-        self._names = list(args.sequence_names)
-        self._starts = [int(x) for x in args.sequence_starts]
-        self._n, self._s = result.text_len, result.num_suffixes
-        if args.seed_mask is not None:
-            self._built = SeedMask.new(args.seed_mask).weight        # sufr_file.rs:528
-        else:
-            self._built = args.max_query_len or result.text_len       # sufr_file.rs:521-527
+        self._set_fields(list(args.sequence_names), [int(x) for x in args.sequence_starts], result.text_len,
+                         result.num_suffixes, args.seed_mask, args.max_query_len)
 
     @classmethod
     def open(cls, path, ctx: Optional[Context] = None, device: int = 0) -> "SufrIndex":
@@ -409,15 +403,19 @@ class SufrIndex:
         self._ctx = ctx or default_context(device)
         self.info = file_info(path)
         _check(_lib.lib().sufr_b200_index_open(self._ctx.handle, str(path).encode(), C.byref(self._h)))
-        self._sub_mql = None
-        self._names = self.info["sequence_names"]
-        self._starts = self.info["sequence_starts"]
-        self._n, self._s = self.info["text_len"], self.info["num_suffixes"]
-        if self.info["seed_mask"] is not None:
-            self._built = SeedMask.new(self.info["seed_mask"]).weight
-        else:
-            self._built = self.info["max_query_len"] or self.info["text_len"]
+        fi = self.info
+        self._set_fields(fi["sequence_names"], fi["sequence_starts"], fi["text_len"], fi["num_suffixes"], fi["seed_mask"],
+                         fi["max_query_len"])
         return self
+
+    def _set_fields(self, names, starts, text_len, num_suffixes, seed_mask, max_query_len):
+        self._sub_mql = None
+        self._names, self._starts = names, starts
+        self._n, self._s = text_len, num_suffixes
+        if seed_mask is not None:
+            self._built = SeedMask.new(seed_mask).weight        # sufr_file.rs:528
+        else:
+            self._built = max_query_len or text_len              # sufr_file.rs:521-527
 
     def close(self):
         if self._h:
@@ -444,25 +442,31 @@ class SufrIndex:
         eff = min(max_query_len, self._built) if max_query_len else self._built
         return eff if eff != self._built else None
 
+    @staticmethod
+    def _pack_queries(queries):
+        """A batch of queries as the C ABI takes it: (blob, offsets), query i = blob[offsets[i]:offsets[i + 1]]."""
+        qs = [q.encode() if isinstance(q, str) else bytes(q) for q in queries]
+        offs = np.zeros(len(qs) + 1, dtype=np.uint64)
+        offs[1:] = np.cumsum([len(q) for q in qs])
+        return np.frombuffer(b"".join(qs) or b"\0", dtype=np.uint8), offs
+
     def search(self, queries: Sequence[str], max_query_len: Optional[int] = None, low_memory: bool = False):
         """SufrFile::suffix_search: per query the half-open rank range in the full suffix array, or None.
         low_memory=False mirrors set_suffix_array_mem (sufr_file.rs:514-560): when the effective max_query_len is
         shorter than what the index was built with, the LCP-subsampled array is searched."""
-        qs = [q.encode() if isinstance(q, str) else bytes(q) for q in queries]
-        offs = np.zeros(len(qs) + 1, dtype=np.uint64)
-        offs[1:] = np.cumsum([len(q) for q in qs])
-        blob = np.frombuffer(b"".join(qs) or b"\0", dtype=np.uint8)
+        blob, offs = self._pack_queries(queries)
+        nq = len(offs) - 1
         eff = self._subsample_mql(max_query_len, low_memory)
         if eff is not None and self._sub_mql != eff:
             self.subsample(eff)
         use_sub = int(eff is not None)
-        b = np.zeros(max(1, len(qs)), dtype=np.uint64)
-        e = np.zeros(max(1, len(qs)), dtype=np.uint64)
-        _check(_lib.lib().sufr_b200_index_search(self._h, blob.ctypes.data, offs.ctypes.data, len(qs),
+        b = np.zeros(max(1, nq), dtype=np.uint64)
+        e = np.zeros(max(1, nq), dtype=np.uint64)
+        _check(_lib.lib().sufr_b200_index_search(self._h, blob.ctypes.data, offs.ctypes.data, nq,
                                                  int(max_query_len is not None), int(max_query_len or 0), use_sub,
                                                  b.ctypes.data, e.ctypes.data))
         none = np.uint64(0xFFFFFFFFFFFFFFFF)
-        return [None if b[i] == none else (int(b[i]), int(e[i])) for i in range(len(qs))]
+        return [None if b[i] == none else (int(b[i]), int(e[i])) for i in range(nq)]
 
     def count(self, queries, max_query_len=None, low_memory=False) -> List[int]:
         return [0 if r is None else r[1] - r[0] for r in self.search(queries, max_query_len, low_memory)]
@@ -477,23 +481,21 @@ class SufrIndex:
         hit_offsets[i] .. hit_offsets[i + 1] in :meth:`hits`.  Absent queries have rank_begin == rank_end == 2**64-1.
         low_memory=False searches the LCP-subsampled array when the effective max_query_len is shorter than the
         build's (sufr_file.rs:514-560), as :meth:`search` does."""
-        qs = [q.encode() if isinstance(q, str) else bytes(q) for q in queries]
-        offs = np.zeros(len(qs) + 1, dtype=np.uint64)
-        offs[1:] = np.cumsum([len(q) for q in qs])
-        blob = np.frombuffer(b"".join(qs) or b"\0", dtype=np.uint8)
-        b = np.zeros(max(1, len(qs)), dtype=np.uint64)
-        e = np.zeros(max(1, len(qs)), dtype=np.uint64)
-        ho = np.zeros(len(qs) + 1, dtype=np.uint64)
+        blob, offs = self._pack_queries(queries)
+        nq = len(offs) - 1
+        b = np.zeros(max(1, nq), dtype=np.uint64)
+        e = np.zeros(max(1, nq), dtype=np.uint64)
+        ho = np.zeros(nq + 1, dtype=np.uint64)
         # the library replaces the index's subsample when this mode needs another one: keep the cache of search() true
         eff = self._subsample_mql(max_query_len, low_memory)
         if eff is not None:
             self._sub_mql = None
-        _check(_lib.lib().sufr_b200_index_locate(self._h, blob.ctypes.data, offs.ctypes.data, len(qs),
+        _check(_lib.lib().sufr_b200_index_locate(self._h, blob.ctypes.data, offs.ctypes.data, nq,
                                                  int(max_query_len is not None), int(max_query_len or 0),
                                                  int(low_memory), b.ctypes.data, e.ctypes.data, ho.ctypes.data))
         if eff is not None:
             self._sub_mql = eff
-        return b[:len(qs)], e[:len(qs)], ho
+        return b[:nq], e[:nq], ho
 
     def hits(self, first: int, count: int):
         """sufr_b200_index_hits: (suffix, sequence, sequence_pos) of hits [first, first + count) of the last locate."""
@@ -530,18 +532,23 @@ class SufrIndex:
         _non_negative(first=first, max_hits=max_hits, prefix_len=prefix_len, suffix_len=suffix_len, max_bytes=max_bytes)
         outs = [np.zeros(max(1, max_hits), dtype=np.uint64) for _ in range(4)]
         offs = np.zeros(max_hits + 1, dtype=np.uint64)
-        num = C.c_uint64()
         P = 0 if prefix_len is None else prefix_len
         S = _U64_MAX if suffix_len is None else suffix_len
-        while True:
-            buf = np.empty(max(1, max_bytes), dtype=np.uint8)
-            _check(_lib.lib().sufr_b200_index_extract(self._h, first, max_hits, P, S, max_bytes, C.byref(num),
-                                                      *[o.ctypes.data for o in outs], offs.ctypes.data, buf.ctypes.data))
-            k = int(num.value)
-            if k or max_hits == 0 or int(offs[1]) <= max_bytes:
-                break
-            max_bytes = int(offs[1])  # the first region alone: retry with a buffer that holds it
+        k, buf = self._fetch_window(_lib.lib().sufr_b200_index_extract, first, max_hits, (P, S), max_bytes, outs, offs)
         return tuple(o[:k] for o in outs) + (offs[:k + 1],), buf[:int(offs[k])].tobytes()
+
+    def _fetch_window(self, fn, first, m, params, max_bytes, outs, offs):
+        """sufr_b200_index_extract / _list over entries [first, first + m) into ``outs`` and ``offs`` with a buffer of
+        ``max_bytes``: (entries, buffer).  A first entry larger than that gets one retry with a buffer of its size."""
+        num, budget = C.c_uint64(), max_bytes
+        while True:
+            buf = np.empty(max(1, budget), dtype=np.uint8)
+            _check(fn(self._h, first, m, *params, budget, C.byref(num), *[o.ctypes.data for o in outs],
+                      offs.ctypes.data, buf.ctypes.data))
+            k = int(num.value)
+            if k or m == 0 or int(offs[1]) <= budget:
+                return k, buf
+            budget = int(offs[1])
 
     def extract(self, queries, prefix_len: Optional[int] = None, suffix_len: Optional[int] = None,
                 max_query_len: Optional[int] = None, low_memory: bool = False) -> List[ExtractResult]:
@@ -583,20 +590,12 @@ class SufrIndex:
         max_bytes = self.EXTRACT_BYTES if max_bytes is None else max_bytes
         L = _U64_MAX if len is None else len
         sufs, lcps, offs, datas = [], [], [np.zeros(1, np.uint64)], []
-        num, base, r, end = C.c_uint64(), 0, first_rank, first_rank + count
+        base, r, end = 0, first_rank, first_rank + count
         while True:
             m = min(rows_window, end - r)
             suf, lcp = np.zeros(max(1, m), np.uint64), np.zeros(max(1, m), np.uint64)
             o = np.zeros(m + 1, np.uint64)
-            budget = max_bytes
-            while True:
-                buf = np.empty(max(1, budget), np.uint8)
-                _check(_lib.lib().sufr_b200_index_list(self._h, r, m, L, budget, C.byref(num), suf.ctypes.data,
-                                                       lcp.ctypes.data, o.ctypes.data, buf.ctypes.data))
-                k = int(num.value)
-                if k or m == 0 or int(o[1]) <= budget:
-                    break
-                budget = int(o[1])
+            k, buf = self._fetch_window(_lib.lib().sufr_b200_index_list, r, m, (L,), max_bytes, (suf, lcp), o)
             if m == 0:
                 break
             sufs.append(suf[:k])
