@@ -167,10 +167,11 @@ static void launch_search(SufrB200Index* idx, const uint8_t* queries, const uint
     P.sa = use_subsample ? (const void*)idx->sub_sa.get() : idx->sa;
     P.rank = use_subsample ? (const void*)idx->sub_rank.get() : nullptr;
     P.len = use_subsample ? idx->sub_len : idx->s;
+    P.num_suffixes = idx->s;
     P.wide = idx->wide;
     P.is_mask = idx->is_mask;
     P.build_mql = idx->build_mql;
-    P.has_run_mql = has_mql ? 1 : 0;
+    P.has_run_mql = has_mql && mql > 0;  // a run-time max_query_len of 0 is no cap, on a capped index too
     P.run_mql = mql;
     P.mask_pos = idx->maskpos.get();
     P.weight = idx->weight;

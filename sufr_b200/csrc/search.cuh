@@ -17,10 +17,11 @@ struct Params {
     const void* sa;           // the array that is searched: full suffix array, or the subsampled one
     const void* rank;         // ranks of the subsampled entries in the full array (NULL: searching the full array)
     uint64_t len;             // entries of `sa`
+    uint64_t num_suffixes;    // entries of the full suffix array
     int wide;                 // entries are u64 (else u32)
     int is_mask;              // SuffixSortType::Mask (else MaxQueryLen(build_mql))
     uint64_t build_mql;       // max_query_len the index was built with (0 = none)
-    int has_run_mql;          // a max_query_len was given at search time
+    int has_run_mql;          // a max_query_len > 0 was given at search time (0 = none, as for the subsample choice)
     uint64_t run_mql;
     const uint32_t* mask_pos; // seed mask: offsets of the care positions
     uint32_t weight;
@@ -150,8 +151,9 @@ __global__ void __launch_bounds__(128) search_kernel(Params P, const uint8_t* __
         rank_begin[i] = (unsigned long long)start;
         rank_end[i] = (unsigned long long)end + 1;
     } else {  // compressed suffix array: sufr_search.rs:121-139
+        // one sampled entry matches: the range runs to the next sampled rank, or to the end of the FULL array
         rank_begin[i] = entry(P.rank, start, P.wide);
-        if (start == end) rank_end[i] = (uint64_t)start == P.len - 1 ? P.len : entry(P.rank, start + 1, P.wide);
+        if (start == end) rank_end[i] = (uint64_t)start == P.len - 1 ? P.num_suffixes : entry(P.rank, start + 1, P.wide);
         else rank_end[i] = entry(P.rank, end, P.wide) + 1;
     }
 }

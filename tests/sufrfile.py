@@ -34,7 +34,9 @@ class SufrFile:
 def parse_sufr(data: bytes) -> SufrFile:
     version, is_dna, amb, soft = data[0], data[1], data[2], data[3]
     text_len, text_pos, sa_pos, lcp_pos, num_suffixes, mql, nseq = struct.unpack_from("<7Q", data, 4)
-    bits = 32 if text_len < 0xFFFFFFFF else 64  # suffix_array.rs:390-402
+    # the element width from the section sizes, so u64 files of short texts (--index-bits 64) read right; the text
+    # length rule of suffix_array.rs:390-402 only for an empty array
+    bits = 8 * (lcp_pos - sa_pos) // num_suffixes if num_suffixes else (32 if text_len < 0xFFFFFFFF else 64)
     w = bits // 8
     dt = np.dtype("<u4") if bits == 32 else np.dtype("<u8")
     off = 60
