@@ -196,8 +196,8 @@ void sufr_b200_index_free(SufrB200Index* index);
  *               low_memory == 0 searches the LCP-subsampled array when the effective max_query_len is shorter than
  *               the build's (sufr_file.rs:514-560; the subsample is made and kept as needed, replacing one of
  *               another max_query_len that index_subsample made), low_memory != 0 the full array.  Ranges and offsets stay on the device for index_hits.
- *    index_hits hits [first_hit, first_hit + count) of the last index_locate, in query order and rank order within a
- *               query: suffix = SA[rank], sequence = index of the record holding it, sequence_pos = suffix - its
+ *    index_hits hits [first_hit, first_hit + count) of the last index_locate or index_mems (below), in query order and
+ *               rank order within a query (after index_mems, MEM order and rank order within a MEM): suffix = SA[rank], sequence = index of the record holding it, sequence_pos = suffix - its
  *               start.  An index without sequence starts gives sequence = UINT64_MAX and sequence_pos = suffix.
  *               Any of the three outputs may be NULL.  A window beyond the total is SUFR_B200_ERR_ARGUMENT.
  *    An index made by index_create takes its sequence starts from args (none when args->num_sequences == 0).
@@ -208,8 +208,8 @@ void sufr_b200_index_free(SufrB200Index* index);
  *      records    record i owns [s_i, e_i) with e_i = s_{i+1}, e_{k-1} = n (the rule of index_hits: a record's region
  *                 can include its delimiter or the final '$').  A position outside every record (k = 0 or p < s_0)
  *                 belongs to [0, s_0), or to [0, n) when k = 0; its sequence is UINT64_MAX.
- *    index_extract  hits [first_hit, first_hit + max_hits) of the last index_locate, in its order (query order, then
- *               rank order).  For a hit at suffix p in record [a, e): rel = p - a, start = rel - min(rel, prefix_len),
+ *    index_extract  hits [first_hit, first_hit + max_hits) of the last index_locate or index_mems, in its order (query
+ *               order, then rank order; the MEMs are the queries after index_mems).  For a hit at suffix p in record [a, e): rel = p - a, start = rel - min(rel, prefix_len),
  *               end = min(rel + suffix_len, e - a) (suffix_len UINT64_MAX = to the end of the record);
  *               region_start / region_end = start / end, relative to the record start, and the bytes are
  *               t[a + start, a + end).  The offset of the suffix in its region is rel - start = p - a - start.
@@ -261,6 +261,40 @@ int sufr_b200_index_list(SufrB200Index* index, uint64_t first_rank, uint64_t max
                          uint64_t len /* UINT64_MAX = whole suffix */, uint64_t max_bytes, uint64_t* num_rows,
                          uint64_t* suffix, uint64_t* lcp, uint64_t* byte_offsets /* max_rows + 1 */, uint8_t* bytes);
 int sufr_b200_index_string_at(SufrB200Index* index, uint64_t pos, uint64_t len, uint8_t* out, uint64_t* out_len);
+
+/* -- matching statistics and maximal exact matches (MEMs) of long queries, on the device, on an index from index_open
+ *    or index_create.  t = the text, n its length, SA the full suffix array (s entries; the LCP array and its
+ *    subsample play no part).  Only indexed suffixes count: the positions SA holds (in DNA mode, positions the build
+ *    does not index are no matches).  A query q of length m is compared byte for byte, as index_search compares it:
+ *    no transformation, and the end of the text sorts first.  cap = the build's max_query_len, or none; there is no
+ *    run-time cap here.  Queries and offsets are those of index_search; the outputs are per byte of the batch.
+ *      matching statistics  for each 0 <= i < m, ms[i] = the largest l <= min(m - i, cap) such that q[i, i+l) is a
+ *               prefix of some indexed suffix, and [rank_begin[i], rank_end[i]) the half-open rank range of all indexed
+ *               suffixes with that prefix (contiguous in SA).  ms[i] = 0: both are UINT64_MAX.
+ *      MEMs with minimum length L >= 1  the pairs (i, ms[i]) with ms[i] >= L and (i == 0 or ms[i-1] <= ms[i]); their
+ *               occurrences are the ranks [rank_begin[i], rank_end[i]).  Without a cap every such occurrence is maximal
+ *               both ways: it cannot extend right, as ms[i] is the longest match, and it cannot extend left, as
+ *               q[i-1, i+ms[i]) occurs nowhere or ms[i-1] would be larger.  Shorter MEMs at other occurrences are not
+ *               listed (the extra matches of MUMmer's -maxmatch): for each query position only its longest match is.
+ *               With a cap, lengths stop at cap: a match of length cap is "at least cap" long, and the maximality
+ *               above holds only for matches shorter than cap.
+ *    index_matching_stats  match_len / rank_begin / rank_end: offsets[num_queries] entries each (ms of byte
+ *               offsets[k] + i of the batch is ms[i] of query k).
+ *    index_mems  the MEMs of every query, in query order and position order: *num_mems of them (at most one per byte,
+ *               so offsets[num_queries] entries suffice for mem_query, mem_pos, mem_len, rank_begin, rank_end);
+ *               hit_offsets[0 .. num_mems] = exclusive scan of their occurrence counts (offsets[num_queries] + 1
+ *               entries).  The MEMs then take the place of locate's queries: index_hits and index_extract return their
+ *               occurrences, windowed and byte-budgeted, until the next index_locate or index_mems.
+ *    A batch of empty queries gives no entries.  SUFR_B200_ERR_ARGUMENT, before any device work: NULL required
+ *    pointers, offsets not ascending, min_len == 0.  SUFR_B200_ERR_UNSUPPORTED: an index built with a seed mask (its
+ *    order is not a lexicographic order of contiguous bytes, so "longest match" has no meaning the array can answer). */
+int sufr_b200_index_matching_stats(SufrB200Index* index, const uint8_t* queries, const uint64_t* offsets,
+                                   uint64_t num_queries, uint64_t* match_len /* offsets[num_queries] */,
+                                   uint64_t* rank_begin, uint64_t* rank_end);
+int sufr_b200_index_mems(SufrB200Index* index, const uint8_t* queries, const uint64_t* offsets, uint64_t num_queries,
+                         uint64_t min_len, uint64_t* num_mems, uint64_t* mem_query, uint64_t* mem_pos,
+                         uint64_t* mem_len, uint64_t* rank_begin, uint64_t* rank_end,
+                         uint64_t* hit_offsets /* offsets[num_queries] + 1 */);
 
 /* -- write: replaces SufrBuilder::write (sufr_builder.rs:817-918), version-6 `.sufr` layout.
  *    Single shard: writes the whole file.  Sharded: every rank calls it with the same path; rank 0

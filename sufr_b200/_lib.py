@@ -142,7 +142,7 @@ ABI_SYMBOLS = [
     "sufr_b200_index_create", "sufr_b200_index_subsample", "sufr_b200_index_search", "sufr_b200_index_suffixes",
     "sufr_b200_index_free", "sufr_b200_file_info", "sufr_b200_file_info_free", "sufr_b200_index_open",
     "sufr_b200_index_locate", "sufr_b200_index_hits", "sufr_b200_index_extract", "sufr_b200_index_list",
-    "sufr_b200_index_string_at",
+    "sufr_b200_index_string_at", "sufr_b200_index_matching_stats", "sufr_b200_index_mems",
     "sufr_b200_seed_mask", "sufr_b200_find_lcp_full_offset", "sufr_b200_read_sequence_file",
     "sufr_b200_sequences_free", "sufr_b200_synth_dna", "sufr_b200_last_error", "sufr_b200_abi_version",
     "sufr_b200_device_count",
@@ -221,6 +221,13 @@ def lib():
                                        C.POINTER(C.c_uint64), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.sufr_b200_index_string_at.restype = C.c_int
     L.sufr_b200_index_string_at.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.POINTER(C.c_uint64)]
+    L.sufr_b200_index_matching_stats.restype = C.c_int
+    L.sufr_b200_index_matching_stats.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p,
+                                                 C.c_void_p, C.c_void_p]
+    L.sufr_b200_index_mems.restype = C.c_int
+    L.sufr_b200_index_mems.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64,
+                                       C.POINTER(C.c_uint64), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p]
     L.sufr_b200_seed_mask.restype = C.c_int64
     L.sufr_b200_seed_mask.argtypes = [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.sufr_b200_find_lcp_full_offset.restype = C.c_uint64

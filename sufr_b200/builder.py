@@ -498,7 +498,8 @@ class SufrIndex:
         return b[:nq], e[:nq], ho
 
     def hits(self, first: int, count: int):
-        """sufr_b200_index_hits: (suffix, sequence, sequence_pos) of hits [first, first + count) of the last locate."""
+        """sufr_b200_index_hits: (suffix, sequence, sequence_pos) of hits [first, first + count) of the last locate or
+        :meth:`mems`."""
         suf = np.zeros(max(1, count), dtype=np.uint64)
         seq = np.zeros(max(1, count), dtype=np.uint64)
         pos = np.zeros(max(1, count), dtype=np.uint64)
@@ -510,11 +511,7 @@ class SufrIndex:
         """SufrFile::locate: per query a list of (rank, suffix, sequence_name, sequence_position) in rank order
         (name None and position = suffix for an index without sequence starts)."""
         b, _, ho = self.locate_ranges(queries, max_query_len, low_memory)
-        total = int(ho[-1])
-        parts = [self.hits(f, min(self.HITS_WINDOW, total - f)) for f in range(0, total, self.HITS_WINDOW)]
-        suf = np.concatenate([p[0] for p in parts]).tolist() if parts else []
-        seq = np.concatenate([p[1] for p in parts]).tolist() if parts else []
-        pos = np.concatenate([p[2] for p in parts]).tolist() if parts else []
+        suf, seq, pos = self._all_hits(int(ho[-1]))
         names, none = self._names, 0xFFFFFFFFFFFFFFFF
         out = []
         for i in range(len(b)):
@@ -522,10 +519,65 @@ class SufrIndex:
             out.append([(r0 + k - lo, suf[k], None if seq[k] == none else names[seq[k]], pos[k]) for k in range(lo, hi)])
         return out
 
+    def _all_hits(self, total: int):
+        """(suffix, sequence, sequence_pos) lists of all ``total`` hits of the last locate / mems, in windows."""
+        parts = [self.hits(f, min(self.HITS_WINDOW, total - f)) for f in range(0, total, self.HITS_WINDOW)]
+        return tuple(np.concatenate([p[k] for p in parts]).tolist() if parts else [] for k in range(3))
+
+    def matching_statistics(self, queries):
+        """sufr_b200_index_matching_stats: per query (lengths, rank_begin, rank_end), numpy uint64 arrays of the
+        query's length.  lengths[i] = the longest l (at most the build's max_query_len) such that query[i:i+l] starts
+        an indexed suffix; [rank_begin[i], rank_end[i]) = the ranks of those suffixes (2**64-1 both when l = 0).  See
+        include/sufr_b200.h for the definitions; an index with a seed mask is refused (ERR_UNSUPPORTED)."""
+        blob, offs = self._pack_queries(queries)
+        nq, total = len(offs) - 1, int(offs[-1])
+        ms, b, e = (np.zeros(max(1, total), dtype=np.uint64) for _ in range(3))
+        _check(_lib.lib().sufr_b200_index_matching_stats(self._h, blob.ctypes.data, offs.ctypes.data, nq, ms.ctypes.data,
+                                                         b.ctypes.data, e.ctypes.data))
+        cuts = offs.astype(np.int64).tolist()
+        return [(ms[lo:hi], b[lo:hi], e[lo:hi]) for lo, hi in zip(cuts[:-1], cuts[1:])]
+
+    def _mems(self, queries, min_len):
+        """sufr_b200_index_mems: (query, position, length, rank_begin, rank_end, hit_offsets) as numpy arrays, one entry
+        per MEM (hit_offsets one longer).  The MEMs become the hits of :meth:`hits` / :meth:`extract_window`."""
+        if min_len < 1:
+            raise SufrError(_lib.ERR_ARGUMENT, f"min_len must be at least 1 (got {min_len})")
+        blob, offs = self._pack_queries(queries)
+        nq, total = len(offs) - 1, int(offs[-1])
+        cols = [np.zeros(max(1, total), dtype=np.uint64) for _ in range(5)]
+        ho = np.zeros(total + 1, dtype=np.uint64)
+        num = C.c_uint64()
+        _check(_lib.lib().sufr_b200_index_mems(self._h, blob.ctypes.data, offs.ctypes.data, nq, min_len, C.byref(num),
+                                               *[c.ctypes.data for c in cols], ho.ctypes.data))
+        k = int(num.value)
+        return tuple(c[:k] for c in cols) + (ho[:k + 1],)
+
+    def mems(self, queries, min_len: int):
+        """Maximal exact matches of at least ``min_len`` bytes (include/sufr_b200.h): per query a list of
+        (query_pos, length, rank_begin, rank_end) in position order.  Afterwards :meth:`hits` and
+        :meth:`extract_window` work on these MEMs (in query order, then position order) as on a locate's queries."""
+        q, p, ln, b, e, _ = self._mems(queries, min_len)
+        out = [[] for _ in range(len(queries))]
+        for row in zip(q.tolist(), p.tolist(), ln.tolist(), b.tolist(), e.tolist()):
+            out[row[0]].append(row[1:])
+        return out
+
+    def locate_mems(self, queries, min_len: int):
+        """:meth:`mems` with every occurrence: per query a list of (query_pos, length, hits) with hits a list of
+        (suffix, sequence_name, sequence_position) in rank order, as :meth:`locate` gives them."""
+        q, p, ln, _, _, ho = self._mems(queries, min_len)
+        suf, seq, pos = self._all_hits(int(ho[-1]))
+        names, none = self._names, 0xFFFFFFFFFFFFFFFF
+        out = [[] for _ in range(len(queries))]
+        for k, (qi, qp, ml) in enumerate(zip(q.tolist(), p.tolist(), ln.tolist())):
+            lo, hi = int(ho[k]), int(ho[k + 1])
+            out[qi].append((qp, ml, [(suf[h], None if seq[h] == none else names[seq[h]], pos[h]) for h in range(lo, hi)]))
+        return out
+
     def extract_window(self, first: int, max_hits: int, prefix_len: Optional[int] = None,
                        suffix_len: Optional[int] = None, max_bytes: Optional[int] = None):
         """sufr_b200_index_extract: the regions of the longest leading run of hits [first, first + max_hits) of the
-        last locate whose bytes fit in ``max_bytes``.  Returns ((suffix, sequence, region_start, region_end,
+        last locate or :meth:`mems` whose bytes fit in ``max_bytes``.  Returns ((suffix, sequence, region_start, region_end,
         byte_offsets), bytes) with numpy arrays of the run's length (byte_offsets one longer; sequence 2**64-1 outside
         every record).  A first region larger than the budget gets one retry with a buffer of its size."""
         max_bytes = self.EXTRACT_BYTES if max_bytes is None else max_bytes

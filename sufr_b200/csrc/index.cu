@@ -46,7 +46,8 @@ struct SufrB200Index {
     // sequence starts (u64) for locate; num_starts == 0: none
     DevBuf<unsigned long long> starts;
     uint64_t num_starts = 0;
-    // the last sufr_b200_index_locate: rank ranges and hit offsets of its queries, for sufr_b200_index_hits
+    // the last sufr_b200_index_locate or _mems: rank ranges and hit offsets of its queries (or MEMs), for
+    // sufr_b200_index_hits and sufr_b200_index_extract
     DevBuf<unsigned long long> loc_begin, loc_end, loc_offsets;
     uint64_t loc_queries = 0, loc_hits = 0;
     bool has_loc = false;
@@ -151,16 +152,23 @@ int sufr_b200_index_subsample(SufrB200Index* idx, uint64_t max_query_len, uint64
     });
 }
 
+// With the context's lock held: a batch of nq queries (blob + offsets) queued for upload to the device.
+struct DeviceQueries {
+    DevBuf<uint8_t> q;
+    DevBuf<uint64_t> off;
+    DeviceQueries(Ctx& ctx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq)
+        : q(ctx.pool, offsets[nq] + 8), off(ctx.pool, nq + 1) {
+        if (offsets[nq]) SUFR_CUDA_CHECK(cudaMemcpyAsync(q.get(), queries, offsets[nq], cudaMemcpyHostToDevice, ctx.stream));
+        SUFR_CUDA_CHECK(cudaMemcpyAsync(off.get(), offsets, (nq + 1) * 8, cudaMemcpyHostToDevice, ctx.stream));
+    }
+};
+
 // With the context's lock held: uploads nq >= 1 queries (blob + offsets) and queues their search, whose rank ranges go
 // to d_b / d_e.
 static void launch_search(SufrB200Index* idx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq, int has_mql,
                           uint64_t mql, int use_subsample, unsigned long long* d_b, unsigned long long* d_e) {
     Ctx& ctx = *idx->ctx;
-    const uint64_t bytes = offsets[nq];
-    DevBuf<uint8_t> d_q(ctx.pool, bytes + 8);
-    DevBuf<uint64_t> d_off(ctx.pool, nq + 1);
-    if (bytes) SUFR_CUDA_CHECK(cudaMemcpyAsync(d_q.get(), queries, bytes, cudaMemcpyHostToDevice, ctx.stream));
-    SUFR_CUDA_CHECK(cudaMemcpyAsync(d_off.get(), offsets, (nq + 1) * 8, cudaMemcpyHostToDevice, ctx.stream));
+    DeviceQueries dq(ctx, queries, offsets, nq);
     search::Params P{};
     P.text = idx->text;
     P.n = idx->n;
@@ -176,7 +184,7 @@ static void launch_search(SufrB200Index* idx, const uint8_t* queries, const uint
     P.mask_pos = idx->maskpos.get();
     P.weight = idx->weight;
     P.mask_len = idx->mask_len;
-    search::search_kernel<<<(unsigned)div_up(nq, 128), 128, 0, ctx.stream>>>(P, d_q.get(), d_off.get(), nq, d_b, d_e);
+    search::search_kernel<<<(unsigned)div_up(nq, 128), 128, 0, ctx.stream>>>(P, dq.q.get(), dq.off.get(), nq, d_b, d_e);
     SUFR_KERNEL_CHECK();
 }
 
@@ -364,13 +372,133 @@ int sufr_b200_index_locate(SufrB200Index* idx, const uint8_t* queries, const uin
     });
 }
 
-// With the context's lock held, under which the last locate wrote the state read here: refuses a window of hits that
-// is not inside the last locate's.
+// Argument checks shared by index_matching_stats and index_mems, before any device work.
+static void check_matching_args(const SufrB200Index* idx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq) {
+    if (nq && !queries && offsets[nq]) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+    for (uint64_t i = 0; i < nq; i++)
+        if (offsets[i + 1] < offsets[i]) throw Error(SUFR_B200_ERR_ARGUMENT, "query offsets are not ascending");
+    if (idx->is_mask)
+        throw Error(SUFR_B200_ERR_UNSUPPORTED, "matching statistics and MEMs need an index without a seed mask: a seed-mask "
+                                               "order does not sort contiguous bytes, so it has no longest match");
+}
+
+// With the context's lock held: queues matching_stats_kernel over the `total` bytes of the uploaded batch.
+static void launch_matching_stats(SufrB200Index* idx, const DeviceQueries& dq, uint64_t nq, uint64_t total,
+                                  unsigned long long* d_ms, unsigned long long* d_b, unsigned long long* d_e) {
+    Ctx& ctx = *idx->ctx;
+    search::Params P{};
+    P.text = idx->text;
+    P.n = idx->n;
+    P.sa = idx->sa;
+    P.len = idx->s;
+    P.num_suffixes = idx->s;
+    P.wide = idx->wide;
+    P.build_mql = idx->build_mql;
+    search::matching_stats_kernel<<<(unsigned)div_up(total, 128), 128, 0, ctx.stream>>>(
+        P, dq.q.get(), reinterpret_cast<const unsigned long long*>(dq.off.get()), nq, total, d_ms, d_b, d_e);
+    SUFR_KERNEL_CHECK();
+}
+
+int sufr_b200_index_matching_stats(SufrB200Index* idx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq,
+                                   uint64_t* match_len, uint64_t* rank_begin, uint64_t* rank_end) {
+    return guarded([&] {
+        if (!idx || !offsets) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        if (offsets[nq] && (!match_len || !rank_begin || !rank_end)) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        check_matching_args(idx, queries, offsets, nq);
+        const uint64_t total = offsets[nq];
+        if (total == 0) return;
+        Ctx& ctx = *idx->ctx;
+        CtxLock lock(ctx);
+        DeviceQueries dq(ctx, queries, offsets, nq);
+        DevBuf<unsigned long long> d_out(ctx.pool, 3 * total);
+        unsigned long long* d = d_out.get();
+        launch_matching_stats(idx, dq, nq, total, d, d + total, d + 2 * total);
+        uint64_t* outs[3] = {match_len, rank_begin, rank_end};
+        for (int k = 0; k < 3; k++)
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(outs[k], d + k * total, total * 8, cudaMemcpyDeviceToHost, ctx.stream));
+        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+    });
+}
+
+int sufr_b200_index_mems(SufrB200Index* idx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq,
+                         uint64_t min_len, uint64_t* num_mems, uint64_t* mem_query, uint64_t* mem_pos, uint64_t* mem_len,
+                         uint64_t* rank_begin, uint64_t* rank_end, uint64_t* hit_offsets) {
+    return guarded([&] {
+        if (!idx || !offsets || !num_mems || !hit_offsets) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        if (offsets[nq] && (!mem_query || !mem_pos || !mem_len || !rank_begin || !rank_end))
+            throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        if (min_len == 0) throw Error(SUFR_B200_ERR_ARGUMENT, "min_len must be at least 1");
+        check_matching_args(idx, queries, offsets, nq);
+        const uint64_t total = offsets[nq];
+        Ctx& ctx = *idx->ctx;
+        CtxLock lock(ctx);
+        idx->has_loc = false;
+        idx->loc_begin.reset();
+        idx->loc_end.reset();
+        idx->loc_offsets.reset();
+        // matching statistics of every byte, then the MEMs compacted by one scan of their flags
+        uint64_t mems = 0;
+        DevBuf<unsigned long long> d_ms, d_mem;
+        if (total) {
+            DeviceQueries dq(ctx, queries, offsets, nq);
+            d_ms = DevBuf<unsigned long long>(ctx.pool, 3 * total);
+            unsigned long long* ms = d_ms.get();
+            launch_matching_stats(idx, dq, nq, total, ms, ms + total, ms + 2 * total);
+            const auto* d_off = reinterpret_cast<const unsigned long long*>(dq.off.get());
+            const search::MemFlagIn in{ms, d_off, nq, min_len};
+            DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(total));
+            scan::scan_reduce(total, in, scan::SumU64{}, partials.get(), ctx.stream);
+            unsigned long long count = 0;
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(&count, partials.get() + div_up(total, scan::CHUNK), 8, cudaMemcpyDeviceToHost,
+                                            ctx.stream));
+            SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+            mems = count;
+            idx->loc_begin = DevBuf<unsigned long long>(ctx.pool, mems + 1);
+            idx->loc_end = DevBuf<unsigned long long>(ctx.pool, mems + 1);
+            // (query, position, length) of every MEM, then the byte each one starts at
+            d_mem = DevBuf<unsigned long long>(ctx.pool, 4 * mems + 1);
+            unsigned long long* m = d_mem.get();
+            scan::scan_apply(total, in, scan::SumU64{}, search::MemOut{m + 3 * mems}, partials.get(), ctx.stream);
+            if (mems) {
+                search::mem_fill_kernel<<<(unsigned)div_up(mems, 256), 256, 0, ctx.stream>>>(
+                    m + 3 * mems, mems, ms, ms + total, ms + 2 * total, d_off, nq, m, m + mems, m + 2 * mems,
+                    idx->loc_begin.get(), idx->loc_end.get());
+                SUFR_KERNEL_CHECK();
+            }
+        } else {
+            idx->loc_begin = DevBuf<unsigned long long>(ctx.pool, 1);
+            idx->loc_end = DevBuf<unsigned long long>(ctx.pool, 1);
+        }
+        // the MEMs take the place of locate's queries: hit offsets = exclusive scan of their occurrence counts
+        idx->loc_offsets = DevBuf<unsigned long long>(ctx.pool, mems + 1);
+        SUFR_CUDA_CHECK(cudaMemsetAsync(idx->loc_offsets.get(), 0, 8, ctx.stream));
+        if (mems) {
+            DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(mems));
+            scan::inclusive_scan(mems, search::HitCountIn{idx->loc_begin.get(), idx->loc_end.get()}, scan::SumU64{},
+                                 search::HitOffsetOut{idx->loc_offsets.get()}, partials.get(), ctx.stream);
+            uint64_t* outs[5] = {mem_query, mem_pos, mem_len, rank_begin, rank_end};
+            const unsigned long long* srcs[5] = {d_mem.get(), d_mem.get() + mems, d_mem.get() + 2 * mems,
+                                                 idx->loc_begin.get(), idx->loc_end.get()};
+            for (int k = 0; k < 5; k++)
+                SUFR_CUDA_CHECK(cudaMemcpyAsync(outs[k], srcs[k], mems * 8, cudaMemcpyDeviceToHost, ctx.stream));
+        }
+        SUFR_CUDA_CHECK(cudaMemcpyAsync(hit_offsets, idx->loc_offsets.get(), (mems + 1) * 8, cudaMemcpyDeviceToHost, ctx.stream));
+        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+        *num_mems = mems;
+        idx->loc_queries = mems;
+        idx->loc_hits = hit_offsets[mems];
+        idx->has_loc = true;
+    });
+}
+
+// With the context's lock held, under which the last locate or mems wrote the state read here: refuses a window of hits
+// that is not inside that call's.
 static void check_hit_window(const SufrB200Index* idx, uint64_t first, uint64_t count) {
-    if (!idx->has_loc) throw Error(SUFR_B200_ERR_ARGUMENT, "sufr_b200_index_locate has not been called");
+    if (!idx->has_loc)
+        throw Error(SUFR_B200_ERR_ARGUMENT, "neither sufr_b200_index_locate nor sufr_b200_index_mems has been called");
     if (first > idx->loc_hits || count > idx->loc_hits - first)
         throw Error(SUFR_B200_ERR_ARGUMENT, "hit window [" + std::to_string(first) + ", +" + std::to_string(count) +
-                                                ") is beyond the " + std::to_string(idx->loc_hits) + " hits of the last locate");
+                                                ") is beyond the " + std::to_string(idx->loc_hits) + " hits of the last locate or mems");
 }
 
 int sufr_b200_index_hits(SufrB200Index* idx, uint64_t first, uint64_t count, uint64_t* suffix, uint64_t* sequence,

@@ -240,6 +240,111 @@ __global__ void __launch_bounds__(256) hits_kernel(const void* sa, int wide, con
     sequence_pos[t] = l.sequence < 0 ? l.suffix : l.suffix - starts[l.sequence];
 }
 
+// ---- matching statistics and MEMs (include/sufr_b200.h gives the definitions) over the full suffix array of an index
+// without a seed mask: ms[i] = the longest l <= min(m - i, cap) such that q[i, i+l) starts an indexed suffix, and the
+// rank range of the suffixes it starts.
+
+// The insertion rank of q: the first rank whose suffix does not sort before q.  search_first's binary search with LCP
+// skipping, without its stop at the first equal suffix.
+__device__ uint64_t search_insert(const Params& P, const uint8_t* q, uint64_t qlen) {
+    long long low = 0, high = (long long)P.len - 1;
+    uint64_t left_lcp = 0, right_lcp = 0;
+    while (high >= low) {
+        const long long mid = low + (high - low) / 2;
+        const Comparison c = compare(P, q, qlen, entry(P.sa, mid, P.wide), left_lcp < right_lcp ? left_lcp : right_lcp);
+        if (c.cmp == 1) { low = mid + 1; left_lcp = c.lcp; }
+        else { high = mid - 1; right_lcp = c.lcp; }
+    }
+    return (uint64_t)low;
+}
+
+// bytes q[0, qlen) shares with the suffix at p
+__device__ __forceinline__ uint64_t common_prefix(const Params& P, const uint8_t* q, uint64_t qlen, uint64_t p) {
+    const uint64_t limit = qlen < P.n - p ? qlen : P.n - p;
+    uint64_t c = 0;
+    while (c < limit && q[c] == P.text[p + c]) c++;
+    return c;
+}
+
+// One thread per byte j of the batch (total = offsets[num_queries]); its query is the last one starting at or before
+// j.  The suffix sharing the longest prefix with q[i..] is a neighbour of its insertion rank r, so
+// ms = max(lcp(q[i..], SA[r-1]), lcp(q[i..], SA[r])), then the range of q[i, i+ms) by search_first / search_last.
+// P searches the full array (rank == NULL) with no run-time cap; P.build_mql caps the query as it caps the order.
+__global__ void __launch_bounds__(128) matching_stats_kernel(Params P, const uint8_t* __restrict__ queries,
+                                                             const unsigned long long* __restrict__ offsets,
+                                                             uint64_t num_queries, uint64_t total,
+                                                             unsigned long long* __restrict__ match_len,
+                                                             unsigned long long* __restrict__ rank_begin,
+                                                             unsigned long long* __restrict__ rank_end) {
+    const uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= total) return;
+    const long long qi = last_at_or_below(offsets, num_queries + 1, j);
+    const uint8_t* q = queries + j;
+    uint64_t len = offsets[qi + 1] - j;
+    if (P.build_mql > 0 && len > P.build_mql) len = P.build_mql;
+    uint64_t ms = 0;
+    if (P.len) {
+        const uint64_t r = search_insert(P, q, len);
+        if (r > 0) ms = common_prefix(P, q, len, entry(P.sa, r - 1, P.wide));
+        if (r < P.len) {
+            const uint64_t next = common_prefix(P, q, len, entry(P.sa, r, P.wide));
+            if (next > ms) ms = next;
+        }
+    }
+    match_len[j] = ms;
+    rank_begin[j] = ~0ull;
+    rank_end[j] = ~0ull;
+    if (ms == 0) return;
+    const long long first = search_first(P, q, ms);  // (>= 0: a suffix starts with q[0, ms))
+    long long last = search_last(P, q, ms, first);
+    if (last < 0) last = first;
+    rank_begin[j] = (unsigned long long)first;
+    rank_end[j] = (unsigned long long)last + 1;
+}
+
+// Byte j starts a MEM iff ms[j] >= min_len and (it starts its query or ms[j-1] <= ms[j]).
+struct MemFlagIn {
+    const unsigned long long* ms;
+    const unsigned long long* offsets;
+    uint64_t num_queries;
+    uint64_t min_len;
+    __device__ unsigned long long operator()(uint64_t j) const {
+        if (ms[j] < min_len) return 0ull;
+        if (j == 0 || ms[j - 1] <= ms[j]) return 1ull;
+        return offsets[last_at_or_below(offsets, num_queries + 1, j)] == j ? 1ull : 0ull;
+    }
+};
+// The compaction stores only where MEM incl - 1 starts (no loads between its stores, scan.cuh); mem_fill_kernel
+// gathers the rest.
+struct MemOut {
+    unsigned long long* at;
+    __device__ void operator()(uint64_t j, unsigned long long v, unsigned long long incl) const {
+        if (v) at[incl - 1] = j;
+    }
+};
+
+// One thread per MEM k starting at byte at[k] of the batch: its query, position in the query, length and rank range.
+__global__ void __launch_bounds__(256) mem_fill_kernel(const unsigned long long* __restrict__ at, uint64_t mems,
+                                                       const unsigned long long* __restrict__ ms,
+                                                       const unsigned long long* __restrict__ rb,
+                                                       const unsigned long long* __restrict__ re,
+                                                       const unsigned long long* __restrict__ offsets,
+                                                       uint64_t num_queries, unsigned long long* __restrict__ mem_query,
+                                                       unsigned long long* __restrict__ mem_pos,
+                                                       unsigned long long* __restrict__ mem_len,
+                                                       unsigned long long* __restrict__ begin,
+                                                       unsigned long long* __restrict__ end) {
+    const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= mems) return;
+    const uint64_t j = at[k];
+    const long long q = last_at_or_below(offsets, num_queries + 1, j);
+    mem_query[k] = (unsigned long long)q;
+    mem_pos[k] = j - offsets[q];
+    mem_len[k] = ms[j];
+    begin[k] = rb[j];
+    end[k] = re[j];
+}
+
 // ---- extract / list (SufrFile::extract, SufrFile::list): one thread per hit or rank computes the text region
 // [src, src + len) of its entry; an inclusive scan of the lengths (ArrayIn + HitOffsetOut) gives the byte offsets of
 // the entries in the output, and gather_regions_kernel copies the regions there.
