@@ -1,26 +1,19 @@
 // The scatter kernel of the stable LSD radix sort of (key, value) pairs, 8-bit digits (driver: radix_sort.cuh).
 //
 // onesweep_kernel ranks the records of a tile (one vote per digit bit + a per-warp counter chain: stable), exchanges
-// them through shared memory and writes digit-contiguous runs.  Input tiles arrive by TMA bulk copies
-// (cp.async.bulk + mbarrier): one elected thread issues two copies per tile instead of every thread issuing a
-// dozen cp.async, which matters in a kernel bound by instruction issue.  Two ways to obtain the global offsets
-// (template parameter LB), both measured on B200 by tools/ubench/sort_bench.cu (profiles/r2_sort_bench_*.txt):
-//   LB == 0  COUNT MATRIX (what the build uses): every block owns a run of consecutive tiles; a counting pass over
-//            the keys fills a [digit][block] matrix whose exclusive scan gives each block its write cursors.
-//   LB  > 0  ONE SWEEP: tiles are handed out by a ticket counter; a tile publishes its per-digit counts and derives
-//            its offsets by DECOUPLED LOOK-BACK over the tiles before it (status words: state | epoch | value, one
-//            64-bit word per (tile, digit), relaxed gpu-scope loads / stores), and counts the NEXT digit of every key
-//            into the next pass's global histogram on the way out, so no pass reads the keys a second time.
-// Measured: per-pass time = 5.6 ms + 16 ns x tiles at 2^30 records for every variant, i.e. large tiles win and the
-// look-back only pays back the counting pass once tiles are large (8.5 vs 7.7 + 1.3 ms); with 2048-record tiles the
-// look-back chain serialises (45-100 ms per pass).  The count matrix is deterministic and has no spin-waits.
+// them through shared memory and writes digit-contiguous runs.  Every block owns a run of consecutive tiles and takes
+// its write cursors from the exclusive scan of a [digit][block] count matrix, filled by a counting pass over the keys.
+// The next tile arrives by TMA bulk copies (cp.async.bulk + mbarrier) while this one is processed: one elected thread
+// issues two copies per tile instead of every thread issuing a dozen cp.async, which matters in a kernel bound by
+// instruction issue.  The name is historical: a one-sweep variant (decoupled look-back over tile status words, the
+// next digit counted on the way out) and other ways of staging a tile were measured on B200 with
+// tools/ubench/sort_bench.cu and lost (profiles/r2_sort_bench_*.txt).  Per-pass time is 5.6 ms + 16 ns per tile at
+// 2^30 records, so large tiles win; at that size the look-back saved less than its cost (8.5 ms against 7.7 + 1.3 ms
+// with the counting pass), and on small tiles its chain serialises.  The count matrix is deterministic and has no
+// spin-waits.  The removed variants are in the history up to commit 44af2d3.
 //
 // Algorithmic bytes per pass and element: 2 * (sizeof(K) + sizeof(V)) (+ sizeof(K) for the counting pass).
 #pragma once
-#include <algorithm>
-#include <utility>
-#include <vector>
-
 #include "common.cuh"
 
 namespace sufr {
@@ -28,22 +21,6 @@ namespace osort {
 
 constexpr int RADIX_BITS = 8;
 constexpr int RADIX = 1 << RADIX_BITS;
-constexpr int kMaxPasses = 8;
-
-// ------------------------------------------------------------------ tile status words (decoupled look-back)
-constexpr int kEpochShift = 54;  // bits 61..54: pass number (stale words of an earlier pass read as "not ready")
-constexpr unsigned long long kStateLocal = 1ull << 62;  // value = records of this digit in this tile
-constexpr unsigned long long kStateIncl = 2ull << 62;   // value = records of this digit in tiles 0..this
-constexpr unsigned long long kValueMask = (1ull << kEpochShift) - 1;
-
-__device__ __forceinline__ void st_relaxed_u64(unsigned long long* p, unsigned long long v) {
-    asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ unsigned long long ld_relaxed_u64(const unsigned long long* p) {
-    unsigned long long v;
-    asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
 
 // ------------------------------------------------------------------ TMA bulk copy global -> shared, mbarrier
 __device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -80,79 +57,29 @@ __device__ __forceinline__ uint32_t digit_of(K key, int shift, uint32_t dmask) {
     return (uint32_t)(key >> shift) & dmask;
 }
 
-// ------------------------------------------------------------------ histogram of all digits, one read of the keys
-// hist[p][d] += number of keys whose digit of pass p (bits [begin_bit + 8p, +8), the last pass may be narrower) is d.
-template <typename K>
-__global__ void __launch_bounds__(256) hist_kernel(const K* __restrict__ keys, uint64_t n, int begin_bit, int end_bit,
-                                                   unsigned long long* __restrict__ hist) {
-    __shared__ uint32_t sh[kMaxPasses][RADIX];
-    const int passes = (end_bit - begin_bit + RADIX_BITS - 1) / RADIX_BITS;
-    for (int i = threadIdx.x; i < passes * RADIX; i += 256) (&sh[0][0])[i] = 0;
-    __syncthreads();
-    // a block walks contiguous chunks so that its counters stay below 2^32
-    const uint64_t per_block = (n + gridDim.x - 1) / gridDim.x;
-    const uint64_t begin = (uint64_t)blockIdx.x * per_block;
-    const uint64_t end = begin + per_block < n ? begin + per_block : n;
-    for (uint64_t i0 = begin + threadIdx.x; i0 < end; i0 += 256 * 4) {
-        K k[4];
-#pragma unroll
-        for (int u = 0; u < 4; u++) k[u] = i0 + 256 * u < end ? keys[i0 + 256 * u] : (K)0;  // four loads in flight
-#pragma unroll
-        for (int u = 0; u < 4; u++) {
-            if (i0 + 256 * u >= end) break;
-#pragma unroll
-            for (int p = 0; p < kMaxPasses; p++) {
-                if (p < passes) {
-                    const int bit = begin_bit + p * RADIX_BITS;
-                    const int nb = end_bit - bit < RADIX_BITS ? end_bit - bit : RADIX_BITS;
-                    atomicAdd(&sh[p][digit_of(k[u], bit, (1u << nb) - 1u)], 1u);
-                }
-            }
-        }
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < passes * RADIX; i += 256) {
-        const uint32_t c = (&sh[0][0])[i];
-        if (c) atomicAdd(&hist[i], (unsigned long long)c);
-    }
-}
-
 // ------------------------------------------------------------------ one pass
-enum : int {
-    kRegsDirect = 0,  // records loaded straight into registers (coalesced), one exchange buffer
-    kRegsBulk = 1,    // next tile staged by TMA bulk copy while this one is processed; records held in registers
-    kDigitsBulk = 2,  // staged tile; registers hold only digits and ranks, records go stage -> exchange buffer
-};
-
-template <typename K, typename V, int BLOCK, int IPT, int MODE>
+template <typename K, typename V, int BLOCK, int IPT>
 struct PassConfig {
     static constexpr int TILE = BLOCK * IPT;
     static constexpr int WARPS = BLOCK / 32;
     static constexpr size_t record = sizeof(K) + sizeof(V);
-    static constexpr size_t dyn_smem = (MODE == kRegsDirect ? 1 : 2) * record * TILE;
+    static constexpr size_t dyn_smem = 2 * record * TILE;  // exchange buffer + staged next tile
 };
 
-// LB > 0: tiles by ticket, offsets by decoupled look-back that inspects LB predecessors per round trip.
-// LB == 0: every block owns `tiles_per_block` consecutive tiles and takes its starting offsets from a scanned
-//          [digit][block] count matrix `bases` (needs a counting pass over the keys first).
-template <typename K, typename V, int BLOCK, int IPT, int MINCTAS, int MODE, int LB>
+// Every block owns `tiles_per_block` consecutive tiles and takes its starting offsets from a scanned [digit][block]
+// count matrix `bases`.  Records are held in registers between the staging buffer and the exchange buffer.
+template <typename K, typename V, int BLOCK, int IPT, int MINCTAS>
 __global__ void __launch_bounds__(BLOCK, MINCTAS)
     onesweep_kernel(const K* __restrict__ kin, K* __restrict__ kout, const V* __restrict__ vin, V* __restrict__ vout,
-                    uint64_t n, int shift, uint32_t dmask, const unsigned long long* __restrict__ hist,
-                    unsigned long long* __restrict__ next_hist, int next_shift, uint32_t next_dmask,
-                    unsigned long long* __restrict__ status, unsigned int* __restrict__ ticket, uint32_t epoch,
-                    const uint32_t* __restrict__ bases, uint32_t tiles_per_block) {
-    using Cfg = PassConfig<K, V, BLOCK, IPT, MODE>;
+                    uint64_t n, int shift, uint32_t dmask, const uint32_t* __restrict__ bases, uint32_t tiles_per_block) {
+    using Cfg = PassConfig<K, V, BLOCK, IPT>;
     constexpr int TILE = Cfg::TILE, WARPS = Cfg::WARPS;
     static_assert(BLOCK >= RADIX && BLOCK % 32 == 0, "thread d owns digit d");
     static_assert(TILE <= 65535, "tile-local slots are 16-bit");
     __shared__ uint16_t wc[WARPS][RADIX];  // per-warp digit counters -> tile-local start of (warp, digit)
     __shared__ uint32_t goff[RADIX];       // global index = goff[d] + tile-local slot (mod 2^32)
-    __shared__ uint32_t nh[RADIX];         // next pass's digit histogram of the records this block moved
     __shared__ uint32_t wtot[RADIX / 32];
-    __shared__ unsigned long long wtot64[RADIX / 32];
-    __shared__ uint32_t tile_s[2];
-    __shared__ uint32_t running[LB == 0 ? RADIX : 1];  // LB == 0: global write cursor of each digit for this block
+    __shared__ uint32_t running[RADIX];    // global write cursor of each digit for this block
     __shared__ __align__(8) uint64_t bar;
     extern __shared__ __align__(128) unsigned char dyn[];
     K* exk = reinterpret_cast<K*>(dyn);
@@ -163,37 +90,13 @@ __global__ void __launch_bounds__(BLOCK, MINCTAS)
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const uint32_t lt_mask = (1u << lane) - 1u;
     const uint64_t total_tiles = (n + TILE - 1) / TILE;
-    const unsigned long long ep = (unsigned long long)epoch << kEpochShift;
 
-    // global start of every digit: exclusive scan of this pass's histogram (thread d owns digit d)
-    unsigned long long base = 0;
-    {
-        const unsigned long long c = (LB > 0 && tid < RADIX) ? hist[tid] : 0ull;
-        unsigned long long incl = c;
-#pragma unroll
-        for (int off = 1; off < 32; off <<= 1) {
-            const unsigned long long o = __shfl_up_sync(0xffffffffu, incl, off);
-            if (lane >= off) incl += o;
-        }
-        if (tid < RADIX && lane == 31) wtot64[warp] = incl;
-        if (tid < RADIX) nh[tid] = 0;
-        if (LB == 0 && tid < RADIX) running[tid] = bases[(uint64_t)tid * gridDim.x + blockIdx.x];
-        if (tid == 0) {
-            if (LB > 0) tile_s[0] = atomicAdd(ticket, 1u);
-            if (MODE != kRegsDirect) {
-                mbar_init(&bar, 1);
-                asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-            }
-        }
-        __syncthreads();
-        if (tid < RADIX) {
-            unsigned long long prefix = 0;
-#pragma unroll
-            for (int w = 0; w < RADIX / 32; w++)
-                if (w < warp) prefix += wtot64[w];
-            base = prefix + incl - c;
-        }
+    if (tid < RADIX) running[tid] = bases[(uint64_t)tid * gridDim.x + blockIdx.x];
+    if (tid == 0) {
+        mbar_init(&bar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
+    __syncthreads();
 
     auto issue = [&](uint64_t t) {  // one thread: stage tile t
         const uint64_t tb = t * TILE;
@@ -205,53 +108,33 @@ __global__ void __launch_bounds__(BLOCK, MINCTAS)
         bulk_g2s(pv, vin + tb, vb, &bar);
     };
 
-    uint64_t tile = LB > 0 ? (uint64_t)tile_s[0] : (uint64_t)blockIdx.x * tiles_per_block;
-    uint64_t last_tile = total_tiles;  // LB == 0: end of this block's run of tiles
-    if (LB == 0) {
-        last_tile = tile + tiles_per_block < total_tiles ? tile + tiles_per_block : total_tiles;
-        if (tile >= last_tile) tile = total_tiles;
-    }
+    uint64_t tile = (uint64_t)blockIdx.x * tiles_per_block;
+    const uint64_t last_tile = tile + tiles_per_block < total_tiles ? tile + tiles_per_block : total_tiles;
+    if (tile >= last_tile) tile = total_tiles;
     uint32_t parity = 0;
-    if (MODE != kRegsDirect) {
-        if (tid == 0 && tile < total_tiles) issue(tile);
-    }
-    int tb2 = 0;
+    if (tid == 0 && tile < total_tiles) issue(tile);
     while (tile < total_tiles) {
         const uint64_t tbase = tile * TILE;
         const uint32_t count = (n - tbase) < (uint64_t)TILE ? (uint32_t)(n - tbase) : (uint32_t)TILE;
-        if (LB > 0 && tid == 0) tile_s[tb2 ^ 1] = atomicAdd(ticket, 1u);
 
-        K key[MODE == kDigitsBulk ? 1 : IPT];
-        V val[MODE == kDigitsBulk ? 1 : IPT];
-        if (MODE != kRegsDirect) {
-            mbar_wait(&bar, parity);
-            parity ^= 1u;
-            if (count < (uint32_t)TILE) {  // block-uniform: padding records get the largest key
-                for (uint32_t i = count + tid; i < (uint32_t)TILE; i += BLOCK) pk[i] = ~(K)0;
-                __syncthreads();
-            }
+        K key[IPT];
+        V val[IPT];
+        mbar_wait(&bar, parity);
+        parity ^= 1u;
+        if (count < (uint32_t)TILE) {  // block-uniform: padding records get the largest key
+            for (uint32_t i = count + tid; i < (uint32_t)TILE; i += BLOCK) pk[i] = ~(K)0;
+            __syncthreads();
         }
-        if (MODE == kRegsBulk) {
 #pragma unroll
-            for (int i = 0; i < IPT; i++) {
-                const uint32_t idx = warp * (32 * IPT) + i * 32 + lane;
-                key[i] = pk[idx];
-                val[i] = pv[idx];
-            }
-        } else if (MODE == kRegsDirect) {
-#pragma unroll
-            for (int i = 0; i < IPT; i++) {
-                const uint32_t idx = warp * (32 * IPT) + i * 32 + lane;
-                key[i] = idx < count ? kin[tbase + idx] : ~(K)0;
-                val[i] = idx < count ? vin[tbase + idx] : (V)0;
-            }
+        for (int i = 0; i < IPT; i++) {
+            const uint32_t idx = warp * (32 * IPT) + i * 32 + lane;
+            key[i] = pk[idx];
+            val[i] = pv[idx];
         }
         for (int i = tid; i < WARPS * RADIX / 2; i += BLOCK) reinterpret_cast<uint32_t*>(&wc[0][0])[i] = 0;
-        __syncthreads();  // (A) counters zero, staged records copied to registers, next ticket visible
-        const uint64_t next = LB > 0 ? (uint64_t)tile_s[tb2 ^ 1] : (tile + 1 < last_tile ? tile + 1 : total_tiles);
-        if (MODE == kRegsBulk) {
-            if (tid == 0 && next < total_tiles) issue(next);
-        }
+        __syncthreads();  // (A) counters zero, staged records copied to registers
+        const uint64_t next = tile + 1 < last_tile ? tile + 1 : total_tiles;
+        if (tid == 0 && next < total_tiles) issue(next);
 
         // ---- rank inside the warp's slice of the tile, rows in tile order => stable
         uint32_t dpack[(IPT + 3) / 4];   // digits, four per register
@@ -262,8 +145,7 @@ __global__ void __launch_bounds__(BLOCK, MINCTAS)
         for (int i = 0; i < (IPT + 1) / 2; i++) spack[i] = 0;
 #pragma unroll
         for (int i = 0; i < IPT; i++) {
-            const uint32_t idx = warp * (32 * IPT) + i * 32 + lane;
-            const uint32_t d = digit_of(MODE == kDigitsBulk ? pk[idx] : key[i], shift, dmask);
+            const uint32_t d = digit_of(key[i], shift, dmask);
             unsigned peers = 0xffffffffu;
 #pragma unroll
             for (int b = 0; b < RADIX_BITS; b++) {
@@ -285,7 +167,7 @@ __global__ void __launch_bounds__(BLOCK, MINCTAS)
         }
         __syncthreads();  // (B)
 
-        // ---- thread d owns digit d: records per digit in the tile, tile-local starts, publication
+        // ---- thread d owns digit d: records per digit in the tile, tile-local starts
         uint32_t tile_count = 0, incl = 0;
         if (tid < RADIX) {
 #pragma unroll
@@ -314,65 +196,24 @@ __global__ void __launch_bounds__(BLOCK, MINCTAS)
             for (int w = 0; w < WARPS; w++) wc[w][tid] = (uint16_t)(wc[w][tid] + tile_start);
             // the padding of a partial tile was counted under the largest digit
             published = tile_count - ((uint32_t)tid == dmask ? (uint32_t)TILE - count : 0u);
-            if (LB > 0) st_relaxed_u64(status + tile * RADIX + tid, (tile == 0 ? kStateIncl : kStateLocal) | ep | published);
         }
         __syncthreads();  // (D) tile-local starts final
 
         // ---- exchange through shared memory so that the global writes are digit-contiguous
 #pragma unroll
         for (int i = 0; i < IPT; i++) {
-            const uint32_t idx = warp * (32 * IPT) + i * 32 + lane;
             const uint32_t d = (dpack[i >> 2] >> (8 * (i & 3))) & 0xFFu;
             const uint32_t s = ((spack[i >> 1] >> (16 * (i & 1))) & 0xFFFFu) + wc[warp][d];
-            if (MODE == kDigitsBulk) {
-                exk[s] = pk[idx];
-                exv[s] = pv[idx];
-            } else {
-                exk[s] = key[i];
-                exv[s] = val[i];
-            }
+            exk[s] = key[i];
+            exv[s] = val[i];
         }
-        // ---- decoupled look-back: records of digit d in all tiles before this one.  LB status words are fetched
-        //      per round trip (independent loads) and consumed in order up to the first inclusive prefix.
         if (tid < RADIX) {
-            if (LB > 0) {
-                unsigned long long excl = 0;
-                if (tile > 0) {
-                    constexpr int W = LB > 0 ? LB : 1;
-                    uint64_t p = tile;  // tiles [p, tile) are summed already
-                    for (;;) {
-                        unsigned long long w[W];
-#pragma unroll
-                        for (int j = 0; j < W; j++)
-                            w[j] = p > (uint64_t)j ? ld_relaxed_u64(status + (p - 1 - j) * RADIX + tid) : (kStateIncl | ep);
-                        int used = 0;
-                        bool fin = false;
-#pragma unroll
-                        for (int j = 0; j < W; j++) {
-                            const unsigned long long x = w[j];
-                            if (!fin && used == j && (x & (0xFFull << kEpochShift)) == ep && (x >> 62) != 0) {
-                                excl += x & kValueMask;
-                                used = j + 1;
-                                fin = (x >> 62) == 2;
-                            }
-                        }
-                        if (fin) break;
-                        p -= used;
-                    }
-                    st_relaxed_u64(status + tile * RADIX + tid, kStateIncl | ep | (excl + published));
-                }
-                goff[tid] = (uint32_t)(base + excl - tile_start);
-            } else {
-                goff[tid] = running[tid] - tile_start;
-                running[tid] += published;
-            }
+            goff[tid] = running[tid] - tile_start;
+            running[tid] += published;
         }
-        __syncthreads();  // (E) exchange buffer and offsets complete; the staged tile has been consumed
-        if (MODE == kDigitsBulk) {
-            if (tid == 0 && next < total_tiles) issue(next);
-        }
+        __syncthreads();  // (E) exchange buffer and offsets complete
 
-        // ---- coalesced scatter; the next pass's histogram is counted on the way out
+        // ---- coalesced scatter
 #pragma unroll
         for (int k = 0; k < IPT; k++) {
             const uint32_t s = k * BLOCK + tid;
@@ -381,44 +222,10 @@ __global__ void __launch_bounds__(BLOCK, MINCTAS)
                 const uint32_t dst = goff[digit_of(kk, shift, dmask)] + s;
                 kout[dst] = kk;
                 vout[dst] = exv[s];
-                if (next_hist) atomicAdd(&nh[digit_of(kk, next_shift, next_dmask)], 1u);
             }
         }
         tile = next;
-        tb2 ^= 1;
     }
-    __syncthreads();
-    if (next_hist && tid < RADIX && nh[tid]) atomicAdd(&next_hist[tid], (unsigned long long)nh[tid]);
-}
-
-// ------------------------------------------------------------------ host side of the look-back variant
-// (measured in tools/ubench/sort_bench.cu; the build itself uses the count-matrix driver in radix_sort.cuh)
-// Scratch memory of one sort call: digit histograms, one ticket counter per pass, tile status words.
-struct Scratch {
-    static size_t header_bytes() { return (size_t)kMaxPasses * RADIX * 8 + 256; }
-    static size_t bytes(uint64_t n, int tile) { return header_bytes() + (size_t)div_up(n ? n : 1, tile) * RADIX * 8; }
-    explicit Scratch(void* p) : base((unsigned char*)p) {}
-    unsigned long long* hist(int pass) const { return reinterpret_cast<unsigned long long*>(base) + (size_t)pass * RADIX; }
-    unsigned int* ticket(int pass) const { return reinterpret_cast<unsigned int*>(base + (size_t)kMaxPasses * RADIX * 8) + pass; }
-    unsigned long long* status() const { return reinterpret_cast<unsigned long long*>(base + header_bytes()); }
-    unsigned char* base;
-};
-
-template <typename K, typename V, int BLOCK, int IPT, int CTAS, int MODE, int LB>
-void launch_pass(const K* kin, K* kout, const V* vin, V* vout, uint64_t n, int bit, int nb, int next_bit, int next_nb,
-                 const Scratch& sc, int pass, bool count_next, cudaStream_t stream) {
-    static_assert(LB > 0, "the count-matrix variant is launched by rsort::sort_pairs");
-    using Cfg = PassConfig<K, V, BLOCK, IPT, MODE>;
-    static bool attr_set[64] = {};
-    auto kern = onesweep_kernel<K, V, BLOCK, IPT, CTAS, MODE, LB>;
-    allow_dynamic_smem(kern, Cfg::dyn_smem, attr_set);
-    const uint64_t tiles = div_up(n, Cfg::TILE);
-    const uint32_t grid = (uint32_t)std::min<uint64_t>(tiles, (uint64_t)num_sms() * CTAS);
-    kern<<<grid, BLOCK, Cfg::dyn_smem, stream>>>(kin, kout, vin, vout, n, bit, (1u << nb) - 1u, sc.hist(pass),
-                                                 count_next ? sc.hist(pass + 1) : nullptr, next_bit,
-                                                 (1u << (next_nb > 0 ? next_nb : 1)) - 1u, sc.status(), sc.ticket(pass),
-                                                 (uint32_t)(pass + 1), nullptr, 0u);
-    SUFR_KERNEL_CHECK();
 }
 
 }  // namespace osort

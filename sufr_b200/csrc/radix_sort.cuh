@@ -3,14 +3,14 @@
 // Per pass:  count    (digit histogram of the run of tiles each scatter block owns -> [digit][block] matrix;
 //                      several counting blocks per scatter block, merged with global atomics)
 //            scan     (exclusive scan of the matrix, digit-major)
-//            scatter  (osort::onesweep_kernel with LB == 0, onesweep.cuh: per tile warp-level vote ranking ->
-//                      block digit offsets -> shared-memory exchange -> coalesced scatter of keys, then values;
+//            scatter  (osort::onesweep_kernel, onesweep.cuh: per tile warp-level vote ranking -> block digit
+//                      offsets -> shared-memory exchange -> coalesced scatter of keys, then values;
 //                      the next tile arrives by a TMA bulk copy while this one is processed)
 // One persistent scatter block of 512 threads per SM, tiles of 8192 records: every block owns a contiguous run of
 // tiles, so the only global state is the 256 x G count matrix (no inter-block dependencies, no look-back spinning).
-// Tile size, block shape and the look-back alternative were chosen from tools/ubench/sort_bench.cu on B200
-// (profiles/r2_sort_bench_*.txt): per-pass time is 5.6 ms + 16 ns per tile at 2^30 records, so the largest tile
-// that fits two buffers in 227 KB of shared memory wins.
+// Tile size and block shape were chosen from tools/ubench/sort_bench.cu on B200 (profiles/r2_sort_bench_*.txt):
+// per-pass time is 5.6 ms + 16 ns per tile at 2^30 records, so the largest tile that fits two buffers in 227 KB of
+// shared memory wins.
 //
 // Algorithmic bytes per pass and element: sizeof(K) (count read) + 2*(sizeof(K)+sizeof(V)) (scatter read + write).
 #pragma once
@@ -32,7 +32,6 @@ struct Tuning {
     static constexpr int BLOCK = 512;
     static constexpr int IPT = (sizeof(K) + sizeof(V) > 12) ? 12 : 16;  // two tile buffers within 227 KB
     static constexpr int CTAS = 1;
-    static constexpr int MODE = osort::kRegsBulk;
     static constexpr int TILE = BLOCK * IPT;
 };
 
@@ -143,11 +142,11 @@ bool sort_pairs(K* keys_a, K* keys_b, V* vals_a, V* vals_b, uint64_t n, int begi
                 uint32_t* counts, cudaStream_t stream, uint64_t* launches = nullptr,
                 EventPairs* scatter_events = nullptr) {
     using T = Tuning<K, V>;
-    using Cfg = osort::PassConfig<K, V, T::BLOCK, T::IPT, T::MODE>;
+    using Cfg = osort::PassConfig<K, V, T::BLOCK, T::IPT>;
     if (n == 0 || end_bit <= begin_bit) return false;
     if (n > 0xFFFFFFFFull) throw Error(3, "rsort: more than 2^32 records need 64-bit write cursors");
     const Plan p = make_plan<K, V>(n);
-    auto kern = osort::onesweep_kernel<K, V, T::BLOCK, T::IPT, T::CTAS, T::MODE, 0>;
+    auto kern = osort::onesweep_kernel<K, V, T::BLOCK, T::IPT, T::CTAS>;
     static bool attr_set[64] = {};  // per instantiation and device
     allow_dynamic_smem(kern, Cfg::dyn_smem, attr_set);
     const uint64_t owner_records = (uint64_t)p.tiles_per_block * T::TILE;
@@ -171,8 +170,7 @@ bool sort_pairs(K* keys_a, K* keys_b, V* vals_a, V* vals_b, uint64_t n, int begi
             SUFR_CUDA_CHECK(cudaEventCreate(&e1));
             SUFR_CUDA_CHECK(cudaEventRecord(e0, stream));
         }
-        kern<<<p.grid, T::BLOCK, Cfg::dyn_smem, stream>>>(kin, kout, vin, vout, n, bit, dmask, nullptr, nullptr, 0, 0u,
-                                                          nullptr, nullptr, 0u, counts, p.tiles_per_block);
+        kern<<<p.grid, T::BLOCK, Cfg::dyn_smem, stream>>>(kin, kout, vin, vout, n, bit, dmask, counts, p.tiles_per_block);
         SUFR_KERNEL_CHECK();
         if (scatter_events) {
             SUFR_CUDA_CHECK(cudaEventRecord(e1, stream));
@@ -182,22 +180,6 @@ bool sort_pairs(K* keys_a, K* keys_b, V* vals_a, V* vals_b, uint64_t n, int begi
         in_b = !in_b;
     }
     return in_b;
-}
-
-// One scatter pass whose (scanned) count matrix the caller provides -- e.g. counted by the kernel that produced the
-// keys.  The matrix must follow make_plan<K, V>(n).
-template <typename K, typename V>
-void scatter_pass(const K* kin, K* kout, const V* vin, V* vout, uint64_t n, int bit, int nb, const uint32_t* counts,
-                  cudaStream_t stream) {
-    using T = Tuning<K, V>;
-    using Cfg = osort::PassConfig<K, V, T::BLOCK, T::IPT, T::MODE>;
-    const Plan p = make_plan<K, V>(n);
-    auto kern = osort::onesweep_kernel<K, V, T::BLOCK, T::IPT, T::CTAS, T::MODE, 0>;
-    static bool attr_set[64] = {};
-    allow_dynamic_smem(kern, Cfg::dyn_smem, attr_set);
-    kern<<<p.grid, T::BLOCK, Cfg::dyn_smem, stream>>>(kin, kout, vin, vout, n, bit, (1u << nb) - 1u, nullptr, nullptr, 0, 0u,
-                                                      nullptr, nullptr, 0u, counts, p.tiles_per_block);
-    SUFR_KERNEL_CHECK();
 }
 
 }  // namespace rsort

@@ -1,7 +1,7 @@
 // Device-wide inclusive scan with functor input/output (reduce -> spine -> apply).
 //
 // Used for every order-preserving compaction on the path (active-group compaction, shard
-// selection, suffix filter) and for the max / segmented-min scans of the refinement stages.
+// selection, suffix filter) and for the max scans of the refinement stages.
 // Three launches, two coalesced reads of the input functor, no inter-block dependencies
 // (so no forward-progress assumptions).  The operator must be associative; it need not commute.
 #pragma once
@@ -31,17 +31,6 @@ struct MaxU32 {
     using T = uint32_t;
     __host__ __device__ static T identity() { return 0; }
     __device__ T operator()(T a, T b) const { return a > b ? a : b; }
-};
-// Segmented min over packed (flag << 32 | value): a set flag on the right operand restarts the segment.
-struct SegMinU64 {
-    using T = unsigned long long;
-    __host__ __device__ static T identity() { return 0x00000000FFFFFFFFull; }
-    __device__ T operator()(T a, T b) const {
-        uint32_t fa = (uint32_t)(a >> 32), fb = (uint32_t)(b >> 32);
-        uint32_t va = (uint32_t)a, vb = (uint32_t)b;
-        uint32_t v = fb ? vb : (va < vb ? va : vb);
-        return ((T)(fa | fb) << 32) | v;
-    }
 };
 
 // Input functors whose values are flags declare it, and the kernels scan them with warp votes instead of shuffles

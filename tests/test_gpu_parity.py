@@ -621,32 +621,29 @@ def test_fast2_deep_repeats_and_shards(S):
         assert np.array_equal(np.concatenate([s.lcp for s in shards]), want.lcp)
 
 
-@pytest.mark.parametrize("fuse", ["1", "0"])
+@pytest.mark.parametrize("world", [2, 3, 8, 33])
 @pytest.mark.parametrize("kw", [dict(is_dna=True), dict(is_dna=True, allow_ambiguity=True), dict()],
                          ids=["filtered", "ambiguity", "bytes"])
-def test_shard_selection_fused_with_first_radix_pass(S, monkeypatch, fuse, kw):
-    """Key-range shards select their records and sort them in four passes; the variant that generates them already in
-    first-digit order (selection fused with key generation and the first radix pass, SUFR_B200_DEBUG_SHARD_FUSE=1:
-    measured, not the default) must give the same arrays.  Both ways for 2, 3, 8 and 33 shards (some of them empty)."""
+def test_shard_selection_many_shards(S, world, kw):
+    """Key-range shards select their records without sorting them, then sort them in four passes: the concatenated
+    shards must give the single-process arrays, for 2, 3, 8 and 33 shards (some of them empty)."""
     from sufr_b200.distributed import previous_last_suffix, shard_layout
-    monkeypatch.setenv("SUFR_B200_DEBUG_SHARD_FUSE", fuse)
-    rng = random.Random(len(kw) + int(fuse))
+    rng = random.Random(len(kw))
     text = dna_with_rare(rng, 90000) + b"ACGT" * 300 + rand_text(rng, 20000, b"ACGT", repeat_p=0.05, max_rep=200)[:-1] + b"$"
     want = O.oracle_build(text, threads=4, **kw)
-    for world in (2, 3, 8, 33):
-        shards = [S.build(S.SufrBuilderArgs(text=text, **kw), rank=r, world_size=world) for r in range(world)]
-        meta = [(s.num_suffixes, s.first_suffix, s.last_suffix) for s in shards]
-        offs, total = shard_layout(meta)
-        assert total == want.num_suffixes
-        for r, sh in enumerate(shards):
-            sh.set_shard_layout(offs[r], total)
-            prev = previous_last_suffix(meta, r)
-            if prev is not None and sh.num_suffixes:
-                sh.patch_seam(prev)
-        assert np.array_equal(np.concatenate([sh.sa for sh in shards]), want.sa)
-        assert np.array_equal(np.concatenate([sh.lcp for sh in shards]), want.lcp)
-        for sh in shards:
-            sh.free()
+    shards = [S.build(S.SufrBuilderArgs(text=text, **kw), rank=r, world_size=world) for r in range(world)]
+    meta = [(s.num_suffixes, s.first_suffix, s.last_suffix) for s in shards]
+    offs, total = shard_layout(meta)
+    assert total == want.num_suffixes
+    for r, sh in enumerate(shards):
+        sh.set_shard_layout(offs[r], total)
+        prev = previous_last_suffix(meta, r)
+        if prev is not None and sh.num_suffixes:
+            sh.patch_seam(prev)
+    assert np.array_equal(np.concatenate([sh.sa for sh in shards]), want.sa)
+    assert np.array_equal(np.concatenate([sh.lcp for sh in shards]), want.lcp)
+    for sh in shards:
+        sh.free()
 
 
 def family_text(rng, n, seg_len=2000, copies=30, mut=0.01):
@@ -750,20 +747,24 @@ def test_cli_create_writes_golden_files(tmp_path, golden, fasta, flags):
     assert out.read_bytes() == (GOLDEN / "expected" / golden).read_bytes()
 
 
-def test_filter_after_full_sort_fast_and_generic_paths(S, monkeypatch):
+def test_filter_after_full_sort(S):
     """Repetitive DNA with scattered N: the filtered attempt gives up, everything is sorted with prefix
-    doubling, and the non-indexed suffixes are dropped afterwards -- by the look-back kernel, and (forced)
-    by the generic segmented-min scan.  A long N run overflows the look-back and takes the scan by itself."""
+    doubling, and the non-indexed suffixes are dropped afterwards by the block-summary kernels.  A long N run
+    spans many blocks, so a kept suffix after it takes its LCP from the per-block summaries.  A text with none of
+    $ACGT that the repetitiveness probe (2^24 positions or more) sends to the full sort keeps no suffix at all."""
     rng = random.Random(37)
     base = dna_with_rare(rng, 60000, rare=b"N", rare_p=0.01, repeat_p=0.0)
     text = base + base[:30000] + base[10000:50000] + b"$"      # long exact repeats => doubling
     _, _, doubling = gpu_vs_oracle(S, text, is_dna=True)
     assert doubling > 0
-    monkeypatch.setenv("SUFR_B200_DEBUG_SLOW_FILTER", "1")
-    gpu_vs_oracle(S, text, is_dna=True)
-    monkeypatch.delenv("SUFR_B200_DEBUG_SLOW_FILTER")
     text2 = base[:20000] + b"N" * 3000 + base[:20000] + b"N" * 700 + base[5000:15000] + b"$"
     gpu_vs_oracle(S, text2, is_dna=True)
+    text3 = bytearray(b"N" * ((1 << 24) + 4096))
+    text3[5::1_000_003] = b"#" * len(text3[5::1_000_003])
+    text3[7::3_000_017] = b"X" * len(text3[7::3_000_017])
+    # the reference cannot draw pivots from a text without ACGT$ positions: ask the oracle for none
+    _, _, doubling = gpu_vs_oracle(S, bytes(text3), is_dna=True, oracle_partitions=0)
+    assert doubling > 0
 
 
 def test_sharded_fallback_on_some_ranks_only(S):
