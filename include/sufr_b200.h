@@ -296,6 +296,47 @@ int sufr_b200_index_mems(SufrB200Index* index, const uint8_t* queries, const uin
                          uint64_t* mem_len, uint64_t* rank_begin, uint64_t* rank_end,
                          uint64_t* hit_offsets /* offsets[num_queries] + 1 */);
 
+/* -- k-mer counting on the device, on an index from index_open or index_create without a seed mask.  t = the text,
+ *    n its length, SA / LCP the full arrays (s entries), sequence starts c_0 < ... < c_{R-1}.  Records follow
+ *    index_extract: record i owns [c_i, c_{i+1}), the last one [c_{R-1}, n), positions before c_0 belong to [0, c_0);
+ *    an index without starts is one record [0, n).
+ *      occurrence  a position p of record [a, e) with p + k <= e - 1: the k bytes lie inside the record and never
+ *               include its last byte (the delimiter, or the final '$').  In a DNA index (is_dna) all k bytes are also
+ *               A, C, G or T, so k-mers with N are not counted.  Every occurrence is an indexed position.
+ *      group    the maximal rank run [b, e) with b == 0 || LCP[b] < k and LCP[r] >= k for b < r < e: the rank range
+ *               index_search returns for its first k bytes.  A group with at least one occurrence is one distinct
+ *               k-mer; its count is the number of its ranks that are occurrences (e - b in a DNA index; smaller in a
+ *               plain index only where a delimiter byte also appears inside a record).
+ *      k        1 <= k, and k <= the build's max_query_len when it has one (LCP values below it are exact, DESIGN.md
+ *               §3 item 4); a k above n gives no k-mers.
+ *    index_kmer_spectrum  histogram[i] = distinct k-mers with count i + 1 for i < num_bins - 1; histogram[num_bins - 1]
+ *               = those with count >= num_bins.  1 <= num_bins <= 65536.  distinct / occurrences / max_count may be
+ *               NULL.
+ *    index_kmers  the groups with b >= first_rank whose count lies in [max(min_count, 1), max_count] (UINT64_MAX = no
+ *               upper bound), in rank order (the byte order of the k-mers), at most max_kmers of them: rank_begin /
+ *               rank_end = [b, e), count, and the k bytes t[SA[b'], +k) at bytes[j * k ..], where b' is the group's
+ *               first occurrence (bytes may be NULL; it needs max_kmers * k bytes).  *next_rank = where the next window
+ *               starts: every group with first_rank <= b < *next_rank has been considered, and *next_rank == s at the
+ *               end.  A group that starts before first_rank is not listed.  A window costs time in proportion to the
+ *               ranks it covers, so an enumeration in windows is one pass over the arrays in total.
+ *    index_kmer_multiplicity  out[i] = the count of the k-mer at position first_pos + i if that position is an
+ *               occurrence, else 0; saturated at UINT32_MAX.  first_pos + num_positions <= n.  Each call is one pass
+ *               over the ranks, whatever the window (the first call for a k one more, whose per-rank counts, 4 s bytes,
+ *               are kept for the next windows).
+ *    Each call leaves the locate state of index_locate / index_mems as it was; the occurrence bitmap of the last k
+ *    (n / 8 bytes) is kept with the index for the next call with the same k, and released with the per-rank counts
+ *    when a call with another k comes.  SUFR_B200_ERR_ARGUMENT, before any
+ *    device work: NULL required pointers, k == 0, k above the build's max_query_len, num_bins out of range,
+ *    min_count > max_count, first_rank > s, a position window beyond n.  SUFR_B200_ERR_UNSUPPORTED: an index built
+ *    with a seed mask. */
+int sufr_b200_index_kmer_spectrum(SufrB200Index* index, uint64_t k, uint64_t num_bins, uint64_t* histogram,
+                                  uint64_t* distinct, uint64_t* occurrences, uint64_t* max_count);
+int sufr_b200_index_kmers(SufrB200Index* index, uint64_t k, uint64_t min_count, uint64_t max_count,
+                          uint64_t first_rank, uint64_t max_kmers, uint64_t* num_kmers, uint64_t* next_rank,
+                          uint64_t* rank_begin, uint64_t* rank_end, uint64_t* count, uint8_t* bytes);
+int sufr_b200_index_kmer_multiplicity(SufrB200Index* index, uint64_t k, uint64_t first_pos, uint64_t num_positions,
+                                      uint32_t* out);
+
 /* -- write: replaces SufrBuilder::write (sufr_builder.rs:817-918), version-6 `.sufr` layout.
  *    Single shard: writes the whole file.  Sharded: every rank calls it with the same path; rank 0
  *    writes header, text and the names tail, every rank pwrites its SA / LCP slice at its offset.

@@ -16,7 +16,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass, field
-from typing import List, Optional, Sequence, Tuple
+from typing import List, NamedTuple, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -374,6 +374,15 @@ class ExtractResult:
     sequences: List[ExtractSequence]
 
 
+class KmerSpectrum(NamedTuple):
+    """:meth:`SufrIndex.kmer_spectrum`: histogram[i] = distinct k-mers with count i + 1 (the last bin: count >= its
+    length)."""
+    histogram: np.ndarray
+    distinct: int
+    occurrences: int
+    max_count: int
+
+
 class SufrIndex:
     """Device-resident index: the read side that consumes the LCP array (``SufrFile::subsample_suffix_array``
     sufr_file.rs:429-456, ``suffix_search`` :777-836, ``locate`` :1132-1169, ``SufrSearch`` sufr_search.rs:104-350).
@@ -574,6 +583,62 @@ class SufrIndex:
             out[qi].append((qp, ml, [(suf[h], None if seq[h] == none else names[seq[h]], pos[h]) for h in range(lo, hi)]))
         return out
 
+    def kmer_spectrum(self, k: int, num_bins: int = 10000) -> "KmerSpectrum":
+        """sufr_b200_index_kmer_spectrum: histogram[i] = distinct k-mers occurring i + 1 times (the last bin: at least
+        num_bins times), with the number of distinct k-mers, of occurrences and the largest count.  A k-mer lies inside
+        one record and never includes its last byte; in a DNA index it is made of ACGT only (include/sufr_b200.h)."""
+        _positive_k(k)
+        _non_negative(num_bins=num_bins)
+        hist = np.zeros(max(1, num_bins), dtype=np.uint64)
+        d, o, m = C.c_uint64(), C.c_uint64(), C.c_uint64()
+        _check(_lib.lib().sufr_b200_index_kmer_spectrum(self._h, k, num_bins, hist.ctypes.data, C.byref(d), C.byref(o),
+                                                        C.byref(m)))
+        return KmerSpectrum(hist[:num_bins], int(d.value), int(o.value), int(m.value))
+
+    def kmers(self, k: int, min_count: int = 1, max_count: Optional[int] = None, window: int = 1 << 24):
+        """sufr_b200_index_kmers over the whole index: the distinct k-mers whose count lies in [min_count, max_count]
+        in byte order, as (rank_begin, rank_end, count, kmers) with kmers a (m, k) uint8 array; [rank_begin,
+        rank_end) is the k-mer's rank range, as :meth:`search` gives it.  Fetched ``window`` k-mers at a time (fewer
+        when their bytes would pass EXTRACT_BYTES)."""
+        _positive_k(k)
+        _non_negative(min_count=min_count, max_count=max_count, window=window)
+        if window < 1:
+            raise SufrError(_lib.ERR_ARGUMENT, f"window must be at least 1 (got {window})")
+        per = max(1, min(window, self.EXTRACT_BYTES // k))
+        hi = _U64_MAX if max_count is None else max_count
+        cols = [np.zeros(per, dtype=np.uint64) for _ in range(3)]
+        buf = np.zeros(per * k, dtype=np.uint8)
+        parts, first = [], 0
+        num, nxt = C.c_uint64(), C.c_uint64()
+        while True:
+            _check(_lib.lib().sufr_b200_index_kmers(self._h, k, min_count, hi, first, per, C.byref(num), C.byref(nxt),
+                                                    *[c.ctypes.data for c in cols], buf.ctypes.data))
+            m = int(num.value)
+            parts.append([c[:m].copy() for c in cols] + [buf[:m * k].reshape(m, k).copy()])
+            first = int(nxt.value)
+            if first >= self._s:
+                break
+        return tuple(np.concatenate([p[j] for p in parts]) for j in range(3)) + (
+            np.concatenate([p[3] for p in parts]).reshape(-1, k),)
+
+    def kmer_multiplicity(self, k: int, start: int = 0, length: Optional[int] = None, window: int = 1 << 28):
+        """sufr_b200_index_kmer_multiplicity: out[i] = the count of the k-mer at text position start + i, 0 where no
+        k-mer starts (saturated at 2**32 - 1), as a numpy uint32 array; ``length`` defaults to the end of the text.
+        Each window of ``window`` positions is one pass over the ranks."""
+        _positive_k(k)
+        _non_negative(start=start, length=length, window=window)
+        if window < 1:
+            raise SufrError(_lib.ERR_ARGUMENT, f"window must be at least 1 (got {window})")
+        if length is None:
+            length = max(0, self._n - start)
+        out = np.zeros(max(1, length), dtype=np.uint32)
+        if length == 0:
+            _check(_lib.lib().sufr_b200_index_kmer_multiplicity(self._h, k, start, 0, out.ctypes.data))
+        for f in range(0, length, window):
+            m = min(window, length - f)
+            _check(_lib.lib().sufr_b200_index_kmer_multiplicity(self._h, k, start + f, m, out[f:].ctypes.data))
+        return out[:length]
+
     def extract_window(self, first: int, max_hits: int, prefix_len: Optional[int] = None,
                        suffix_len: Optional[int] = None, max_bytes: Optional[int] = None):
         """sufr_b200_index_extract: the regions of the longest leading run of hits [first, first + max_hits) of the
@@ -673,6 +738,11 @@ class SufrIndex:
 
 
 _U64_MAX = 0xFFFFFFFFFFFFFFFF
+
+
+def _positive_k(k):
+    if k < 1:
+        raise SufrError(_lib.ERR_ARGUMENT, f"k must be at least 1 (got {k})")
 
 
 def _non_negative(**values):

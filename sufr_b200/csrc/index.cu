@@ -14,12 +14,24 @@
 #include "../../include/sufr_b200.h"
 #include "context.hpp"
 #include "host_io.hpp"
+#include "kmers.cuh"
 #include "pool.hpp"
 #include "scan.cuh"
 #include "search.cuh"
 #include "stream_io.hpp"
 
 using namespace sufr;
+
+// With the context's lock held: the total of one reduce of `in` over n >= 1 elements.
+template <typename Op, typename In>
+static unsigned long long kmer_reduce(Ctx& ctx, uint64_t n, In in, Op op) {
+    DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(n));
+    scan::scan_reduce(n, in, op, partials.get(), ctx.stream);
+    unsigned long long total = 0;
+    SUFR_CUDA_CHECK(cudaMemcpyAsync(&total, partials.get() + div_up(n, scan::CHUNK), 8, cudaMemcpyDeviceToHost, ctx.stream));
+    SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+    return total;
+}
 
 extern "C" {
 
@@ -51,6 +63,15 @@ struct SufrB200Index {
     DevBuf<unsigned long long> loc_begin, loc_end, loc_offsets;
     uint64_t loc_queries = 0, loc_hits = 0;
     bool has_loc = false;
+    // DNA index: k-mers are made of ACGT only
+    bool is_dna = false;
+    // the k-mer occurrence bitmap of the last k-mer call (kmer_occ_k == 0: none), so that the windows of one
+    // enumeration or multiplicity track do not each pass over the text again
+    DevBuf<uint32_t> kmer_occ;
+    uint64_t kmer_occ_k = 0;
+    // each group's count at its last rank (u32 per rank) for kmer_occ_k, made by the first multiplicity window and kept
+    // for the next ones; released with the bitmap when another k comes
+    DevBuf<uint32_t> kmer_tail;
     // max_query_len the index was built with, as sufr_file.rs:521-528 defines it: the mask weight, else the build's
     // max_query_len, else the text length
     uint64_t built_mql() const { return is_mask ? weight : (build_mql ? build_mql : n); }
@@ -95,6 +116,7 @@ int sufr_b200_index_create(SufrB200Ctx* c, const SufrB200Args* args, const SufrB
         idx->text_readable = r->text_len;
         idx->s = r->num_suffixes;
         idx->wide = r->index_bits == 64;
+        idx->is_dna = args->is_dna;
         if (args->num_sequences && !args->sequence_starts) throw Error(SUFR_B200_ERR_ARGUMENT, "sequence_starts is NULL");
         CtxLock lock(*ctx);
         index_set_mask(*idx, *ctx, args->seed_mask, args->has_max_query_len, args->max_query_len);
@@ -294,6 +316,7 @@ int sufr_b200_index_open(SufrB200Ctx* c, const char* path, SufrB200Index** out) 
         idx->n = fi.text_len;
         idx->s = fi.num_suffixes;
         idx->wide = fi.index_bits == 64;
+        idx->is_dna = fi.is_dna;
         const size_t w = fi.index_bits / 8;
         idx->own_text = DevBuf<unsigned char>(ctx->pool, fi.text_len + 16);
         idx->text_readable = fi.text_len + 16;
@@ -621,6 +644,221 @@ int sufr_b200_index_string_at(SufrB200Index* idx, uint64_t pos, uint64_t len, ui
             SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
         }
         *out_len = k;
+    });
+}
+
+// ---- k-mers (kmers.cuh)
+
+// Checks shared by the three k-mer calls, before any device work.
+static void check_kmer_args(const SufrB200Index* idx, uint64_t k) {
+    if (idx->is_mask)
+        throw Error(SUFR_B200_ERR_UNSUPPORTED, "k-mers need an index without a seed mask: a seed-mask order does not "
+                                               "sort contiguous bytes, so equal k-mers are not adjacent in it");
+    if (k == 0) throw Error(SUFR_B200_ERR_ARGUMENT, "k must be at least 1");
+    if (idx->build_mql && k > idx->build_mql)
+        throw Error(SUFR_B200_ERR_ARGUMENT, "k = " + std::to_string(k) + " is above the max_query_len " +
+                                                std::to_string(idx->build_mql) +
+                                                " the index was built with: LCP values above it are not exact");
+}
+
+// With the context's lock held: the occurrence bitmap of k (bit p of word p / 32: position p is a k-mer occurrence),
+// made by a pass over the text unless the last k-mer call left it for the same k.
+static const uint32_t* kmer_occurrences(SufrB200Index* idx, uint64_t k) {
+    if (idx->kmer_occ_k == k) return idx->kmer_occ.get();
+    Ctx& ctx = *idx->ctx;
+    idx->kmer_occ.reset();
+    idx->kmer_tail.reset();
+    idx->kmer_occ_k = 0;
+    const uint64_t P = div_up(idx->n, 32) * 32;
+    DevBuf<uint32_t> excl(ctx.pool, P / 32 + 1), occ(ctx.pool, P / 32 + 1);
+    if (P) {
+        kmers::excluded_kernel<<<(unsigned)div_up(P, 256), 256, 0, ctx.stream>>>(idx->text, idx->n, P, idx->is_dna,
+                                                                                  excl.get());
+        SUFR_KERNEL_CHECK();
+        if (idx->num_starts) {
+            kmers::record_ends_kernel<<<(unsigned)div_up(idx->num_starts, 256), 256, 0, ctx.stream>>>(
+                idx->starts.get(), idx->num_starts, excl.get());
+            SUFR_KERNEL_CHECK();
+        }
+        DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(P));
+        scan::inclusive_scan(P, kmers::NextExcludedIn{excl.get(), P}, kmers::MinU64{},
+                             kmers::OccurrenceOut{occ.get(), P, k}, partials.get(), ctx.stream);
+    }
+    idx->kmer_occ = std::move(occ);
+    idx->kmer_occ_k = k;
+    return idx->kmer_occ.get();
+}
+
+static kmers::Ranks kmer_ranks(SufrB200Index* idx, uint64_t k) {
+    return kmers::Ranks{idx->sa, idx->lcp, idx->wide, kmer_occurrences(idx, k), idx->s, k};
+}
+
+int sufr_b200_index_kmer_spectrum(SufrB200Index* idx, uint64_t k, uint64_t num_bins, uint64_t* histogram,
+                                  uint64_t* distinct, uint64_t* occurrences, uint64_t* max_count) {
+    return guarded([&] {
+        if (!idx || !histogram) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        check_kmer_args(idx, k);
+        if (num_bins < 1 || num_bins > 65536)
+            throw Error(SUFR_B200_ERR_ARGUMENT, "num_bins = " + std::to_string(num_bins) + " is not in [1, 65536]");
+        Ctx& ctx = *idx->ctx;
+        CtxLock lock(ctx);
+        DevBuf<unsigned long long> d_out(ctx.pool, num_bins + 2);  // histogram, then occurrences and the maximum
+        unsigned long long* d = d_out.get();
+        SUFR_CUDA_CHECK(cudaMemsetAsync(d, 0, (num_bins + 2) * 8, ctx.stream));
+        if (idx->s) {
+            const kmers::Ranks R = kmer_ranks(idx, k);
+            const uint64_t rows = div_up(idx->s, 32) * 32;  // (whole rows: SpectrumOut votes per row)
+            DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(rows));
+            scan::inclusive_scan(rows, kmers::GroupIn<62>{R, 0}, kmers::SpanOp{},
+                                 kmers::SpectrumOut{num_bins, d, d + num_bins}, partials.get(), ctx.stream);
+        }
+        std::vector<uint64_t> totals(2);
+        SUFR_CUDA_CHECK(cudaMemcpyAsync(histogram, d, num_bins * 8, cudaMemcpyDeviceToHost, ctx.stream));
+        SUFR_CUDA_CHECK(cudaMemcpyAsync(totals.data(), d + num_bins, 16, cudaMemcpyDeviceToHost, ctx.stream));
+        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+        uint64_t sum = 0;
+        for (uint64_t i = 0; i < num_bins; i++) sum += histogram[i];
+        if (distinct) *distinct = sum;
+        if (occurrences) *occurrences = totals[0];
+        if (max_count) *max_count = totals[1];
+    });
+}
+
+// With the context's lock held: the group that starts at rank lo and runs at least to rank a - 1 (longer than an
+// enumeration chunk).  Its end is the first rank at or after a that starts a group, or s, found in windows that double
+// from a - lo ranks, so the search costs time in proportion to the group; its count is one sum over its ranks.
+static void kmer_long_group(SufrB200Index* idx, const kmers::Ranks& R, uint64_t lo, uint64_t a, uint64_t& end,
+                            uint64_t& count) {
+    Ctx& ctx = *idx->ctx;
+    end = idx->s;
+    for (uint64_t w = a - lo; a < idx->s; a += w, w *= 2) {
+        w = std::min(w, idx->s - a);
+        const unsigned long long e = kmer_reduce(ctx, w, kmers::BoundaryIn{R, a}, kmers::MinU64{});
+        if (e != kmers::NONE) {
+            end = e;
+            break;
+        }
+    }
+    count = kmer_reduce(ctx, end - lo, kmers::OccIn{R, lo}, scan::SumU64{});
+}
+
+int sufr_b200_index_kmers(SufrB200Index* idx, uint64_t k, uint64_t min_count, uint64_t max_count, uint64_t first_rank,
+                          uint64_t max_kmers, uint64_t* num_kmers, uint64_t* next_rank, uint64_t* rank_begin,
+                          uint64_t* rank_end, uint64_t* count, uint8_t* bytes) {
+    return guarded([&] {
+        if (!idx || !num_kmers || !next_rank || (max_kmers && (!rank_begin || !rank_end || !count)))
+            throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        check_kmer_args(idx, k);
+        if (min_count > max_count)
+            throw Error(SUFR_B200_ERR_ARGUMENT, "min_count " + std::to_string(min_count) + " is above max_count " +
+                                                    std::to_string(max_count));
+        const uint64_t s = idx->s;
+        if (first_rank > s)
+            throw Error(SUFR_B200_ERR_ARGUMENT, "first_rank " + std::to_string(first_rank) + " is beyond the " +
+                                                    std::to_string(s) + " suffixes");
+        *num_kmers = 0;
+        *next_rank = first_rank;
+        if (first_rank == s || max_kmers == 0) return;
+        Ctx& ctx = *idx->ctx;
+        CtxLock lock(ctx);
+        const kmers::Ranks R = kmer_ranks(idx, k);
+        const uint64_t lo = first_rank, lo_count = min_count ? min_count : 1;  // (a group without occurrences is no k-mer)
+        // a chunk of ranks from lo, cut after its last complete group: twice max_kmers ranks hold max_kmers groups or
+        // cover twice the ranks the window lists, so a window costs time in proportion to the ranks it covers
+        const uint64_t L = std::min({s - lo, std::max<uint64_t>(max_kmers < s ? 2 * max_kmers : s, 1u << 16),
+                                     kmers::CHUNK_MAX});
+        DevBuf<unsigned long long> d_listed(ctx.pool, L), partials(ctx.pool, scan::partials_count(L));
+        DevBuf<uint32_t> listed_partials(ctx.pool, scan::partials_count(L));
+        scan::inclusive_scan(L, kmers::GroupIn<31>{R, lo}, kmers::ChunkOp{},
+                             kmers::KmerChunkOut{d_listed.get()},
+                             partials.get(), ctx.stream);
+        const kmers::ListedIn listed_in{d_listed.get(), lo_count, max_count};
+        scan::scan_reduce(L, listed_in, scan::SumU32{}, listed_partials.get(), ctx.stream);
+        uint32_t listed = 0;
+        uint64_t tail_next = 0;
+        SUFR_CUDA_CHECK(cudaMemcpyAsync(&listed, listed_partials.get() + div_up(L, scan::CHUNK), 4, cudaMemcpyDeviceToHost,
+                                        ctx.stream));
+        unsigned long long last = 0;
+        SUFR_CUDA_CHECK(cudaMemcpyAsync(&last, d_listed.get() + L - 1, 8, cudaMemcpyDeviceToHost, ctx.stream));
+        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+        // where the next window starts if every group of the chunk is listed: lo + L when the chunk ends at a group
+        // boundary or holds no group start, else the start of the group it cuts
+        tail_next = ((last & kmers::TAIL) || !(last & kmers::HEAD)) ? lo + L : lo + ((last >> 31) & kmers::ChunkOp::COUNT);
+        uint64_t m = 0, next = tail_next;
+        DevBuf<unsigned long long> d_out;
+        if (tail_next == lo) {  // the group that starts at lo runs past the chunk (lo + L < s: rank s - 1 ends a group)
+            uint64_t e, c;
+            kmer_long_group(idx, R, lo, lo + L, e, c);
+            next = e;
+            if (c >= lo_count && c <= max_count) {
+                m = 1;
+                rank_begin[0] = lo;
+                rank_end[0] = e;
+                count[0] = c;
+                d_out = DevBuf<unsigned long long>(ctx.pool, 1);
+                SUFR_CUDA_CHECK(cudaMemcpyAsync(d_out.get(), rank_begin, 8, cudaMemcpyHostToDevice, ctx.stream));
+            }
+        } else if (listed) {
+            m = std::min<uint64_t>(listed, max_kmers);
+            d_out = DevBuf<unsigned long long>(ctx.pool, 3 * m);
+            unsigned long long* o = d_out.get();
+            scan::scan_apply(L, listed_in, scan::SumU32{}, kmers::ListedOut{d_listed.get(), lo, m, o, o + m, o + 2 * m},
+                             listed_partials.get(), ctx.stream);
+            uint64_t* outs[3] = {rank_begin, rank_end, count};
+            for (int j = 0; j < 3; j++)
+                SUFR_CUDA_CHECK(cudaMemcpyAsync(outs[j], o + j * m, m * 8, cudaMemcpyDeviceToHost, ctx.stream));
+        }
+        DevBuf<unsigned long long> d_pos;
+        DevBuf<uint8_t> d_bytes;
+        if (m && bytes) {  // d_out starts with the groups' first ranks
+            d_pos = DevBuf<unsigned long long>(ctx.pool, m);
+            kmers::kmer_positions_kernel<<<(unsigned)div_up(m, 256), 256, 0, ctx.stream>>>(R, d_out.get(), m, d_pos.get());
+            SUFR_KERNEL_CHECK();
+            const uint64_t total = m * k;
+            d_bytes = DevBuf<uint8_t>(ctx.pool, total);
+            kmers::kmer_bytes_kernel<<<(unsigned)div_up(total, 256), 256, 0, ctx.stream>>>(idx->text, d_pos.get(), k,
+                                                                                            total, d_bytes.get());
+            SUFR_KERNEL_CHECK();
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(bytes, d_bytes.get(), total, cudaMemcpyDeviceToHost, ctx.stream));
+        }
+        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+        if (listed > max_kmers && tail_next != lo) next = rank_end[m - 1];
+        *num_kmers = m;
+        *next_rank = next;
+    });
+}
+
+int sufr_b200_index_kmer_multiplicity(SufrB200Index* idx, uint64_t k, uint64_t first_pos, uint64_t num_positions,
+                                      uint32_t* out) {
+    return guarded([&] {
+        if (!idx || (num_positions && !out)) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        check_kmer_args(idx, k);
+        if (first_pos > idx->n || num_positions > idx->n - first_pos)
+            throw Error(SUFR_B200_ERR_ARGUMENT, "position window [" + std::to_string(first_pos) + ", +" +
+                                                    std::to_string(num_positions) + ") is beyond the text length " +
+                                                    std::to_string(idx->n));
+        if (num_positions == 0) return;
+        Ctx& ctx = *idx->ctx;
+        CtxLock lock(ctx);
+        DevBuf<uint32_t> d_out(ctx.pool, num_positions);
+        SUFR_CUDA_CHECK(cudaMemsetAsync(d_out.get(), 0, num_positions * 4, ctx.stream));
+        if (idx->s) {
+            const kmers::Ranks R = kmer_ranks(idx, k);
+            DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(idx->s));
+            // each group's count at its last rank, once per k (the windows of a track share it) ...
+            if (!idx->kmer_tail.get()) {
+                DevBuf<uint32_t> at_tail(ctx.pool, idx->s);
+                scan::inclusive_scan(idx->s, kmers::GroupIn<62>{R, 0}, kmers::SpanOp{}, kmers::GroupCountOut{at_tail.get()},
+                                     partials.get(), ctx.stream);
+                idx->kmer_tail = std::move(at_tail);
+            }
+            // ... then back over the group and out to the text positions in the window
+            scan::inclusive_scan(idx->s, kmers::GroupCountIn{R, idx->kmer_tail.get()}, kmers::SpanOp{},
+                                 kmers::MultiplicityOut{R, first_pos, num_positions, d_out.get()}, partials.get(),
+                                 ctx.stream);
+        }
+        SUFR_CUDA_CHECK(cudaMemcpyAsync(out, d_out.get(), num_positions * 4, cudaMemcpyDeviceToHost, ctx.stream));
+        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
     });
 }
 

@@ -176,6 +176,14 @@ template <typename Out, typename T>
 struct has_staged_load<Out, T, std::void_t<decltype(std::declval<const Out&>().load(uint64_t(0), std::declval<T>(), std::declval<T>()))>>
     : std::true_type {};
 
+// An output functor that keeps per-block state (a shared-memory histogram, say) declares
+// `static constexpr bool kBlockHooks = true` and gets `begin()` before the block's first load and `finish()` after its
+// last store; both are called by every thread of the block, and finish() may synchronise the block.
+template <typename Out, typename = void>
+struct has_block_hooks : std::false_type {};
+template <typename Out>
+struct has_block_hooks<Out, std::enable_if_t<Out::kBlockHooks>> : std::true_type {};
+
 // the last phase of apply_kernel: row k of the warp, value v, inclusive scan value incl
 template <typename Out, typename T, typename Rows>
 __device__ __forceinline__ void emit_rows(const Out& out, uint64_t n, uint64_t w0, const Rows& rows) {
@@ -207,6 +215,7 @@ __global__ void __launch_bounds__(BLOCK) apply_kernel(uint64_t n, In in, Op op, 
     __shared__ T smem[BLOCK / 32];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint64_t w0 = (uint64_t)blockIdx.x * CHUNK + (uint64_t)warp * (32 * ITEMS) + lane;
+    if constexpr (has_block_hooks<Out>::value) out.begin();
     if constexpr (is_flags<In>::value) {
         // ---- flags: votes.  b0 / b1 = the row's ballots of bit 0 / bit 32; counts before a row are warp-uniform.
         constexpr bool kPair = sizeof(T) == 8;
@@ -313,6 +322,7 @@ __global__ void __launch_bounds__(BLOCK) apply_kernel(uint64_t n, In in, Op op, 
         for (int k = 0; k < ITEMS; k++) rows.s[k] = op(prefix, rows.s[k]);
         emit_rows<Out, T>(out, n, w0, rows);
     }
+    if constexpr (has_block_hooks<Out>::value) out.finish();
 }
 
 inline size_t partials_count(uint64_t n) { return (size_t)div_up(n, CHUNK) + 1; }
