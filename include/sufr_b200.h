@@ -296,6 +296,44 @@ int sufr_b200_index_mems(SufrB200Index* index, const uint8_t* queries, const uin
                          uint64_t* mem_len, uint64_t* rank_begin, uint64_t* rank_end,
                          uint64_t* hit_offsets /* offsets[num_queries] + 1 */);
 
+/* -- search with mismatches, on the device, on an index from index_open or index_create without a seed mask.  t = the
+ *    text, n its length, SA the full suffix array (the LCP array and its subsample play no part).
+ *      separators  Z = the byte t[n - 1] and the byte t[c_i - 1] of every sequence start c_i > 0 ('$' and '%' with the
+ *               default delimiter), as byte values.  Computed once per index and kept with it.
+ *      match    of a query q of length m with budget k (max_mismatches): let m' = min(m, cap), cap = the build's
+ *               max_query_len, or m without one (index_locate compares the same first cap bytes).  A match is a string
+ *               w of m' bytes such that (a) w = t[p, p + m') for an indexed position p (an entry of SA) with
+ *               p + m' <= n; (b) w differs from q[0, m') in at most k positions, bytes compared as they are (as
+ *               index_search compares them); (c) no position where they differ holds a byte of Z in w: a substitution
+ *               never puts a record separator into a match, while an equal separator byte still matches.  So k = 0
+ *               gives the range index_locate gives (full array, no run-time cap) for every non-empty query.  An empty
+ *               query, or one with m' > n, has no match.
+ *    index_approx  the matches of every query, one per distinct w: [rank_begin, rank_end) = the half-open rank range of
+ *               the suffixes that start with w (contiguous in SA; for a cap index the order is exact on the first cap
+ *               bytes, DESIGN.md §3 item 4), and mismatches = the Hamming distance of w to q[0, m').  In query order,
+ *               then rank order (the byte order of the w).  match_offsets[q] .. match_offsets[q + 1] are the matches
+ *               of query q (num_queries + 1 entries); *num_hits = their occurrences in all.  The matches take the
+ *               place of locate's queries: index_hits and index_extract return their occurrences, windowed and
+ *               byte-budgeted, until the next index_locate, index_mems or index_approx (the k-mer calls leave them).
+ *               Device memory is bounded whatever the batch: a level of the search with more nodes than fit is
+ *               expanded in slices (DESIGN.md §7b).
+ *    index_approx_matches  matches [first, first + count) of the last index_approx: mismatches, rank_begin, rank_end
+ *               (count entries each) and hit_offsets (count + 1 entries, global indices into the hits).  Any output
+ *               may be NULL.
+ *    index_approx_levels  the profile of the last index_approx: nodes[d] / steps[d] = the search nodes at depth d and
+ *               the binary-search steps that counted their children (the expansion repeats them), for
+ *               d < min(max_levels, *num_levels); *num_levels = the longest m' of the batch.  nodes / steps may be NULL.
+ *    SUFR_B200_ERR_ARGUMENT, before any device work: NULL required pointers, offsets not ascending,
+ *    max_mismatches > 16; for index_approx_matches, a window beyond the matches, or a locate state that the last
+ *    index_locate / index_mems set.  SUFR_B200_ERR_UNSUPPORTED: an index built with a seed mask (its order is not
+ *    over contiguous bytes), with the locate state left as it was. */
+int sufr_b200_index_approx(SufrB200Index* index, const uint8_t* queries, const uint64_t* offsets, uint64_t num_queries,
+                           uint64_t max_mismatches, uint64_t* match_offsets /* num_queries + 1 */, uint64_t* num_hits);
+int sufr_b200_index_approx_matches(SufrB200Index* index, uint64_t first, uint64_t count, uint64_t* mismatches,
+                                   uint64_t* rank_begin, uint64_t* rank_end, uint64_t* hit_offsets /* count + 1 */);
+int sufr_b200_index_approx_levels(SufrB200Index* index, uint64_t max_levels, uint64_t* num_levels, uint64_t* nodes,
+                                  uint64_t* steps);
+
 /* -- k-mer counting on the device, on an index from index_open or index_create without a seed mask.  t = the text,
  *    n its length, SA / LCP the full arrays (s entries), sequence starts c_0 < ... < c_{R-1}.  Records follow
  *    index_extract: record i owns [c_i, c_{i+1}), the last one [c_{R-1}, n), positions before c_0 belong to [0, c_0);

@@ -144,6 +144,7 @@ ABI_SYMBOLS = [
     "sufr_b200_index_locate", "sufr_b200_index_hits", "sufr_b200_index_extract", "sufr_b200_index_list",
     "sufr_b200_index_string_at", "sufr_b200_index_matching_stats", "sufr_b200_index_mems",
     "sufr_b200_index_kmer_spectrum", "sufr_b200_index_kmers", "sufr_b200_index_kmer_multiplicity",
+    "sufr_b200_index_approx", "sufr_b200_index_approx_matches", "sufr_b200_index_approx_levels",
     "sufr_b200_seed_mask", "sufr_b200_find_lcp_full_offset", "sufr_b200_read_sequence_file",
     "sufr_b200_sequences_free", "sufr_b200_synth_dna", "sufr_b200_last_error", "sufr_b200_abi_version",
     "sufr_b200_device_count",
@@ -238,6 +239,14 @@ def lib():
                                         C.c_void_p, C.c_void_p]
     L.sufr_b200_index_kmer_multiplicity.restype = C.c_int
     L.sufr_b200_index_kmer_multiplicity.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p]
+    L.sufr_b200_index_approx.restype = C.c_int
+    L.sufr_b200_index_approx.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p,
+                                         C.POINTER(C.c_uint64)]
+    L.sufr_b200_index_approx_matches.restype = C.c_int
+    L.sufr_b200_index_approx_matches.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                 C.c_void_p]
+    L.sufr_b200_index_approx_levels.restype = C.c_int
+    L.sufr_b200_index_approx_levels.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64), C.c_void_p, C.c_void_p]
     L.sufr_b200_seed_mask.restype = C.c_int64
     L.sufr_b200_seed_mask.argtypes = [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.sufr_b200_find_lcp_full_offset.restype = C.c_uint64

@@ -507,8 +507,8 @@ class SufrIndex:
         return b[:nq], e[:nq], ho
 
     def hits(self, first: int, count: int):
-        """sufr_b200_index_hits: (suffix, sequence, sequence_pos) of hits [first, first + count) of the last locate or
-        :meth:`mems`."""
+        """sufr_b200_index_hits: (suffix, sequence, sequence_pos) of hits [first, first + count) of the last locate,
+        :meth:`mems` or :meth:`approx_matches`."""
         suf = np.zeros(max(1, count), dtype=np.uint64)
         seq = np.zeros(max(1, count), dtype=np.uint64)
         pos = np.zeros(max(1, count), dtype=np.uint64)
@@ -582,6 +582,62 @@ class SufrIndex:
             lo, hi = int(ho[k]), int(ho[k + 1])
             out[qi].append((qp, ml, [(suf[h], None if seq[h] == none else names[seq[h]], pos[h]) for h in range(lo, hi)]))
         return out
+
+    APPROX_WINDOW = 1 << 24  # matches fetched per sufr_b200_index_approx_matches call
+
+    def _approx(self, queries, max_mismatches):
+        """sufr_b200_index_approx, then every match in windows: (mismatches, rank_begin, rank_end, hit_offsets,
+        match_offsets) as numpy arrays (hit_offsets one longer than the matches, match_offsets one longer than the
+        queries).  The matches become the hits of :meth:`hits` / :meth:`extract_window`."""
+        _non_negative(max_mismatches=max_mismatches)
+        blob, offs = self._pack_queries(queries)
+        nq = len(offs) - 1
+        mo = np.zeros(nq + 1, dtype=np.uint64)
+        hits = C.c_uint64()
+        L = _lib.lib()
+        _check(L.sufr_b200_index_approx(self._h, blob.ctypes.data, offs.ctypes.data, nq, max_mismatches, mo.ctypes.data,
+                                        C.byref(hits)))
+        total = int(mo[-1])
+        cols = [np.zeros(max(1, total), dtype=np.uint64) for _ in range(3)]
+        ho = np.zeros(total + 1, dtype=np.uint64)
+        for f in range(0, total, self.APPROX_WINDOW):
+            c = min(self.APPROX_WINDOW, total - f)
+            _check(L.sufr_b200_index_approx_matches(self._h, f, c, *[x[f:].ctypes.data for x in cols],
+                                                    ho[f:].ctypes.data))
+        return tuple(x[:total] for x in cols) + (ho, mo)
+
+    def approx_matches(self, queries, max_mismatches: int):
+        """Search with mismatches (include/sufr_b200.h): per query a list of (mismatches, rank_begin, rank_end) in
+        rank order, one per distinct string w of the query's length (capped at the build's max_query_len) that occurs
+        in the text within ``max_mismatches`` substitutions of the query, no substitution onto a record separator.
+        An index with a seed mask is refused (ERR_UNSUPPORTED)."""
+        mis, b, e, _, mo = self._approx(queries, max_mismatches)
+        rows = list(zip(mis.tolist(), b.tolist(), e.tolist()))
+        cuts = mo.astype(np.int64).tolist()
+        return [rows[lo:hi] for lo, hi in zip(cuts[:-1], cuts[1:])]
+
+    def locate_approx(self, queries, max_mismatches: int):
+        """:meth:`approx_matches` with every occurrence: per query a list of (mismatches, hits) with hits a list of
+        (suffix, sequence_name, sequence_position) in rank order, as :meth:`locate_mems` gives them."""
+        mis, _, _, ho, mo = self._approx(queries, max_mismatches)
+        suf, seq, pos = self._all_hits(int(ho[-1]))
+        names, none = self._names, 0xFFFFFFFFFFFFFFFF
+        rows = []
+        for k, e in enumerate(mis.tolist()):
+            lo, hi = int(ho[k]), int(ho[k + 1])
+            rows.append((e, [(suf[h], None if seq[h] == none else names[seq[h]], pos[h]) for h in range(lo, hi)]))
+        cuts = mo.astype(np.int64).tolist()
+        return [rows[lo:hi] for lo, hi in zip(cuts[:-1], cuts[1:])]
+
+    def approx_levels(self):
+        """The profile of the last search with mismatches: (nodes, steps), numpy arrays indexed by depth."""
+        num = C.c_uint64()
+        L = _lib.lib()
+        _check(L.sufr_b200_index_approx_levels(self._h, 0, C.byref(num), None, None))
+        nodes = np.zeros(max(1, num.value), dtype=np.uint64)
+        steps = np.zeros(max(1, num.value), dtype=np.uint64)
+        _check(L.sufr_b200_index_approx_levels(self._h, num.value, C.byref(num), nodes.ctypes.data, steps.ctypes.data))
+        return nodes[:num.value], steps[:num.value]
 
     def kmer_spectrum(self, k: int, num_bins: int = 10000) -> "KmerSpectrum":
         """sufr_b200_index_kmer_spectrum: histogram[i] = distinct k-mers occurring i + 1 times (the last bin: at least

@@ -140,6 +140,13 @@ using pos_t = uint64_t;
 #include "build_impl.inl"
 }  // namespace p64
 
+// the radix sort for the read side (approx.cuh): the instance the 32-bit build already uses, so no new kernel
+bool sort_u64_u32_pairs(uint64_t* keys_a, uint64_t* keys_b, uint32_t* vals_a, uint32_t* vals_b, uint64_t n, int end_bit,
+                        uint32_t* counts, cudaStream_t stream) {
+    return rsort::sort_pairs<uint64_t, uint32_t>(keys_a, keys_b, vals_a, vals_b, n, 0, end_bit, counts, stream);
+}
+size_t sort_counts_words() { return rsort::counts_words(); }
+
 // texts of u32::MAX bytes and more need 64-bit positions; SUFR_B200_DEBUG_POS64 forces them (tests)
 static void run_build(Ctx& ctx, const SufrB200Args& args, uint32_t index_bits, int text_memory, int result_memory,
                       SufrB200Result* out) {

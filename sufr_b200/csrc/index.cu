@@ -12,6 +12,7 @@
 #include <vector>
 
 #include "../../include/sufr_b200.h"
+#include "approx.cuh"
 #include "context.hpp"
 #include "host_io.hpp"
 #include "kmers.cuh"
@@ -58,11 +59,18 @@ struct SufrB200Index {
     // sequence starts (u64) for locate; num_starts == 0: none
     DevBuf<unsigned long long> starts;
     uint64_t num_starts = 0;
-    // the last sufr_b200_index_locate or _mems: rank ranges and hit offsets of its queries (or MEMs), for
-    // sufr_b200_index_hits and sufr_b200_index_extract
+    // the last sufr_b200_index_locate, _mems or _approx: rank ranges and hit offsets of its queries (or MEMs, or
+    // matches), for sufr_b200_index_hits and sufr_b200_index_extract
     DevBuf<unsigned long long> loc_begin, loc_end, loc_offsets;
     uint64_t loc_queries = 0, loc_hits = 0;
     bool has_loc = false;
+    // set when that call was _approx: the mismatches of its matches, for sufr_b200_index_approx_matches
+    DevBuf<unsigned long long> loc_mismatches;
+    bool loc_approx = false;
+    // the separator bytes of index_approx (a 256-bit mask, made by its first call), and the nodes and binary-search
+    // steps per depth of its last call
+    DevBuf<uint32_t> sep;
+    std::vector<unsigned long long> approx_levels;
     // DNA index: k-mers are made of ACGT only
     bool is_dna = false;
     // the k-mer occurrence bitmap of the last k-mer call (kmer_occ_k == 0: none), so that the windows of one
@@ -351,6 +359,16 @@ int sufr_b200_index_open(SufrB200Ctx* c, const char* path, SufrB200Index** out) 
     });
 }
 
+// With the context's lock held: drops the locate state before a call that replaces it.
+static void reset_loc(SufrB200Index* idx) {
+    idx->has_loc = false;
+    idx->loc_approx = false;
+    idx->loc_begin.reset();
+    idx->loc_end.reset();
+    idx->loc_offsets.reset();
+    idx->loc_mismatches.reset();
+}
+
 int sufr_b200_index_locate(SufrB200Index* idx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq, int has_mql,
                            uint64_t mql, int low_memory, uint64_t* rank_begin, uint64_t* rank_end, uint64_t* hit_offsets) {
     return guarded([&] {
@@ -360,10 +378,7 @@ int sufr_b200_index_locate(SufrB200Index* idx, const uint8_t* queries, const uin
             if (offsets[i + 1] < offsets[i]) throw Error(SUFR_B200_ERR_ARGUMENT, "query offsets are not ascending");
         Ctx& ctx = *idx->ctx;
         CtxLock lock(ctx);
-        idx->has_loc = false;
-        idx->loc_begin.reset();
-        idx->loc_end.reset();
-        idx->loc_offsets.reset();
+        reset_loc(idx);
         // sufr_file.rs:514-560: the in-memory mode searches the LCP-subsampled array when the effective max_query_len
         // is shorter than the build's
         int use_sub = 0;
@@ -455,10 +470,7 @@ int sufr_b200_index_mems(SufrB200Index* idx, const uint8_t* queries, const uint6
         const uint64_t total = offsets[nq];
         Ctx& ctx = *idx->ctx;
         CtxLock lock(ctx);
-        idx->has_loc = false;
-        idx->loc_begin.reset();
-        idx->loc_end.reset();
-        idx->loc_offsets.reset();
+        reset_loc(idx);
         // matching statistics of every byte, then the MEMs compacted by one scan of their flags
         uint64_t mems = 0;
         DevBuf<unsigned long long> d_ms, d_mem;
@@ -514,14 +526,15 @@ int sufr_b200_index_mems(SufrB200Index* idx, const uint8_t* queries, const uint6
     });
 }
 
-// With the context's lock held, under which the last locate or mems wrote the state read here: refuses a window of hits
+// With the context's lock held, under which the last locate, mems or approx wrote the state read here: refuses a window of hits
 // that is not inside that call's.
 static void check_hit_window(const SufrB200Index* idx, uint64_t first, uint64_t count) {
     if (!idx->has_loc)
-        throw Error(SUFR_B200_ERR_ARGUMENT, "neither sufr_b200_index_locate nor sufr_b200_index_mems has been called");
+        throw Error(SUFR_B200_ERR_ARGUMENT, "none of sufr_b200_index_locate, _mems and _approx has been called");
     if (first > idx->loc_hits || count > idx->loc_hits - first)
         throw Error(SUFR_B200_ERR_ARGUMENT, "hit window [" + std::to_string(first) + ", +" + std::to_string(count) +
-                                                ") is beyond the " + std::to_string(idx->loc_hits) + " hits of the last locate or mems");
+                                                ") is beyond the " + std::to_string(idx->loc_hits) +
+                                                " hits of the last locate, mems or approx");
 }
 
 int sufr_b200_index_hits(SufrB200Index* idx, uint64_t first, uint64_t count, uint64_t* suffix, uint64_t* sequence,
@@ -644,6 +657,260 @@ int sufr_b200_index_string_at(SufrB200Index* idx, uint64_t pos, uint64_t len, ui
             SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
         }
         *out_len = k;
+    });
+}
+
+// ---- search with mismatches (approx.cuh)
+
+// bits that hold v (at least 1)
+static int bits_for(uint64_t v) {
+    int b = 1;
+    while (b < 64 && (v >> b)) b++;
+    return b;
+}
+
+// Children one slice of a level may hold.  A level that has more is expanded in slices, each taken to completion
+// before the next, so the search keeps at most one sliced level per depth: the budget is set so that max_depth + 2
+// levels (nodes, 32 bytes, and their packed offsets, 8 bytes, each) fit in half the memory the pool and the device
+// have free.  Below 2^24 (the packed counts of a level stay under 2^32).  SUFR_B200_DEBUG_APPROX_NODES=<n> sets it,
+// so that tests reach the sliced path on small inputs.
+static uint64_t approx_node_budget(Ctx& ctx, uint64_t max_depth) {
+    if (const char* dbg = getenv("SUFR_B200_DEBUG_APPROX_NODES"))
+        return std::min<uint64_t>(1ull << 22, std::max<uint64_t>(1, strtoull(dbg, nullptr, 10)));
+    size_t free_b = 0, total_b = 0;
+    SUFR_CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
+    const uint64_t avail = free_b + (ctx.pool.capacity() - ctx.pool.in_use());
+    const uint64_t per = (sizeof(approx::Node) + 8) * (max_depth + 2);
+    return std::max<uint64_t>(1024, std::min<uint64_t>(1ull << 22, avail / 2 / per));
+}
+
+// One level of the search: its nodes (all at one depth), the exclusive scan of their packed counts, and the slices
+// [cuts[j], cuts[j + 1]) it is expanded in, with the scan's value at each cut.
+struct ApproxLevel {
+    DevBuf<approx::Node> nodes;
+    uint64_t count = 0;
+    uint32_t depth = 0;
+    DevBuf<unsigned long long> excl;
+    std::vector<uint64_t> cuts;
+    std::vector<unsigned long long> at;
+    size_t next = 0;
+};
+
+// With the context's lock held: every match of the queries whose offsets are d_off, unsorted, into `finals` (grown as
+// needed); returns their number.  d_stats[2 d], [2 d + 1] += the nodes and search steps at depth d.
+static uint64_t approx_search(SufrB200Index* idx, const approx::Params& P, const unsigned long long* d_off, uint64_t nq,
+                              uint64_t max_depth, DevBuf<approx::Final>& finals, unsigned long long* d_stats) {
+    Ctx& ctx = *idx->ctx;
+    const uint64_t budget = approx_node_budget(ctx, max_depth);
+    const uint64_t cap = idx->build_mql;
+    uint64_t num_finals = 0;
+    std::vector<ApproxLevel> stack;
+    for (uint64_t q0 = 0; q0 < nq; q0 += budget) {  // roots: the queries, `budget` at a time
+        ApproxLevel root;
+        root.count = std::min(budget, nq - q0);
+        root.nodes = DevBuf<approx::Node>(ctx.pool, root.count);
+        approx::root_kernel<<<(unsigned)div_up(root.count, 256), 256, 0, ctx.stream>>>(d_off, q0, root.count, cap, idx->n,
+                                                                                      idx->s, root.nodes.get());
+        SUFR_KERNEL_CHECK();
+        stack.push_back(std::move(root));
+        while (!stack.empty()) {
+            ApproxLevel& L = stack.back();
+            if (L.cuts.empty()) {  // count the level's children, and cut it into slices of at most `budget` of them
+                DevBuf<unsigned long long> counts(ctx.pool, L.count), partials(ctx.pool, scan::partials_count(L.count));
+                approx::count_kernel<<<(unsigned)div_up(L.count, approx::BLOCK), approx::BLOCK, 0, ctx.stream>>>(
+                    P, L.nodes.get(), L.count, counts.get(), d_stats + 2 * L.depth);
+                SUFR_KERNEL_CHECK();
+                L.excl = DevBuf<unsigned long long>(ctx.pool, L.count);
+                scan::inclusive_scan(L.count, search::ArrayIn{counts.get()}, scan::SumU64{}, approx::ExclOut{L.excl.get()},
+                                     partials.get(), ctx.stream);
+                unsigned long long total = 0;
+                SUFR_CUDA_CHECK(cudaMemcpyAsync(&total, partials.get() + div_up(L.count, scan::CHUNK), 8,
+                                                cudaMemcpyDeviceToHost, ctx.stream));
+                SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+                L.cuts = {0};
+                L.at = {0};
+                if ((uint32_t)total > budget) {
+                    std::vector<unsigned long long> h(L.count + 1);
+                    SUFR_CUDA_CHECK(cudaMemcpyAsync(h.data(), L.excl.get(), L.count * 8, cudaMemcpyDeviceToHost, ctx.stream));
+                    SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+                    h[L.count] = total;
+                    for (uint64_t i = 1; i < L.count; i++)  // (a slice holds one node at least)
+                        if ((uint32_t)h[i + 1] - (uint32_t)L.at.back() > budget) {
+                            L.cuts.push_back(i);
+                            L.at.push_back(h[i]);
+                        }
+                }
+                L.cuts.push_back(L.count);
+                L.at.push_back(total);
+            }
+            const uint64_t a = L.cuts[L.next], b = L.cuts[L.next + 1];
+            const unsigned long long span = L.at[L.next + 1] - L.at[L.next];
+            const uint64_t children = (uint32_t)span, matches = span >> 32;
+            L.next++;
+            ApproxLevel child;
+            child.count = children;
+            child.depth = L.depth + 1;
+            if (children) child.nodes = DevBuf<approx::Node>(ctx.pool, children);
+            if (num_finals + matches > finals.size()) {
+                DevBuf<approx::Final> bigger(ctx.pool, std::max<uint64_t>(num_finals + matches, 2 * finals.size()));
+                if (num_finals)
+                    SUFR_CUDA_CHECK(cudaMemcpyAsync(bigger.get(), finals.get(), num_finals * sizeof(approx::Final),
+                                                    cudaMemcpyDeviceToDevice, ctx.stream));
+                finals = std::move(bigger);
+            }
+            if (span) {
+                approx::expand_kernel<<<(unsigned)div_up(b - a, approx::BLOCK), approx::BLOCK, 0, ctx.stream>>>(
+                    P, L.nodes.get(), L.excl.get(), a, b, child.nodes.get(), finals.get(), num_finals);
+                SUFR_KERNEL_CHECK();
+            }
+            num_finals += matches;
+            if (L.next + 1 == L.cuts.size()) stack.pop_back();  // (its buffers go back to the pool in stream order)
+            if (children) stack.push_back(std::move(child));
+        }
+    }
+    return num_finals;
+}
+
+int sufr_b200_index_approx(SufrB200Index* idx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq,
+                           uint64_t max_mismatches, uint64_t* match_offsets, uint64_t* num_hits) {
+    return guarded([&] {
+        if (!idx || !offsets || !match_offsets || !num_hits || (nq && !queries && offsets[nq]))
+            throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        for (uint64_t i = 0; i < nq; i++)
+            if (offsets[i + 1] < offsets[i]) throw Error(SUFR_B200_ERR_ARGUMENT, "query offsets are not ascending");
+        if (max_mismatches > 16)
+            throw Error(SUFR_B200_ERR_ARGUMENT, "max_mismatches = " + std::to_string(max_mismatches) + " is above 16");
+        if (idx->is_mask)
+            throw Error(SUFR_B200_ERR_UNSUPPORTED, "search with mismatches needs an index without a seed mask: a seed-mask "
+                                                   "order does not sort contiguous bytes");
+        const int rank_bits = bits_for(idx->s ? idx->s - 1 : 0), query_bits = bits_for(nq ? nq - 1 : 0);
+        if (rank_bits + query_bits > 64)
+            throw Error(SUFR_B200_ERR_ARGUMENT, std::to_string(nq) + " queries are too many for one call on " +
+                                                    std::to_string(idx->s) + " suffixes: split the batch");
+        uint64_t max_depth = 0;  // the longest m' that can match
+        for (uint64_t i = 0; i < nq; i++) {
+            uint64_t m = offsets[i + 1] - offsets[i];
+            if (idx->build_mql && m > idx->build_mql) m = idx->build_mql;
+            if (m <= idx->n && m > max_depth) max_depth = m;
+        }
+        if (max_depth > 0xFFFFFFFFull) throw Error(SUFR_B200_ERR_ARGUMENT, "a query is longer than 2^32 - 1 bytes");
+        Ctx& ctx = *idx->ctx;
+        CtxLock lock(ctx);
+        reset_loc(idx);
+        idx->approx_levels.assign(2 * max_depth, 0);
+        approx::Params P{};
+        P.text = idx->text;
+        P.n = idx->n;
+        P.sa = idx->sa;
+        P.wide = idx->wide;
+        P.k = (uint32_t)max_mismatches;
+        if (!idx->sep) {
+            idx->sep = DevBuf<uint32_t>(ctx.pool, 8);
+            SUFR_CUDA_CHECK(cudaMemsetAsync(idx->sep.get(), 0, 32, ctx.stream));
+            approx::separators_kernel<<<(unsigned)div_up(idx->num_starts + 1, 256), 256, 0, ctx.stream>>>(
+                idx->text, idx->n, idx->starts.get(), idx->num_starts, idx->sep.get());
+            SUFR_KERNEL_CHECK();
+        }
+        P.sep = idx->sep.get();
+        uint64_t matches = 0;
+        DevBuf<uint64_t> keys_a, keys_b;
+        DevBuf<uint32_t> vals_a, vals_b;
+        bool sorted_in_b = false;
+        idx->loc_begin = DevBuf<unsigned long long>(ctx.pool, 1);  // (replaced below when there are matches)
+        idx->loc_end = DevBuf<unsigned long long>(ctx.pool, 1);
+        idx->loc_mismatches = DevBuf<unsigned long long>(ctx.pool, 1);
+        if (max_depth && idx->s) {
+            DeviceQueries dq(ctx, queries, offsets, nq);
+            const auto* d_off = reinterpret_cast<const unsigned long long*>(dq.off.get());
+            P.queries = dq.q.get();
+            P.offsets = d_off;
+            DevBuf<unsigned long long> d_stats(ctx.pool, 2 * max_depth);
+            SUFR_CUDA_CHECK(cudaMemsetAsync(d_stats.get(), 0, 2 * max_depth * 8, ctx.stream));
+            DevBuf<approx::Final> finals;
+            matches = approx_search(idx, P, d_off, nq, max_depth, finals, d_stats.get());
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(idx->approx_levels.data(), d_stats.get(), 2 * max_depth * 8,
+                                            cudaMemcpyDeviceToHost, ctx.stream));
+            if (matches > 0xFFFFFFFFull)
+                throw Error(SUFR_B200_ERR_UNSUPPORTED, std::to_string(matches) + " matches: more than 2^32 - 1 in one "
+                                                                                 "call, split the batch");
+            if (matches) {  // (query, rank_begin) order: one radix sort of the packed pair
+                keys_a = DevBuf<uint64_t>(ctx.pool, matches);
+                keys_b = DevBuf<uint64_t>(ctx.pool, matches);
+                vals_a = DevBuf<uint32_t>(ctx.pool, matches);
+                vals_b = DevBuf<uint32_t>(ctx.pool, matches);
+                DevBuf<uint32_t> counts(ctx.pool, sort_counts_words());
+                approx::final_keys_kernel<<<(unsigned)div_up(matches, 256), 256, 0, ctx.stream>>>(
+                    finals.get(), matches, rank_bits, keys_a.get(), vals_a.get());
+                SUFR_KERNEL_CHECK();
+                sorted_in_b = sort_u64_u32_pairs(keys_a.get(), keys_b.get(), vals_a.get(), vals_b.get(), matches,
+                                                 rank_bits + query_bits, counts.get(), ctx.stream);
+                idx->loc_begin = DevBuf<unsigned long long>(ctx.pool, matches);
+                idx->loc_end = DevBuf<unsigned long long>(ctx.pool, matches);
+                idx->loc_mismatches = DevBuf<unsigned long long>(ctx.pool, matches);
+                approx::final_gather_kernel<<<(unsigned)div_up(matches, 256), 256, 0, ctx.stream>>>(
+                    finals.get(), (sorted_in_b ? vals_b : vals_a).get(), matches, idx->loc_begin.get(),
+                    idx->loc_end.get(), idx->loc_mismatches.get());
+                SUFR_KERNEL_CHECK();
+            }
+        }
+        DevBuf<unsigned long long> d_mo(ctx.pool, nq + 1);
+        approx::match_offsets_kernel<<<(unsigned)div_up(nq + 1, 256), 256, 0, ctx.stream>>>(
+            (sorted_in_b ? keys_b : keys_a).get(), matches, rank_bits, nq, d_mo.get());
+        SUFR_KERNEL_CHECK();
+        SUFR_CUDA_CHECK(cudaMemcpyAsync(match_offsets, d_mo.get(), (nq + 1) * 8, cudaMemcpyDeviceToHost, ctx.stream));
+        // the matches take the place of locate's queries: hit offsets = exclusive scan of their occurrence counts
+        idx->loc_offsets = DevBuf<unsigned long long>(ctx.pool, matches + 1);
+        SUFR_CUDA_CHECK(cudaMemsetAsync(idx->loc_offsets.get(), 0, 8, ctx.stream));
+        if (matches) {
+            DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(matches));
+            scan::inclusive_scan(matches, search::HitCountIn{idx->loc_begin.get(), idx->loc_end.get()}, scan::SumU64{},
+                                 search::HitOffsetOut{idx->loc_offsets.get()}, partials.get(), ctx.stream);
+        }
+        uint64_t hits = 0;
+        SUFR_CUDA_CHECK(cudaMemcpyAsync(&hits, idx->loc_offsets.get() + matches, 8, cudaMemcpyDeviceToHost, ctx.stream));
+        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+        *num_hits = hits;
+        idx->loc_queries = matches;
+        idx->loc_hits = hits;
+        idx->has_loc = true;
+        idx->loc_approx = true;
+    });
+}
+
+int sufr_b200_index_approx_matches(SufrB200Index* idx, uint64_t first, uint64_t count, uint64_t* mismatches,
+                                   uint64_t* rank_begin, uint64_t* rank_end, uint64_t* hit_offsets) {
+    return guarded([&] {
+        if (!idx) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        Ctx& ctx = *idx->ctx;
+        CtxLock lock(ctx);
+        if (!idx->has_loc || !idx->loc_approx)
+            throw Error(SUFR_B200_ERR_ARGUMENT, "the last call that set the locate state was not sufr_b200_index_approx");
+        if (first > idx->loc_queries || count > idx->loc_queries - first)
+            throw Error(SUFR_B200_ERR_ARGUMENT, "match window [" + std::to_string(first) + ", +" + std::to_string(count) +
+                                                    ") is beyond the " + std::to_string(idx->loc_queries) + " matches");
+        const std::pair<uint64_t*, const unsigned long long*> outs[3] = {
+            {mismatches, idx->loc_mismatches.get()}, {rank_begin, idx->loc_begin.get()}, {rank_end, idx->loc_end.get()}};
+        for (const auto& o : outs)
+            if (o.first && count)
+                SUFR_CUDA_CHECK(cudaMemcpyAsync(o.first, o.second + first, count * 8, cudaMemcpyDeviceToHost, ctx.stream));
+        if (hit_offsets)
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(hit_offsets, idx->loc_offsets.get() + first, (count + 1) * 8,
+                                            cudaMemcpyDeviceToHost, ctx.stream));
+        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+    });
+}
+
+int sufr_b200_index_approx_levels(SufrB200Index* idx, uint64_t max_levels, uint64_t* num_levels, uint64_t* nodes,
+                                  uint64_t* steps) {
+    return guarded([&] {
+        if (!idx || !num_levels) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        CtxLock lock(*idx->ctx);
+        const uint64_t levels = idx->approx_levels.size() / 2;
+        for (uint64_t d = 0; d < std::min(levels, max_levels); d++) {
+            if (nodes) nodes[d] = idx->approx_levels[2 * d];
+            if (steps) steps[d] = idx->approx_levels[2 * d + 1];
+        }
+        *num_levels = levels;
     });
 }
 
