@@ -167,8 +167,10 @@ int sufr_b200_verify(SufrB200Ctx* ctx, const SufrB200Args* args, const SufrB200R
  *      subsample  SufrFile::subsample_suffix_array (sufr_file.rs:429-456): the entries with lcp < max_query_len and
  *                 their ranks ("compressed" in-memory suffix array)
  *      search     SufrSearch::search (sufr_search.rs:104-350) for a batch of queries, one GPU thread per query:
- *                 queries = concatenated bytes, offsets[num_queries + 1]; has/max_query_len = the run-time `-m`
- *                 (a max_query_len of 0 is no run-time cap, also on an index built with one);
+ *                 queries = concatenated bytes, offsets[num_queries + 1], ascending (SUFR_B200_ERR_ARGUMENT "query
+ *                 offsets are not ascending" otherwise, as in every call that takes a batch);
+ *                 has/max_query_len = the run-time `-m` (a max_query_len of 0 is no run-time cap, also on an index
+ *                 built with one);
  *                 use_subsample != 0 searches the subsampled array and maps the hits back through the ranks.
  *                 rank_begin / rank_end (host, num_queries each) = half-open rank range in the full suffix array
  *                 (SearchResultLocations::ranks), both UINT64_MAX when the query does not occur; count = end - begin.

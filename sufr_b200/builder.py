@@ -520,18 +520,24 @@ class SufrIndex:
         """SufrFile::locate: per query a list of (rank, suffix, sequence_name, sequence_position) in rank order
         (name None and position = suffix for an index without sequence starts)."""
         b, _, ho = self.locate_ranges(queries, max_query_len, low_memory)
-        suf, seq, pos = self._all_hits(int(ho[-1]))
-        names, none = self._names, 0xFFFFFFFFFFFFFFFF
-        out = []
-        for i in range(len(b)):
-            lo, hi, r0 = int(ho[i]), int(ho[i + 1]), int(b[i])
-            out.append([(r0 + k - lo, suf[k], None if seq[k] == none else names[seq[k]], pos[k]) for k in range(lo, hi)])
-        return out
+        hits = self._split(self._all_hits(int(ho[-1])), ho)
+        return [[(r0 + k,) + h for k, h in enumerate(hs)] for r0, hs in zip(b.tolist(), hits)]
 
     def _all_hits(self, total: int):
-        """(suffix, sequence, sequence_pos) lists of all ``total`` hits of the last locate / mems, in windows."""
+        """The rows (suffix, sequence name or None, sequence position) of all ``total`` hits of the last locate, mems
+        or approx, fetched in windows."""
         parts = [self.hits(f, min(self.HITS_WINDOW, total - f)) for f in range(0, total, self.HITS_WINDOW)]
-        return tuple(np.concatenate([p[k] for p in parts]).tolist() if parts else [] for k in range(3))
+        if not parts:
+            return []
+        suf, seq, pos = (np.concatenate([p[k] for p in parts]).tolist() for k in range(3))
+        names, none = self._names, 0xFFFFFFFFFFFFFFFF
+        return [(s, None if q == none else names[q], p) for s, q, p in zip(suf, seq, pos)]
+
+    @staticmethod
+    def _split(rows, offsets):
+        """``rows`` cut into one list per entry of an offsets array: entry i gets rows[offsets[i]:offsets[i + 1]]."""
+        cuts = np.asarray(offsets).astype(np.int64).tolist()
+        return [rows[lo:hi] for lo, hi in zip(cuts[:-1], cuts[1:])]
 
     def matching_statistics(self, queries):
         """sufr_b200_index_matching_stats: per query (lengths, rank_begin, rank_end), numpy uint64 arrays of the
@@ -543,8 +549,7 @@ class SufrIndex:
         ms, b, e = (np.zeros(max(1, total), dtype=np.uint64) for _ in range(3))
         _check(_lib.lib().sufr_b200_index_matching_stats(self._h, blob.ctypes.data, offs.ctypes.data, nq, ms.ctypes.data,
                                                          b.ctypes.data, e.ctypes.data))
-        cuts = offs.astype(np.int64).tolist()
-        return [(ms[lo:hi], b[lo:hi], e[lo:hi]) for lo, hi in zip(cuts[:-1], cuts[1:])]
+        return list(zip(*(self._split(x, offs) for x in (ms, b, e))))
 
     def _mems(self, queries, min_len):
         """sufr_b200_index_mems: (query, position, length, rank_begin, rank_end, hit_offsets) as numpy arrays, one entry
@@ -575,12 +580,10 @@ class SufrIndex:
         """:meth:`mems` with every occurrence: per query a list of (query_pos, length, hits) with hits a list of
         (suffix, sequence_name, sequence_position) in rank order, as :meth:`locate` gives them."""
         q, p, ln, _, _, ho = self._mems(queries, min_len)
-        suf, seq, pos = self._all_hits(int(ho[-1]))
-        names, none = self._names, 0xFFFFFFFFFFFFFFFF
+        hits = self._split(self._all_hits(int(ho[-1])), ho)
         out = [[] for _ in range(len(queries))]
-        for k, (qi, qp, ml) in enumerate(zip(q.tolist(), p.tolist(), ln.tolist())):
-            lo, hi = int(ho[k]), int(ho[k + 1])
-            out[qi].append((qp, ml, [(suf[h], None if seq[h] == none else names[seq[h]], pos[h]) for h in range(lo, hi)]))
+        for qi, qp, ml, hs in zip(q.tolist(), p.tolist(), ln.tolist(), hits):
+            out[qi].append((qp, ml, hs))
         return out
 
     APPROX_WINDOW = 1 << 24  # matches fetched per sufr_b200_index_approx_matches call
@@ -612,22 +615,14 @@ class SufrIndex:
         in the text within ``max_mismatches`` substitutions of the query, no substitution onto a record separator.
         An index with a seed mask is refused (ERR_UNSUPPORTED)."""
         mis, b, e, _, mo = self._approx(queries, max_mismatches)
-        rows = list(zip(mis.tolist(), b.tolist(), e.tolist()))
-        cuts = mo.astype(np.int64).tolist()
-        return [rows[lo:hi] for lo, hi in zip(cuts[:-1], cuts[1:])]
+        return self._split(list(zip(mis.tolist(), b.tolist(), e.tolist())), mo)
 
     def locate_approx(self, queries, max_mismatches: int):
         """:meth:`approx_matches` with every occurrence: per query a list of (mismatches, hits) with hits a list of
         (suffix, sequence_name, sequence_position) in rank order, as :meth:`locate_mems` gives them."""
         mis, _, _, ho, mo = self._approx(queries, max_mismatches)
-        suf, seq, pos = self._all_hits(int(ho[-1]))
-        names, none = self._names, 0xFFFFFFFFFFFFFFFF
-        rows = []
-        for k, e in enumerate(mis.tolist()):
-            lo, hi = int(ho[k]), int(ho[k + 1])
-            rows.append((e, [(suf[h], None if seq[h] == none else names[seq[h]], pos[h]) for h in range(lo, hi)]))
-        cuts = mo.astype(np.int64).tolist()
-        return [rows[lo:hi] for lo, hi in zip(cuts[:-1], cuts[1:])]
+        hits = self._split(self._all_hits(int(ho[-1])), ho)
+        return self._split(list(zip(mis.tolist(), hits)), mo)
 
     def approx_levels(self):
         """The profile of the last search with mismatches: (nodes, steps), numpy arrays indexed by depth."""

@@ -23,16 +23,60 @@
 
 using namespace sufr;
 
-// With the context's lock held: the total of one reduce of `in` over n >= 1 elements.
-template <typename Op, typename In>
-static unsigned long long kmer_reduce(Ctx& ctx, uint64_t n, In in, Op op) {
-    DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(n));
-    scan::scan_reduce(n, in, op, partials.get(), ctx.stream);
-    unsigned long long total = 0;
-    SUFR_CUDA_CHECK(cudaMemcpyAsync(&total, partials.get() + div_up(n, scan::CHUNK), 8, cudaMemcpyDeviceToHost, ctx.stream));
+// Refuses a batch of nq queries (blob + offsets[0..nq]) before any lock is taken or state is dropped.
+static void check_queries(const uint8_t* queries, const uint64_t* offsets, uint64_t nq) {
+    if (!offsets || (!queries && offsets[nq])) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+    for (uint64_t i = 0; i < nq; i++)
+        if (offsets[i + 1] < offsets[i]) throw Error(SUFR_B200_ERR_ARGUMENT, "query offsets are not ascending");
+}
+
+// With the context's lock held: the grand total a scan over n elements left in `partials`, once the stream is done.
+template <typename T>
+static T read_total(Ctx& ctx, T* partials, uint64_t n) {
+    T total = 0;
+    SUFR_CUDA_CHECK(cudaMemcpyAsync(&total, scan::total_ptr(partials, n), sizeof(T), cudaMemcpyDeviceToHost, ctx.stream));
     SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
     return total;
 }
+
+// With the context's lock held: d_off[0] = 0 and d_off[1..m] = the inclusive sums of `in` over m entries, queued.
+template <typename In>
+static void exclusive_offsets(Ctx& ctx, uint64_t m, In in, unsigned long long* d_off) {
+    SUFR_CUDA_CHECK(cudaMemsetAsync(d_off, 0, 8, ctx.stream));
+    if (!m) return;
+    DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(m));
+    scan::inclusive_scan(m, in, scan::SumU64{}, search::HitOffsetOut{d_off}, partials.get(), ctx.stream);
+}
+
+// With the context's lock held: the total of one reduce of `in` over n >= 1 elements.
+template <typename Op, typename In>
+static typename Op::T kmer_reduce(Ctx& ctx, uint64_t n, In in, Op op) {
+    DevBuf<typename Op::T> partials(ctx.pool, scan::partials_count(n));
+    scan::scan_reduce(n, in, op, partials.get(), ctx.stream);
+    return read_total(ctx, partials.get(), n);
+}
+
+// The last sufr_b200_index_locate, _mems or _approx (`source`): rank ranges and hit offsets of its `entries` queries
+// (or MEMs, or matches), for sufr_b200_index_hits and _extract, and after _approx the mismatches of its matches, for
+// sufr_b200_index_approx_matches.
+struct LocateState {
+    DevBuf<unsigned long long> begin, end, offsets, mismatches;
+    uint64_t entries = 0, hits = 0;
+    enum Source { NONE, LOCATE, MEMS, APPROX } source = NONE;
+
+    // With the context's lock held, once the call that replaces the state has queued the rank ranges of its m entries
+    // into begin / end: queues their hit offsets (the exclusive scan of their occurrence counts) and passes them, on the
+    // device, to copy_out, which queues the call's copies, synchronises and returns the total of the hits.  Only then
+    // is the state recorded as `from`'s.
+    template <typename CopyOut>
+    void set(Ctx& ctx, uint64_t m, Source from, CopyOut copy_out) {
+        offsets = DevBuf<unsigned long long>(ctx.pool, m + 1);
+        exclusive_offsets(ctx, m, search::HitCountIn{begin.get(), end.get()}, offsets.get());
+        hits = copy_out(offsets.get());
+        entries = m;
+        source = from;
+    }
+};
 
 extern "C" {
 
@@ -59,14 +103,7 @@ struct SufrB200Index {
     // sequence starts (u64) for locate; num_starts == 0: none
     DevBuf<unsigned long long> starts;
     uint64_t num_starts = 0;
-    // the last sufr_b200_index_locate, _mems or _approx: rank ranges and hit offsets of its queries (or MEMs, or
-    // matches), for sufr_b200_index_hits and sufr_b200_index_extract
-    DevBuf<unsigned long long> loc_begin, loc_end, loc_offsets;
-    uint64_t loc_queries = 0, loc_hits = 0;
-    bool has_loc = false;
-    // set when that call was _approx: the mismatches of its matches, for sufr_b200_index_approx_matches
-    DevBuf<unsigned long long> loc_mismatches;
-    bool loc_approx = false;
+    LocateState loc;
     // the separator bytes of index_approx (a 256-bit mask, made by its first call), and the nodes and binary-search
     // steps per depth of its last call
     DevBuf<uint32_t> sep;
@@ -157,8 +194,7 @@ static uint64_t index_subsample_locked(SufrB200Index* idx, uint64_t max_query_le
     uint32_t total = 0;
     if (idx->s) {
         scan::scan_reduce(idx->s, in, scan::SumU32{}, partials.get(), ctx.stream);
-        SUFR_CUDA_CHECK(cudaMemcpyAsync(&total, partials.get() + div_up(idx->s, scan::CHUNK), 4, cudaMemcpyDeviceToHost, ctx.stream));
-        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+        total = read_total(ctx, partials.get(), idx->s);
     }
     idx->sub_sa = DevBuf<unsigned char>(ctx.pool, (size_t)total * w + 8);
     idx->sub_rank = DevBuf<unsigned char>(ctx.pool, (size_t)total * w + 8);
@@ -193,27 +229,37 @@ struct DeviceQueries {
     }
 };
 
+// The search parameters that come from the index: its full suffix array, without a run-time cap.
+static search::Params search_params(const SufrB200Index* idx) {
+    search::Params P{};
+    P.text = idx->text;
+    P.n = idx->n;
+    P.sa = idx->sa;
+    P.len = idx->s;
+    P.num_suffixes = idx->s;
+    P.wide = idx->wide;
+    P.is_mask = idx->is_mask;
+    P.build_mql = idx->build_mql;
+    P.mask_pos = idx->maskpos.get();
+    P.weight = idx->weight;
+    P.mask_len = idx->mask_len;
+    return P;
+}
+
 // With the context's lock held: uploads nq >= 1 queries (blob + offsets) and queues their search, whose rank ranges go
 // to d_b / d_e.
 static void launch_search(SufrB200Index* idx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq, int has_mql,
                           uint64_t mql, int use_subsample, unsigned long long* d_b, unsigned long long* d_e) {
     Ctx& ctx = *idx->ctx;
     DeviceQueries dq(ctx, queries, offsets, nq);
-    search::Params P{};
-    P.text = idx->text;
-    P.n = idx->n;
-    P.sa = use_subsample ? (const void*)idx->sub_sa.get() : idx->sa;
-    P.rank = use_subsample ? (const void*)idx->sub_rank.get() : nullptr;
-    P.len = use_subsample ? idx->sub_len : idx->s;
-    P.num_suffixes = idx->s;
-    P.wide = idx->wide;
-    P.is_mask = idx->is_mask;
-    P.build_mql = idx->build_mql;
+    search::Params P = search_params(idx);
+    if (use_subsample) {
+        P.sa = idx->sub_sa.get();
+        P.rank = idx->sub_rank.get();
+        P.len = idx->sub_len;
+    }
     P.has_run_mql = has_mql && mql > 0;  // a run-time max_query_len of 0 is no cap, on a capped index too
     P.run_mql = mql;
-    P.mask_pos = idx->maskpos.get();
-    P.weight = idx->weight;
-    P.mask_len = idx->mask_len;
     search::search_kernel<<<(unsigned)div_up(nq, 128), 128, 0, ctx.stream>>>(P, dq.q.get(), dq.off.get(), nq, d_b, d_e);
     SUFR_KERNEL_CHECK();
 }
@@ -221,7 +267,8 @@ static void launch_search(SufrB200Index* idx, const uint8_t* queries, const uint
 int sufr_b200_index_search(SufrB200Index* idx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq, int has_mql,
                            uint64_t mql, int use_subsample, uint64_t* rank_begin, uint64_t* rank_end) {
     return guarded([&] {
-        if (!idx || !offsets || !rank_begin || !rank_end || (nq && !queries && offsets[nq])) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        if (!idx || !rank_begin || !rank_end) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        check_queries(queries, offsets, nq);
         if (use_subsample && !idx->has_sub) throw Error(SUFR_B200_ERR_ARGUMENT, "sufr_b200_index_subsample has not been called");
         if (nq == 0) return;
         Ctx& ctx = *idx->ctx;
@@ -359,26 +406,14 @@ int sufr_b200_index_open(SufrB200Ctx* c, const char* path, SufrB200Index** out) 
     });
 }
 
-// With the context's lock held: drops the locate state before a call that replaces it.
-static void reset_loc(SufrB200Index* idx) {
-    idx->has_loc = false;
-    idx->loc_approx = false;
-    idx->loc_begin.reset();
-    idx->loc_end.reset();
-    idx->loc_offsets.reset();
-    idx->loc_mismatches.reset();
-}
-
 int sufr_b200_index_locate(SufrB200Index* idx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq, int has_mql,
                            uint64_t mql, int low_memory, uint64_t* rank_begin, uint64_t* rank_end, uint64_t* hit_offsets) {
     return guarded([&] {
-        if (!idx || !offsets || (nq && (!rank_begin || !rank_end)) || !hit_offsets || (nq && !queries && offsets[nq]))
-            throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
-        for (uint64_t i = 0; i < nq; i++)
-            if (offsets[i + 1] < offsets[i]) throw Error(SUFR_B200_ERR_ARGUMENT, "query offsets are not ascending");
+        if (!idx || (nq && (!rank_begin || !rank_end)) || !hit_offsets) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        check_queries(queries, offsets, nq);
         Ctx& ctx = *idx->ctx;
         CtxLock lock(ctx);
-        reset_loc(idx);
+        idx->loc = LocateState{};
         // sufr_file.rs:514-560: the in-memory mode searches the LCP-subsampled array when the effective max_query_len
         // is shorter than the build's
         int use_sub = 0;
@@ -390,31 +425,24 @@ int sufr_b200_index_locate(SufrB200Index* idx, const uint8_t* queries, const uin
                 use_sub = 1;
             }
         }
-        idx->loc_begin = DevBuf<unsigned long long>(ctx.pool, nq + 1);
-        idx->loc_end = DevBuf<unsigned long long>(ctx.pool, nq + 1);
-        idx->loc_offsets = DevBuf<unsigned long long>(ctx.pool, nq + 1);
-        SUFR_CUDA_CHECK(cudaMemsetAsync(idx->loc_offsets.get(), 0, 8, ctx.stream));
-        if (nq) {
-            launch_search(idx, queries, offsets, nq, has_mql, mql, use_sub, idx->loc_begin.get(), idx->loc_end.get());
-            DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(nq));
-            scan::inclusive_scan(nq, search::HitCountIn{idx->loc_begin.get(), idx->loc_end.get()}, scan::SumU64{},
-                                 search::HitOffsetOut{idx->loc_offsets.get()}, partials.get(), ctx.stream);
-            SUFR_CUDA_CHECK(cudaMemcpyAsync(rank_begin, idx->loc_begin.get(), nq * 8, cudaMemcpyDeviceToHost, ctx.stream));
-            SUFR_CUDA_CHECK(cudaMemcpyAsync(rank_end, idx->loc_end.get(), nq * 8, cudaMemcpyDeviceToHost, ctx.stream));
-        }
-        SUFR_CUDA_CHECK(cudaMemcpyAsync(hit_offsets, idx->loc_offsets.get(), (nq + 1) * 8, cudaMemcpyDeviceToHost, ctx.stream));
-        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
-        idx->loc_queries = nq;
-        idx->loc_hits = hit_offsets[nq];
-        idx->has_loc = true;
+        LocateState& loc = idx->loc;
+        loc.begin = DevBuf<unsigned long long>(ctx.pool, nq + 1);
+        loc.end = DevBuf<unsigned long long>(ctx.pool, nq + 1);
+        if (nq) launch_search(idx, queries, offsets, nq, has_mql, mql, use_sub, loc.begin.get(), loc.end.get());
+        loc.set(ctx, nq, LocateState::LOCATE, [&](const unsigned long long* d_hit_offsets) {
+            if (nq) {
+                SUFR_CUDA_CHECK(cudaMemcpyAsync(rank_begin, loc.begin.get(), nq * 8, cudaMemcpyDeviceToHost, ctx.stream));
+                SUFR_CUDA_CHECK(cudaMemcpyAsync(rank_end, loc.end.get(), nq * 8, cudaMemcpyDeviceToHost, ctx.stream));
+            }
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(hit_offsets, d_hit_offsets, (nq + 1) * 8, cudaMemcpyDeviceToHost, ctx.stream));
+            SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+            return hit_offsets[nq];
+        });
     });
 }
 
-// Argument checks shared by index_matching_stats and index_mems, before any device work.
-static void check_matching_args(const SufrB200Index* idx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq) {
-    if (nq && !queries && offsets[nq]) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
-    for (uint64_t i = 0; i < nq; i++)
-        if (offsets[i + 1] < offsets[i]) throw Error(SUFR_B200_ERR_ARGUMENT, "query offsets are not ascending");
+// The refusal shared by index_matching_stats and index_mems, before any device work.
+static void check_matching_args(const SufrB200Index* idx) {
     if (idx->is_mask)
         throw Error(SUFR_B200_ERR_UNSUPPORTED, "matching statistics and MEMs need an index without a seed mask: a seed-mask "
                                                "order does not sort contiguous bytes, so it has no longest match");
@@ -424,25 +452,18 @@ static void check_matching_args(const SufrB200Index* idx, const uint8_t* queries
 static void launch_matching_stats(SufrB200Index* idx, const DeviceQueries& dq, uint64_t nq, uint64_t total,
                                   unsigned long long* d_ms, unsigned long long* d_b, unsigned long long* d_e) {
     Ctx& ctx = *idx->ctx;
-    search::Params P{};
-    P.text = idx->text;
-    P.n = idx->n;
-    P.sa = idx->sa;
-    P.len = idx->s;
-    P.num_suffixes = idx->s;
-    P.wide = idx->wide;
-    P.build_mql = idx->build_mql;
     search::matching_stats_kernel<<<(unsigned)div_up(total, 128), 128, 0, ctx.stream>>>(
-        P, dq.q.get(), reinterpret_cast<const unsigned long long*>(dq.off.get()), nq, total, d_ms, d_b, d_e);
+        search_params(idx), dq.q.get(), reinterpret_cast<const unsigned long long*>(dq.off.get()), nq, total, d_ms, d_b, d_e);
     SUFR_KERNEL_CHECK();
 }
 
 int sufr_b200_index_matching_stats(SufrB200Index* idx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq,
                                    uint64_t* match_len, uint64_t* rank_begin, uint64_t* rank_end) {
     return guarded([&] {
-        if (!idx || !offsets) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        if (!idx) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        check_queries(queries, offsets, nq);
         if (offsets[nq] && (!match_len || !rank_begin || !rank_end)) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
-        check_matching_args(idx, queries, offsets, nq);
+        check_matching_args(idx);
         const uint64_t total = offsets[nq];
         if (total == 0) return;
         Ctx& ctx = *idx->ctx;
@@ -462,15 +483,17 @@ int sufr_b200_index_mems(SufrB200Index* idx, const uint8_t* queries, const uint6
                          uint64_t min_len, uint64_t* num_mems, uint64_t* mem_query, uint64_t* mem_pos, uint64_t* mem_len,
                          uint64_t* rank_begin, uint64_t* rank_end, uint64_t* hit_offsets) {
     return guarded([&] {
-        if (!idx || !offsets || !num_mems || !hit_offsets) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        if (!idx || !num_mems || !hit_offsets) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        check_queries(queries, offsets, nq);
         if (offsets[nq] && (!mem_query || !mem_pos || !mem_len || !rank_begin || !rank_end))
             throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
         if (min_len == 0) throw Error(SUFR_B200_ERR_ARGUMENT, "min_len must be at least 1");
-        check_matching_args(idx, queries, offsets, nq);
+        check_matching_args(idx);
         const uint64_t total = offsets[nq];
         Ctx& ctx = *idx->ctx;
         CtxLock lock(ctx);
-        reset_loc(idx);
+        idx->loc = LocateState{};
+        LocateState& loc = idx->loc;
         // matching statistics of every byte, then the MEMs compacted by one scan of their flags
         uint64_t mems = 0;
         DevBuf<unsigned long long> d_ms, d_mem;
@@ -483,13 +506,9 @@ int sufr_b200_index_mems(SufrB200Index* idx, const uint8_t* queries, const uint6
             const search::MemFlagIn in{ms, d_off, nq, min_len};
             DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(total));
             scan::scan_reduce(total, in, scan::SumU64{}, partials.get(), ctx.stream);
-            unsigned long long count = 0;
-            SUFR_CUDA_CHECK(cudaMemcpyAsync(&count, partials.get() + div_up(total, scan::CHUNK), 8, cudaMemcpyDeviceToHost,
-                                            ctx.stream));
-            SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
-            mems = count;
-            idx->loc_begin = DevBuf<unsigned long long>(ctx.pool, mems + 1);
-            idx->loc_end = DevBuf<unsigned long long>(ctx.pool, mems + 1);
+            mems = read_total(ctx, partials.get(), total);
+            loc.begin = DevBuf<unsigned long long>(ctx.pool, mems + 1);
+            loc.end = DevBuf<unsigned long long>(ctx.pool, mems + 1);
             // (query, position, length) of every MEM, then the byte each one starts at
             d_mem = DevBuf<unsigned long long>(ctx.pool, 4 * mems + 1);
             unsigned long long* m = d_mem.get();
@@ -497,43 +516,38 @@ int sufr_b200_index_mems(SufrB200Index* idx, const uint8_t* queries, const uint6
             if (mems) {
                 search::mem_fill_kernel<<<(unsigned)div_up(mems, 256), 256, 0, ctx.stream>>>(
                     m + 3 * mems, mems, ms, ms + total, ms + 2 * total, d_off, nq, m, m + mems, m + 2 * mems,
-                    idx->loc_begin.get(), idx->loc_end.get());
+                    loc.begin.get(), loc.end.get());
                 SUFR_KERNEL_CHECK();
             }
         } else {
-            idx->loc_begin = DevBuf<unsigned long long>(ctx.pool, 1);
-            idx->loc_end = DevBuf<unsigned long long>(ctx.pool, 1);
+            loc.begin = DevBuf<unsigned long long>(ctx.pool, 1);
+            loc.end = DevBuf<unsigned long long>(ctx.pool, 1);
         }
-        // the MEMs take the place of locate's queries: hit offsets = exclusive scan of their occurrence counts
-        idx->loc_offsets = DevBuf<unsigned long long>(ctx.pool, mems + 1);
-        SUFR_CUDA_CHECK(cudaMemsetAsync(idx->loc_offsets.get(), 0, 8, ctx.stream));
-        if (mems) {
-            DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(mems));
-            scan::inclusive_scan(mems, search::HitCountIn{idx->loc_begin.get(), idx->loc_end.get()}, scan::SumU64{},
-                                 search::HitOffsetOut{idx->loc_offsets.get()}, partials.get(), ctx.stream);
-            uint64_t* outs[5] = {mem_query, mem_pos, mem_len, rank_begin, rank_end};
-            const unsigned long long* srcs[5] = {d_mem.get(), d_mem.get() + mems, d_mem.get() + 2 * mems,
-                                                 idx->loc_begin.get(), idx->loc_end.get()};
-            for (int k = 0; k < 5; k++)
-                SUFR_CUDA_CHECK(cudaMemcpyAsync(outs[k], srcs[k], mems * 8, cudaMemcpyDeviceToHost, ctx.stream));
-        }
-        SUFR_CUDA_CHECK(cudaMemcpyAsync(hit_offsets, idx->loc_offsets.get(), (mems + 1) * 8, cudaMemcpyDeviceToHost, ctx.stream));
-        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
-        *num_mems = mems;
-        idx->loc_queries = mems;
-        idx->loc_hits = hit_offsets[mems];
-        idx->has_loc = true;
+        // the MEMs take the place of locate's queries
+        loc.set(ctx, mems, LocateState::MEMS, [&](const unsigned long long* d_hit_offsets) {
+            if (mems) {
+                uint64_t* outs[5] = {mem_query, mem_pos, mem_len, rank_begin, rank_end};
+                const unsigned long long* srcs[5] = {d_mem.get(), d_mem.get() + mems, d_mem.get() + 2 * mems,
+                                                     loc.begin.get(), loc.end.get()};
+                for (int k = 0; k < 5; k++)
+                    SUFR_CUDA_CHECK(cudaMemcpyAsync(outs[k], srcs[k], mems * 8, cudaMemcpyDeviceToHost, ctx.stream));
+            }
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(hit_offsets, d_hit_offsets, (mems + 1) * 8, cudaMemcpyDeviceToHost, ctx.stream));
+            SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+            *num_mems = mems;
+            return hit_offsets[mems];
+        });
     });
 }
 
 // With the context's lock held, under which the last locate, mems or approx wrote the state read here: refuses a window of hits
 // that is not inside that call's.
 static void check_hit_window(const SufrB200Index* idx, uint64_t first, uint64_t count) {
-    if (!idx->has_loc)
+    if (idx->loc.source == LocateState::NONE)
         throw Error(SUFR_B200_ERR_ARGUMENT, "none of sufr_b200_index_locate, _mems and _approx has been called");
-    if (first > idx->loc_hits || count > idx->loc_hits - first)
+    if (first > idx->loc.hits || count > idx->loc.hits - first)
         throw Error(SUFR_B200_ERR_ARGUMENT, "hit window [" + std::to_string(first) + ", +" + std::to_string(count) +
-                                                ") is beyond the " + std::to_string(idx->loc_hits) +
+                                                ") is beyond the " + std::to_string(idx->loc.hits) +
                                                 " hits of the last locate, mems or approx");
 }
 
@@ -548,7 +562,7 @@ int sufr_b200_index_hits(SufrB200Index* idx, uint64_t first, uint64_t count, uin
         DevBuf<unsigned long long> d_out(ctx.pool, 3 * count);
         unsigned long long* d_suf = d_out.get();
         search::hits_kernel<<<(unsigned)div_up(count, 256), 256, 0, ctx.stream>>>(
-            idx->sa, idx->wide, idx->loc_begin.get(), idx->loc_offsets.get(), idx->loc_queries, idx->starts.get(),
+            idx->sa, idx->wide, idx->loc.begin.get(), idx->loc.offsets.get(), idx->loc.entries, idx->starts.get(),
             idx->num_starts, first, count, d_suf, d_suf + count, d_suf + 2 * count);
         SUFR_KERNEL_CHECK();
         uint64_t* outs[3] = {suffix, sequence, sequence_pos};
@@ -566,10 +580,7 @@ static uint64_t index_gather(SufrB200Index* idx, uint64_t m, const unsigned long
                              uint64_t max_bytes, uint64_t* byte_offsets, uint8_t* bytes, DevBuf<uint8_t>& d_bytes) {
     Ctx& ctx = *idx->ctx;
     DevBuf<unsigned long long> d_off(ctx.pool, m + 1);
-    DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(m));
-    SUFR_CUDA_CHECK(cudaMemsetAsync(d_off.get(), 0, 8, ctx.stream));
-    scan::inclusive_scan(m, search::ArrayIn{d_len}, scan::SumU64{}, search::HitOffsetOut{d_off.get()}, partials.get(),
-                         ctx.stream);
+    exclusive_offsets(ctx, m, search::ArrayIn{d_len}, d_off.get());
     SUFR_CUDA_CHECK(cudaMemcpyAsync(byte_offsets, d_off.get(), (m + 1) * 8, cudaMemcpyDeviceToHost, ctx.stream));
     SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
     const uint64_t k = (uint64_t)(std::upper_bound(byte_offsets, byte_offsets + m + 1, max_bytes) - byte_offsets) - 1;
@@ -601,7 +612,7 @@ int sufr_b200_index_extract(SufrB200Index* idx, uint64_t first, uint64_t max_hit
         DevBuf<unsigned long long> d_out(ctx.pool, 6 * m);
         unsigned long long* d = d_out.get();
         search::extract_regions_kernel<<<(unsigned)div_up(m, 256), 256, 0, ctx.stream>>>(
-            idx->sa, idx->wide, idx->loc_begin.get(), idx->loc_offsets.get(), idx->loc_queries, idx->starts.get(),
+            idx->sa, idx->wide, idx->loc.begin.get(), idx->loc.offsets.get(), idx->loc.entries, idx->starts.get(),
             idx->num_starts, idx->n, first, m, prefix_len, suffix_len, d, d + m, d + 2 * m, d + 3 * m, d + 4 * m, d + 5 * m);
         SUFR_KERNEL_CHECK();
         DevBuf<uint8_t> d_bytes;
@@ -723,10 +734,7 @@ static uint64_t approx_search(SufrB200Index* idx, const approx::Params& P, const
                 L.excl = DevBuf<unsigned long long>(ctx.pool, L.count);
                 scan::inclusive_scan(L.count, search::ArrayIn{counts.get()}, scan::SumU64{}, approx::ExclOut{L.excl.get()},
                                      partials.get(), ctx.stream);
-                unsigned long long total = 0;
-                SUFR_CUDA_CHECK(cudaMemcpyAsync(&total, partials.get() + div_up(L.count, scan::CHUNK), 8,
-                                                cudaMemcpyDeviceToHost, ctx.stream));
-                SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+                const unsigned long long total = read_total(ctx, partials.get(), L.count);
                 L.cuts = {0};
                 L.at = {0};
                 if ((uint32_t)total > budget) {
@@ -774,10 +782,8 @@ static uint64_t approx_search(SufrB200Index* idx, const approx::Params& P, const
 int sufr_b200_index_approx(SufrB200Index* idx, const uint8_t* queries, const uint64_t* offsets, uint64_t nq,
                            uint64_t max_mismatches, uint64_t* match_offsets, uint64_t* num_hits) {
     return guarded([&] {
-        if (!idx || !offsets || !match_offsets || !num_hits || (nq && !queries && offsets[nq]))
-            throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
-        for (uint64_t i = 0; i < nq; i++)
-            if (offsets[i + 1] < offsets[i]) throw Error(SUFR_B200_ERR_ARGUMENT, "query offsets are not ascending");
+        if (!idx || !match_offsets || !num_hits) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
+        check_queries(queries, offsets, nq);
         if (max_mismatches > 16)
             throw Error(SUFR_B200_ERR_ARGUMENT, "max_mismatches = " + std::to_string(max_mismatches) + " is above 16");
         if (idx->is_mask)
@@ -796,7 +802,8 @@ int sufr_b200_index_approx(SufrB200Index* idx, const uint8_t* queries, const uin
         if (max_depth > 0xFFFFFFFFull) throw Error(SUFR_B200_ERR_ARGUMENT, "a query is longer than 2^32 - 1 bytes");
         Ctx& ctx = *idx->ctx;
         CtxLock lock(ctx);
-        reset_loc(idx);
+        idx->loc = LocateState{};
+        LocateState& loc = idx->loc;
         idx->approx_levels.assign(2 * max_depth, 0);
         approx::Params P{};
         P.text = idx->text;
@@ -816,9 +823,9 @@ int sufr_b200_index_approx(SufrB200Index* idx, const uint8_t* queries, const uin
         DevBuf<uint64_t> keys_a, keys_b;
         DevBuf<uint32_t> vals_a, vals_b;
         bool sorted_in_b = false;
-        idx->loc_begin = DevBuf<unsigned long long>(ctx.pool, 1);  // (replaced below when there are matches)
-        idx->loc_end = DevBuf<unsigned long long>(ctx.pool, 1);
-        idx->loc_mismatches = DevBuf<unsigned long long>(ctx.pool, 1);
+        loc.begin = DevBuf<unsigned long long>(ctx.pool, 1);  // (replaced below when there are matches)
+        loc.end = DevBuf<unsigned long long>(ctx.pool, 1);
+        loc.mismatches = DevBuf<unsigned long long>(ctx.pool, 1);
         if (max_depth && idx->s) {
             DeviceQueries dq(ctx, queries, offsets, nq);
             const auto* d_off = reinterpret_cast<const unsigned long long*>(dq.off.get());
@@ -844,12 +851,12 @@ int sufr_b200_index_approx(SufrB200Index* idx, const uint8_t* queries, const uin
                 SUFR_KERNEL_CHECK();
                 sorted_in_b = sort_u64_u32_pairs(keys_a.get(), keys_b.get(), vals_a.get(), vals_b.get(), matches,
                                                  rank_bits + query_bits, counts.get(), ctx.stream);
-                idx->loc_begin = DevBuf<unsigned long long>(ctx.pool, matches);
-                idx->loc_end = DevBuf<unsigned long long>(ctx.pool, matches);
-                idx->loc_mismatches = DevBuf<unsigned long long>(ctx.pool, matches);
+                loc.begin = DevBuf<unsigned long long>(ctx.pool, matches);
+                loc.end = DevBuf<unsigned long long>(ctx.pool, matches);
+                loc.mismatches = DevBuf<unsigned long long>(ctx.pool, matches);
                 approx::final_gather_kernel<<<(unsigned)div_up(matches, 256), 256, 0, ctx.stream>>>(
-                    finals.get(), (sorted_in_b ? vals_b : vals_a).get(), matches, idx->loc_begin.get(),
-                    idx->loc_end.get(), idx->loc_mismatches.get());
+                    finals.get(), (sorted_in_b ? vals_b : vals_a).get(), matches, loc.begin.get(), loc.end.get(),
+                    loc.mismatches.get());
                 SUFR_KERNEL_CHECK();
             }
         }
@@ -858,22 +865,12 @@ int sufr_b200_index_approx(SufrB200Index* idx, const uint8_t* queries, const uin
             (sorted_in_b ? keys_b : keys_a).get(), matches, rank_bits, nq, d_mo.get());
         SUFR_KERNEL_CHECK();
         SUFR_CUDA_CHECK(cudaMemcpyAsync(match_offsets, d_mo.get(), (nq + 1) * 8, cudaMemcpyDeviceToHost, ctx.stream));
-        // the matches take the place of locate's queries: hit offsets = exclusive scan of their occurrence counts
-        idx->loc_offsets = DevBuf<unsigned long long>(ctx.pool, matches + 1);
-        SUFR_CUDA_CHECK(cudaMemsetAsync(idx->loc_offsets.get(), 0, 8, ctx.stream));
-        if (matches) {
-            DevBuf<unsigned long long> partials(ctx.pool, scan::partials_count(matches));
-            scan::inclusive_scan(matches, search::HitCountIn{idx->loc_begin.get(), idx->loc_end.get()}, scan::SumU64{},
-                                 search::HitOffsetOut{idx->loc_offsets.get()}, partials.get(), ctx.stream);
-        }
-        uint64_t hits = 0;
-        SUFR_CUDA_CHECK(cudaMemcpyAsync(&hits, idx->loc_offsets.get() + matches, 8, cudaMemcpyDeviceToHost, ctx.stream));
-        SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
-        *num_hits = hits;
-        idx->loc_queries = matches;
-        idx->loc_hits = hits;
-        idx->has_loc = true;
-        idx->loc_approx = true;
+        // the matches take the place of locate's queries
+        loc.set(ctx, matches, LocateState::APPROX, [&](const unsigned long long* d_hit_offsets) {
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(num_hits, d_hit_offsets + matches, 8, cudaMemcpyDeviceToHost, ctx.stream));
+            SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
+            return *num_hits;
+        });
     });
 }
 
@@ -883,18 +880,19 @@ int sufr_b200_index_approx_matches(SufrB200Index* idx, uint64_t first, uint64_t 
         if (!idx) throw Error(SUFR_B200_ERR_ARGUMENT, "NULL argument");
         Ctx& ctx = *idx->ctx;
         CtxLock lock(ctx);
-        if (!idx->has_loc || !idx->loc_approx)
+        const LocateState& loc = idx->loc;
+        if (loc.source != LocateState::APPROX)
             throw Error(SUFR_B200_ERR_ARGUMENT, "the last call that set the locate state was not sufr_b200_index_approx");
-        if (first > idx->loc_queries || count > idx->loc_queries - first)
+        if (first > loc.entries || count > loc.entries - first)
             throw Error(SUFR_B200_ERR_ARGUMENT, "match window [" + std::to_string(first) + ", +" + std::to_string(count) +
-                                                    ") is beyond the " + std::to_string(idx->loc_queries) + " matches");
+                                                    ") is beyond the " + std::to_string(loc.entries) + " matches");
         const std::pair<uint64_t*, const unsigned long long*> outs[3] = {
-            {mismatches, idx->loc_mismatches.get()}, {rank_begin, idx->loc_begin.get()}, {rank_end, idx->loc_end.get()}};
+            {mismatches, loc.mismatches.get()}, {rank_begin, loc.begin.get()}, {rank_end, loc.end.get()}};
         for (const auto& o : outs)
             if (o.first && count)
                 SUFR_CUDA_CHECK(cudaMemcpyAsync(o.first, o.second + first, count * 8, cudaMemcpyDeviceToHost, ctx.stream));
         if (hit_offsets)
-            SUFR_CUDA_CHECK(cudaMemcpyAsync(hit_offsets, idx->loc_offsets.get() + first, (count + 1) * 8,
+            SUFR_CUDA_CHECK(cudaMemcpyAsync(hit_offsets, loc.offsets.get() + first, (count + 1) * 8,
                                             cudaMemcpyDeviceToHost, ctx.stream));
         SUFR_CUDA_CHECK(cudaStreamSynchronize(ctx.stream));
     });
@@ -1043,7 +1041,7 @@ int sufr_b200_index_kmers(SufrB200Index* idx, uint64_t k, uint64_t min_count, ui
         scan::scan_reduce(L, listed_in, scan::SumU32{}, listed_partials.get(), ctx.stream);
         uint32_t listed = 0;
         uint64_t tail_next = 0;
-        SUFR_CUDA_CHECK(cudaMemcpyAsync(&listed, listed_partials.get() + div_up(L, scan::CHUNK), 4, cudaMemcpyDeviceToHost,
+        SUFR_CUDA_CHECK(cudaMemcpyAsync(&listed, scan::total_ptr(listed_partials.get(), L), 4, cudaMemcpyDeviceToHost,
                                         ctx.stream));
         unsigned long long last = 0;
         SUFR_CUDA_CHECK(cudaMemcpyAsync(&last, d_listed.get() + L - 1, 8, cudaMemcpyDeviceToHost, ctx.stream));

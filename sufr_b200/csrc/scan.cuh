@@ -326,6 +326,9 @@ __global__ void __launch_bounds__(BLOCK) apply_kernel(uint64_t n, In in, Op op, 
 }
 
 inline size_t partials_count(uint64_t n) { return (size_t)div_up(n, CHUNK) + 1; }
+// Where a scan_reduce or inclusive_scan over n elements leaves its grand total in `partials`.
+template <typename T>
+inline T* total_ptr(T* partials, uint64_t n) { return partials + div_up(n, CHUNK); }
 
 // Two-step form: scan_reduce leaves the exclusive chunk prefixes in `partials` (and the grand total in its last
 // element) so that the caller can size its outputs before scan_apply runs the second pass.

@@ -14,7 +14,8 @@ import pytest
 
 from conftest import GOLDEN, GOLDEN_CASES
 import approx_reference as R
-from test_kmers import SPECS, Case
+from index_matrix import IndexMatrix, device_index
+from test_kmers import SPECS
 
 EXPECTED = GOLDEN / "expected"
 
@@ -99,6 +100,14 @@ def make_queries(text, starts, k, cap, seed):
 def S():
     import sufr_b200
     return sufr_b200
+
+
+class Case(IndexMatrix):
+    def __init__(self, S, name, tmp):
+        (text, starts, names), flags, sources = SPECS[name]
+        super().__init__(S, name, text, starts, names, flags, sources, tmp)
+        self.text = text
+        self.cap = flags.get("max_query_len") or 0
 
 
 @pytest.fixture(scope="module", params=list(SPECS))
@@ -223,12 +232,7 @@ def test_approx_golden(golden, S):
 
 @pytest.mark.gpu
 def test_approx_argument_errors(S):
-    import torch
-    text = b"ACGTACGTTTGA$"
-    t = torch.frombuffer(bytearray(text), dtype=torch.uint8).cuda()
-    args = S.SufrBuilderArgs(text=b"")
-    r = S.build(args, index_bits=32, result_memory=S.MEM_DEVICE, device_text=(t.data_ptr(), t.numel()))
-    index = S.SufrIndex(r, args)
+    index, r = device_index(S, b"ACGTACGTTTGA$", None, None)
     try:
         L = S._lib.lib()
         blob = np.frombuffer(b"ACGTAC", np.uint8)

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN, GOLDEN_CASES, ROOT
+from index_matrix import device_index
 from sufrfile import parse_sufr
 
 EXPECTED = GOLDEN / "expected"
@@ -115,15 +116,6 @@ def check_against_locate(idx, f, queries, mql=None, low_memory=False):
         assert [r.query for r in got] == list(queries)
         want = restate_extract(f.text, f.sequence_starts, f.sequence_names, located, P, S_)
         assert as_rows(got) == want, (P, S_, mql, low_memory)
-
-
-def device_index(S, text, starts, names, index_bits=32, **flags):
-    import torch
-    t = torch.frombuffer(bytearray(text), dtype=torch.uint8).cuda()
-    args = S.SufrBuilderArgs(text=b"", sequence_starts=starts, sequence_names=names, **flags)
-    r = S.build(args, index_bits=index_bits, result_memory=S.MEM_DEVICE, device_text=(t.data_ptr(), t.numel()))
-    r._keep = t
-    return S.SufrIndex(r, args), r
 
 
 # ------------------------------------------------------------------ GPU: every golden, every field

@@ -12,6 +12,7 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN, GOLDEN_CASES, ROOT
+from index_matrix import device_index
 from sufrfile import parse_sufr
 
 EXE = ROOT / "sufr_b200" / "sufr-b200"
@@ -285,15 +286,9 @@ def test_cli_query_file_and_counts(S, tmp_path):
 
 
 def _device_index(S, fasta, flags, index_bits=32):
-    import torch
     flags = dict(flags)
-    delim = flags.pop("delimiter", b"%")
-    seq = S.read_sequence_file(GOLDEN / "inputs" / fasta, delim)
-    t = torch.frombuffer(bytearray(seq.seq), dtype=torch.uint8).cuda()
-    args = S.SufrBuilderArgs(text=b"", sequence_starts=seq.start_positions, sequence_names=seq.sequence_names, **flags)
-    r = S.build(args, index_bits=index_bits, result_memory=S.MEM_DEVICE, device_text=(t.data_ptr(), t.numel()))
-    r._keep = t
-    return S.SufrIndex(r, args), r
+    seq = S.read_sequence_file(GOLDEN / "inputs" / fasta, flags.pop("delimiter", b"%"))
+    return device_index(S, seq.seq, seq.start_positions, seq.sequence_names, index_bits, **flags)
 
 
 @pytest.mark.gpu
@@ -445,12 +440,7 @@ def test_device_locate_against_numpy(S, tmp_path):
 
 @pytest.mark.gpu
 def test_index_without_sequence_starts(S):
-    import torch
-    text = b"ACGTACGTACGT$"
-    t = torch.frombuffer(bytearray(text), dtype=torch.uint8).cuda()
-    args = S.SufrBuilderArgs(text=b"", is_dna=True, sequence_starts=(), sequence_names=())
-    r = S.build(args, index_bits=32, result_memory=S.MEM_DEVICE, device_text=(t.data_ptr(), t.numel()))
-    idx = S.SufrIndex(r, args)
+    idx, r = device_index(S, b"ACGTACGTACGT$", (), (), is_dna=True)
     try:
         (hs,) = idx.locate(["CGT"])
         assert sorted(h[1] for h in hs) == [1, 5, 9]
@@ -474,3 +464,34 @@ def test_suffix_array_entry_beyond_text_is_refused(S, tmp_path):
     assert e.value.code == _lib.ERR_IO and "suffix array entry" in str(e.value)
     r = subprocess.run([str(EXE), "count", str(bad), "AC"], capture_output=True, text=True)
     assert r.returncode == 1 and r.stderr.startswith("Error: ")
+
+
+@pytest.mark.gpu
+def test_batch_calls_refuse_offsets_that_are_not_ascending(S):
+    """Every call that takes a query batch refuses offsets that are not ascending before any device work, and leaves
+    the hits of the last locate readable."""
+    from sufr_b200 import _lib
+    L = _lib.lib()
+    idx = S.SufrIndex.open(EXPECTED / "2.sufr")
+    try:
+        _, _, ho = idx.locate_ranges(["AC", "GT"])
+        n = int(ho[-1])
+        assert n > 0
+        before = [x.tolist() for x in idx.hits(0, n)]
+        blob = np.frombuffer(b"ACGTACGT", np.uint8)
+        bad = np.array([0, 4, 3], np.uint64)
+        out = [np.zeros(8, np.uint64) for _ in range(6)]
+        h, q, o, p, num = idx._h, blob.ctypes.data, bad.ctypes.data, [x.ctypes.data for x in out], C.c_uint64()
+        calls = {
+            "index_search": lambda: L.sufr_b200_index_search(h, q, o, 2, 0, 0, 0, p[0], p[1]),
+            "index_locate": lambda: L.sufr_b200_index_locate(h, q, o, 2, 0, 0, 1, p[0], p[1], p[2]),
+            "index_matching_stats": lambda: L.sufr_b200_index_matching_stats(h, q, o, 2, p[0], p[1], p[2]),
+            "index_mems": lambda: L.sufr_b200_index_mems(h, q, o, 2, 1, C.byref(num), *p),
+            "index_approx": lambda: L.sufr_b200_index_approx(h, q, o, 2, 1, p[0], C.byref(num)),
+        }
+        for name, call in calls.items():
+            assert call() == _lib.ERR_ARGUMENT, name
+            assert "ascending" in L.sufr_b200_last_error().decode(), name
+            assert [x.tolist() for x in idx.hits(0, n)] == before, name
+    finally:
+        idx.close()

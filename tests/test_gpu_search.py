@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN
+from index_matrix import device_index
 import oracle as O
 
 pytestmark = pytest.mark.gpu
@@ -20,13 +21,8 @@ def S():
 
 
 def make_index(S, fasta, index_bits=32, delimiter=b"%", **kw):
-    import torch
     seq = S.read_sequence_file(GOLDEN / "inputs" / fasta, delimiter)
-    t = torch.frombuffer(bytearray(seq.seq), dtype=torch.uint8).cuda()
-    args = S.SufrBuilderArgs(text=b"", sequence_starts=seq.start_positions, sequence_names=seq.sequence_names, **kw)
-    r = S.build(args, index_bits=index_bits, result_memory=S.MEM_DEVICE, device_text=(t.data_ptr(), t.numel()))
-    r._keep = t
-    return S.SufrIndex(r, args), r, seq
+    return device_index(S, seq.seq, seq.start_positions, seq.sequence_names, index_bits, **kw) + (seq,)
 
 
 def parse_relative(path):

@@ -11,9 +11,8 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN, GOLDEN_CASES
+from index_matrix import ACGT, ALL, PROTEIN, IndexMatrix, make_text, with_records
 import kmer_reference as K
-from test_mems import with_records
-from test_search_reference import ACGT, PROTEIN, make_text
 
 EXPECTED = GOLDEN / "expected"
 U64_MAX = 0xFFFFFFFFFFFFFFFF
@@ -67,9 +66,6 @@ def test_reference_against_spec_groups():
 
 
 # ------------------------------------------------------------------ GPU fixtures
-ALL = [("built", 32), ("built", 64), ("file", 32), ("file", 64)]
-
-
 def n_run_text():
     t = bytearray(make_text(50, 6000, ACGT, copies=60, runs=[(b"T", 40)], rare=b"N", rare_p=0.01))
     t[2000:3200] = b"N" * 1200  # an N run of 1200: the N-run LCP rule
@@ -97,33 +93,13 @@ def S():
     return sufr_b200
 
 
-class Case:
+class Case(IndexMatrix):
     def __init__(self, S, name, tmp):
-        import torch
         (text, starts, names), flags, sources = SPECS[name]
-        self.text, self.starts, self.flags = text, starts, flags
+        super().__init__(S, name, text, starts, names, flags, sources, tmp)
+        self.text = text
         self.dna = bool(flags.get("is_dna"))
         self.cap = flags.get("max_query_len") or 0
-        self.indexes, self._results = [], []
-        try:
-            for kind, bits in sources:
-                if kind == "built":
-                    t = torch.frombuffer(bytearray(text), dtype=torch.uint8).cuda()
-                    args = S.SufrBuilderArgs(text=b"", sequence_starts=starts, sequence_names=names, **flags)
-                    r = S.build(args, index_bits=bits, result_memory=S.MEM_DEVICE, device_text=(t.data_ptr(), t.numel()))
-                    r._keep = t
-                    self._results.append(r)
-                    index = S.SufrIndex(r, args)
-                else:
-                    path = tmp / f"{name}_u{bits}.sufr"
-                    b = S.SufrBuilder(S.SufrBuilderArgs(text=text, path=str(path), sequence_starts=starts,
-                                                        sequence_names=names, **flags), bits)
-                    b._res.free()
-                    index = S.SufrIndex.open(path)
-                self.indexes.append((f"{kind}_u{bits}", index))
-        except BaseException:
-            self.close()
-            raise
 
     def ks(self):
         n = len(self.text)
@@ -133,13 +109,6 @@ class Case:
         if self.cap:
             ks = {k for k in ks if k <= self.cap} | {self.cap}
         return sorted(ks)
-
-    def close(self):
-        for _, index in self.indexes:
-            index.close()
-        for r in self._results:
-            r.free()
-        self.indexes, self._results = [], []
 
 
 @pytest.fixture(scope="module", params=list(SPECS))

@@ -12,11 +12,11 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN, GOLDEN_CASES
+from index_matrix import ACGT, ALL, PROTEIN, WIDE, IndexMatrix, make_text, with_records
 import mems_reference as M
 import search_reference as R
 from sufrfile import parse_sufr
 from test_extract import concat_windows, restate_region
-from test_search_reference import ACGT, PROTEIN, WIDE, make_text
 
 EXPECTED = GOLDEN / "expected"
 NONE = M.NONE
@@ -97,20 +97,6 @@ def test_reference_against_all_pairs_mems():
 
 
 # ------------------------------------------------------------------ GPU fixtures
-def with_records(text, k, seed):
-    """`text` with k - 1 of its bytes replaced by the delimiter '%': (text, sequence starts, names)."""
-    n = len(text)
-    if k <= 1 or n < 4 * k:
-        return text, [0], ["r0"]
-    rng = random.Random(seed)
-    cut = sorted(rng.sample(range(1, n - 2), k - 1))
-    t = bytearray(text)
-    for c in cut:
-        t[c] = ord("%")
-    return bytes(t), [0] + [c + 1 for c in cut], [f"r{i}" for i in range(k)]
-
-
-ALL = [("built", 32), ("built", 64), ("file", 32), ("file", 64)]
 SPECS = {
     # name -> (text, starts, names), build flags, index sources
     "tiny_1": ((b"NNNA", [0], ["r0"]), dict(is_dna=True), ALL),
@@ -168,46 +154,14 @@ def S():
     return sufr_b200
 
 
-class Case:
+class Case(IndexMatrix):
     """One text built every way its spec lists, its reference matcher and queries."""
 
     def __init__(self, S, name, tmp):
-        import torch
         (text, starts, names), flags, sources = SPECS[name]
-        self.name, self.flags, self.starts, self.names = name, flags, starts, names
-        self.indexes, self._results, arrays = [], [], None
-        try:
-            for kind, bits in sources:
-                if kind == "built":
-                    t = torch.frombuffer(bytearray(text), dtype=torch.uint8).cuda()
-                    args = S.SufrBuilderArgs(text=b"", sequence_starts=starts, sequence_names=names, **flags)
-                    r = S.build(args, index_bits=bits, result_memory=S.MEM_DEVICE, device_text=(t.data_ptr(), t.numel()))
-                    r._keep = t
-                    self._results.append(r)
-                    udt = np.uint32 if bits == 32 else np.uint64
-                    got = (r.text_tensor().cpu().numpy().tobytes(), r.sa_tensor().cpu().numpy().view(udt),
-                           r.lcp_tensor().cpu().numpy().view(udt))
-                    index = S.SufrIndex(r, args)
-                else:
-                    path = tmp / f"{name}_u{bits}.sufr"
-                    b = S.SufrBuilder(S.SufrBuilderArgs(text=text, path=str(path), sequence_starts=starts,
-                                                        sequence_names=names, **flags), bits)
-                    b._res.free()
-                    f = parse_sufr(path.read_bytes())
-                    assert f.index_bits == bits
-                    got = (f.text, f.sa, f.lcp)
-                    index = S.SufrIndex.open(path)
-                self.indexes.append((f"{kind}_u{bits}", index))
-                got = (got[0], got[1].astype(np.int64), got[2].astype(np.int64))
-                if arrays is None:
-                    arrays = got
-                else:
-                    assert got[0] == arrays[0] and np.array_equal(got[1], arrays[1]) and np.array_equal(got[2], arrays[2])
-        except BaseException:
-            self.close()
-            raise
-        self.ref = R.Index(arrays[0], arrays[1], arrays[2], flags.get("max_query_len") or 0)
-        self.text = arrays[0]
+        super().__init__(S, name, text, starts, names, flags, sources, tmp)
+        self.ref = R.Index(*self.arrays, flags.get("max_query_len") or 0)
+        self.text = self.arrays[0]
         self.matcher = M.Matcher(self.ref)
         alphabet = sorted(set(text)) or [65]
         self.queries = make_queries(self.text, starts, name, alphabet, whole=len(text) <= 8000)
@@ -225,13 +179,6 @@ class Case:
 
     def want_mems(self, min_len):
         return [M.mems_of(*w, min_len) for w in self.want]
-
-    def close(self):
-        for _, index in self.indexes:
-            index.close()
-        for r in self._results:
-            r.free()
-        self.indexes, self._results = [], []
 
 
 @pytest.fixture(scope="module", params=list(SPECS))

@@ -13,6 +13,7 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN, ROOT
+from index_matrix import ACGT, ALL, PROTEIN, WIDE, IndexMatrix, make_text
 import search_reference as R
 from sufrfile import parse_sufr
 from test_file_query import CLI_FIXTURES, _want, format_locate
@@ -156,31 +157,6 @@ def test_reference_against_brute_force():
 
 
 # ------------------------------------------------------------------ GPU: search_kernel against the reference
-def make_text(seed, n, alphabet, *, copies=0, copy_len=(10, 100), runs=(), rare=b"", rare_p=0.0, dollar=True):
-    """n random bytes of `alphabet`, with `copies` segments copied from elsewhere in the text (repeats, long LCPs),
-    tandem runs of the given units, and bytes of `rare` sprinkled at rate rare_p."""
-    rng = np.random.default_rng(seed)
-    t = np.frombuffer(alphabet, np.uint8)[rng.integers(0, len(alphabet), n)]
-    for _ in range(copies):
-        ln = int(rng.integers(copy_len[0], copy_len[1] + 1))
-        if ln >= n:
-            continue
-        src, dst = (int(x) for x in rng.integers(0, n - ln, 2))
-        t[dst:dst + ln] = t[src:src + ln].copy()
-    for unit, count in runs:
-        u = np.frombuffer(unit, np.uint8)
-        ln = min(n, len(u) * count)
-        dst = int(rng.integers(0, n - ln + 1))
-        t[dst:dst + ln] = np.tile(u, count)[:ln]
-    if rare:
-        hit = np.flatnonzero(rng.random(n) < rare_p)
-        t[hit] = np.frombuffer(rare, np.uint8)[rng.integers(0, len(rare), len(hit))]
-    return t.tobytes() + (b"$" if dollar else b"")
-
-
-ACGT, PROTEIN = b"ACGT", b"ACDEFGHIKLMNPQRSTVWY"
-WIDE = bytes(range(1, 97)) + bytes(range(123, 256))  # (lowercase bytes would be uppercased by the build)
-ALL = [("built", 32), ("built", 64), ("file", 32), ("file", 64)]
 MASKS = ["101", "11011", "10111011", "1101101101", "111010010100110111"]
 
 # name -> (text, build flags, index sources, query generator settings)
@@ -277,59 +253,20 @@ def S():
     return sufr_b200
 
 
-class Case:
+class Case(IndexMatrix):
     """One text built every way its spec lists, its reference index and queries, and the expected answers."""
 
     def __init__(self, S, name, tmp):
-        import torch
         text, flags, sources = SPECS[name]
-        self.name, self.flags = name, flags
-        self.indexes, self._results = [], []
-        arrays = None
-        try:
-            for kind, bits in sources:
-                if kind == "built":
-                    t = torch.frombuffer(bytearray(text), dtype=torch.uint8).cuda()
-                    args = S.SufrBuilderArgs(text=b"", **flags)
-                    r = S.build(args, index_bits=bits, result_memory=S.MEM_DEVICE, device_text=(t.data_ptr(), t.numel()))
-                    r._keep = t
-                    self._results.append(r)
-                    udt = np.uint32 if bits == 32 else np.uint64  # (the tensors hold the same bits as signed)
-                    got = (r.text_tensor().cpu().numpy().tobytes(), r.sa_tensor().cpu().numpy().view(udt),
-                           r.lcp_tensor().cpu().numpy().view(udt))
-                    index = S.SufrIndex(r, args)
-                else:
-                    path = tmp / f"{name}_u{bits}.sufr"
-                    b = S.SufrBuilder(S.SufrBuilderArgs(text=text, path=str(path), **flags), bits)
-                    b._res.free()
-                    f = parse_sufr(path.read_bytes())
-                    assert f.index_bits == bits
-                    got = (f.text, f.sa, f.lcp)
-                    index = S.SufrIndex.open(path)
-                self.indexes.append((f"{kind}_u{bits}", index))
-                got = (got[0], got[1].astype(np.int64), got[2].astype(np.int64))
-                if arrays is None:
-                    arrays = got
-                else:  # every source holds the same index
-                    assert got[0] == arrays[0] and np.array_equal(got[1], arrays[1]) and np.array_equal(got[2], arrays[2])
-        except BaseException:
-            self.close()
-            raise
-        self.ref = R.Index(arrays[0], arrays[1], arrays[2], flags.get("max_query_len") or 0, flags.get("seed_mask"))
+        super().__init__(S, name, text, None, None, flags, sources, tmp)
+        self.ref = R.Index(*self.arrays, flags.get("max_query_len") or 0, flags.get("seed_mask"))
         self.caps = run_caps(flags, self.ref.n)
-        alphabet = sorted(set(arrays[0])) or [65]
+        alphabet = sorted(set(self.arrays[0])) or [65]
         self.queries = make_queries(self.ref, name, self.caps, alphabet)
         self.full = {m: R.full_ranges(self.ref, self.queries, m) for m in self.caps}
 
     def expected(self, m, low_memory):
         return R.expected(self.ref, self.queries, m, low_memory, self.full[m])
-
-    def close(self):
-        for _, index in self.indexes:
-            index.close()
-        for r in self._results:
-            r.free()
-        self.indexes, self._results = [], []
 
 
 @pytest.fixture(scope="module", params=list(SPECS))
